@@ -1,11 +1,13 @@
 """bench.py -- images/sec of the PoseNet hot path (backbone + heads + multi-pose decode).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c3|c4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c2|c3|c4] [--dump-outputs DIR]
 
 One "step" = one pass of  uint8 images -> (fused preprocess) stem -> 13 separable blocks -> heads ->
 part candidates -> greedy decode  over one batch.  Default workload = BASELINE.json configs[1]:
 MobileNetV1 model 101, 513x513, output stride 16, batch 64 per GPU, bf16, random-init weights, synthetic images.
-Rank 0 prints ONE JSON line (see the keys below).  ``--impl reference`` times the reference's own CPU code on the host
+Rank 0 prints ONE JSON line (see the keys below); with ``--dump-outputs DIR`` it also writes the pose records of the last
+timed step to ``DIR/*.npy`` (inputs and weights are seeded, so two builds can be compared output for output).
+``--impl reference`` times the reference's own CPU code on the host
 cores instead: the unmodified reference package byte-compiled into ``oracle/_ref`` by ``oracle/make_ref.py``
 (``cpu_baseline.kind`` "reference"), or, when that build is absent, the oracle port (``kind`` "port": torch-CPU fp32
 convs + numpy float64 decode).  Both arms print the same ``config`` dict; how each arm batches the workload is in ``run``.
@@ -319,6 +321,25 @@ def h2d_ceiling(host_batches, dev, world, reps=6):
     return world * reps * host_batches[0].numel() / (ms * 1e-3) / 1e9
 
 
+DUMP_NAMES = ("pose_scores", "keypoint_scores", "keypoint_coords", "pose_offsets", "pose_counts")   # decode_multiple_poses_batch
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, outputs):
+    """Write the records of one step as ``out_dir/<name>.npy`` (float64, first axis = image).  Above DUMP_LIMIT bytes only a
+    fixed, seeded sample of images is written, and their batch indices go to ``image_index.npy``."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = [t.numpy().astype(np.float64) for t in outputs]
+    n = arrays[0].shape[0]
+    per_image = sum(a.nbytes for a in arrays) // n
+    if n * per_image > DUMP_LIMIT:
+        index = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT // (per_image + 8), replace=False))
+        arrays = [a[index] for a in arrays]
+        np.save(os.path.join(out_dir, "image_index.npy"), index.astype(np.float64))
+    for name, a in zip(DUMP_NAMES, arrays):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_b200(args):
     if PKG not in sys.path:
         sys.path.insert(0, PKG)
@@ -390,6 +411,7 @@ def run_b200(args):
     barrier()
     sampler.window = (t_begin, time.perf_counter())
     ms = e0.elapsed_time(e1)
+    last_step = [t.cpu() for t in graphs[(args.steps - 1) % n_sets][1]] if args.dump_outputs and rank == 0 else None
     # the nvidia-smi fallback answers in ~100 ms and the timed region can be shorter than that: keep the SAME load running
     # (untimed) until the sampler has at least 5 readings; NVML readings (~0.1 ms each) land inside the timed region
     t_extra = time.perf_counter()
@@ -537,6 +559,8 @@ def run_b200(args):
         line["value_sustained"] = sustained["value"]
     if cpu:
         line["cpu_baseline"] = cpu
+    if last_step is not None:
+        dump_outputs(args.dump_outputs, last_step)
     print(json.dumps(line), flush=True)
     if world > 1:
         torch.distributed.destroy_process_group()
@@ -555,7 +579,10 @@ def main():
     ap.add_argument("--sustain", type=float, default=3.0, help="seconds of back-to-back replays for the sustained leg (0: skip)")
     ap.add_argument("--depth", type=int, default=3, help="batches in flight in the end-to-end leg (BatchPipeline depth)")
     ap.add_argument("--unfused", action="store_true", help="run every block as depthwise + pointwise kernels (A/B against the fused blocks)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write rank 0's pose records of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs records the B200 arm only")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
@@ -26,8 +27,8 @@ def _ref_kind():
     return "reference" if make_ref.available() else "port"
 
 
-def test_product_arm_line():
-    d = _run("--steps", "4", "--warmup", "3", "--sustain", "1.0")
+def test_product_arm_line(tmp_path):
+    d = _run("--steps", "4", "--warmup", "3", "--sustain", "1.0", "--dump-outputs", str(tmp_path))
     assert d["metric"] == "images/sec (backbone+decode)" and d["unit"] == "images/sec" and d["higher_is_better"] is True
     assert d["n_gpus"] == 1 and d["steps"] == 4 and d["warmup"] == 3 and d["scaling"] == "weak" and d["vs_baseline"] is None
     assert d["dtype"] == "bf16" and d["data"] == "synthetic" and "BASELINE configs[1]" in d["config"]["workload"]
@@ -51,6 +52,23 @@ def test_product_arm_line():
     assert d["value_sustained"] == su["value"] and su["seconds"] >= 0.9 and 0.3 < su["vs_burst"] < 1.2
     assert su["clocks"]["sm_mhz"] and isinstance(su["clocks"]["reasons"], list)
     assert d["run"]["batch_per_gpu"] == 64 and d["config"]["model"] == "mobilenet_v1_101"
+    # --dump-outputs: the records of the last timed step (step 3 of 4 reads input set 3), float64, equal to an eager run of
+    # the same seeded model on the same seeded images
+    sys.path.insert(0, ROOT)
+    import bench
+    import posenet
+    import torch
+    dumped = [np.load(tmp_path / (name + ".npy")) for name in bench.DUMP_NAMES]
+    assert sorted(os.listdir(tmp_path)) == sorted(name + ".npy" for name in bench.DUMP_NAMES)
+    assert all(a.dtype == np.float64 for a in dumped) and dumped[2].shape == (64, 10, 17, 2)
+    rng = np.random.default_rng(1234)
+    x = [rng.integers(0, 256, (64, 513, 513, 3), dtype=np.uint8) for _ in range(4)][3]
+    torch.manual_seed(0)
+    model = posenet.MobileNetV1(101, output_stride=16).cuda().set_compute_dtype("bf16").set_fused(True)
+    ref = posenet.decode_multiple_poses_batch(*model.forward_u8(torch.from_numpy(x).cuda()), output_stride=16, **bench.DECODE_KW)
+    for a, b in zip(dumped, ref):
+        assert np.array_equal(a, b.cpu().numpy().astype(np.float64))
+    assert np.array_equal(dumped[4], (dumped[0] != 0).sum(1))
 
 
 def test_reference_arm_line():
