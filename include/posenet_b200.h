@@ -145,6 +145,20 @@ int pn_decode_pose(double root_score, int root_id, const double *root_image_coor
 int pn_scale_keypoint_coords(double *kp_coords, int n_img, int points_per_img, const double *scales, double scale_y,
                              double scale_x, pn_stream_t stream);
 
+/* ---- N4: posenet/utils.py draw_skel_and_kp (image_demo.py:53) / draw_skeleton for a batch of frames ON THE DEVICE, drawn in
+ * place and bit-exact with cv2 (drawKeypoints DRAW_RICH_KEYPOINTS circles, then polylines; colour (255, 255, 0) BGR).
+ * frames: uint8 BGR HWC, image i at frames + i * frame_stride (bytes, >= h*w*3), rows w_i*3 bytes apart.  frame_hw: device
+ * int32 [n_img, 2] with each frame's (h_i, w_i) (<= h, w; other rows, e.g. (0, 0), are skipped), or NULL for h x w everywhere.  The records
+ * are pn_decode_greedy's (float64, coordinates (y, x) in frame pixels): pose_scores [n_img, max_poses], kp_scores
+ * [n_img, max_poses, 17], kp_coords [n_img, max_poses, 17, 2]; max_poses <= 512.  `what`: PN_DRAW_KEYPOINTS | PN_DRAW_SKELETON
+ * (both: draw_skel_and_kp; PN_DRAW_SKELETON alone: draw_skeleton).  Nothing outside a frame is written, whatever the
+ * coordinates; within +-2^26 px they match cv2 bit for bit. */
+#define PN_DRAW_KEYPOINTS 1
+#define PN_DRAW_SKELETON 2
+int pn_draw_poses(uint8_t *frames, int n_img, int h, int w, int64_t frame_stride, const int *frame_hw, const double *pose_scores,
+                  const double *kp_scores, const double *kp_coords, int max_poses, double min_pose_score, double min_part_score,
+                  int what, pn_stream_t stream);
+
 /* ---- Whole-network plan: mobilenet_v1.py:130-162 (MobileNetV1.__init__/forward) --------------------
  * The layer table is computed by the caller (posenet/models/mobilenet_v1.py mirrors
  * _to_output_strided_layers, mobilenet_v1.py:8-39) and passed in explicitly. */

@@ -16,6 +16,7 @@ PN_F32, PN_BF16 = 0, 1
 NUM_PARTS, NUM_EDGES, HEAD_CHANNELS, HEAD_ROWS = 17, 16, 115, 128
 ABI_VERSION = 5
 PLAN_UNFUSED = 1
+DRAW_KEYPOINTS, DRAW_SKELETON = 1, 2
 
 
 class NativeError(RuntimeError):
@@ -72,6 +73,8 @@ _SIGNATURES = {
     "pn_decode_pose": (C.c_int, [C.c_double, C.c_int, C.POINTER(C.c_double), C.POINTER(Map), C.POINTER(Map), C.POINTER(Map),
                                  C.POINTER(Map), C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "pn_scale_keypoint_coords": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_double, C.c_double, C.c_void_p]),
+    "pn_draw_poses": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                C.c_int, C.c_double, C.c_double, C.c_int, C.c_void_p]),
     "pn_plan_query": (C.c_int, [C.POINTER(NetDesc), C.POINTER(C.c_size_t), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "pn_plan_create": (C.c_int, [C.POINTER(NetDesc), C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p)]),
     "pn_plan_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

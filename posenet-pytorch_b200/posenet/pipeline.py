@@ -26,7 +26,7 @@ from posenet.decode_multi import decode_multiple_poses_batch, split_pose_records
 
 class BatchPipeline:
     def __init__(self, model, batch, height, width, depth=2, use_graph=True, output_stride=None, scale_factor=1.0,
-                 source_coords=False, mixed=False, gather=False, group=None, **decode_kw):
+                 source_coords=False, mixed=False, gather=False, group=None, overlay=None, **decode_kw):
         """``height`` x ``width``: size of the uint8 frames handed to ``submit`` (``mixed=True``: the LARGEST frame; each
         frame of a batch then comes with its own size).  The network runs at ``valid_resolution(width * scale_factor,
         height * scale_factor)`` (utils.py:7-10); frames of any other size go through the bit-exact cv2 resize
@@ -36,7 +36,11 @@ class BatchPipeline:
         the record buffer on the device (``pn_scale_keypoint_coords``), per frame in mixed mode.
         ``gather``: with an initialised process group, every step ends with an all-gather of the ranks' record buffers (NCCL over
         NVLink) on its own stream -- the kernels of the next batch do not wait for it -- and rank 0 reads ALL ranks' records back
-        (``result(..., gathered=True)``); the other ranks read back their own, as without ``gather``."""
+        (``result(..., gathered=True)``); the other ranks read back their own, as without ``gather``.
+        ``overlay=(min_pose_score, min_part_score)``: the step also draws ``draw_skel_and_kp`` (image_demo.py:53) on the submitted
+        frames at their own size, on the device (``pn_draw_poses``, bit-exact with cv2), and copies them back after the records;
+        ``result`` then returns the frames as a fifth item.  Frames that are resized need ``source_coords=True`` (the overlay is
+        drawn in their coordinates).  With ``gather``, the frames stay on their rank."""
         nat.require_device()
         assert depth >= 1
         self.model, self.batch, self.h, self.w = model, int(batch), int(height), int(width)
@@ -47,6 +51,9 @@ class BatchPipeline:
         self.resize = self.mixed or (self.th, self.tw) != (self.h, self.w)
         self.scale = np.array([self.h / self.th, self.w / self.tw])           # utils.py:19, for mapping coordinates back
         self.source_coords = bool(source_coords)
+        self.overlay = None if overlay is None else (float(overlay[0]), float(overlay[1]))
+        assert self.overlay is None or self.source_coords or not self.resize, \
+            "overlay on resized frames needs source_coords=True (the records must be in the frames' coordinates)"
         self.decode_kw = dict(decode_kw)
         self.P = int(self.decode_kw.get("max_pose_detections", 10))
         dev = model._device()
@@ -72,10 +79,16 @@ class BatchPipeline:
                          rec_host=torch.zeros((self.world if self.collect_all else 1) * nrec, dtype=torch.float64).pin_memory(),
                          scales=torch.ones((self.batch, 2), dtype=torch.float64, device=dev) if self.mixed else None,
                          scales_host=torch.ones((self.batch, 2), dtype=torch.float64).pin_memory() if self.mixed else None,
+                         frames_host=torch.empty((self.batch, self.h, self.w, 3), dtype=torch.uint8).pin_memory() if self.overlay else None,
+                         hw=torch.zeros((self.batch, 2), dtype=torch.int32, device=dev) if self.overlay and self.mixed else None,
+                         hw_host=torch.zeros((self.batch, 2), dtype=torch.int32).pin_memory() if self.overlay and self.mixed else None,
+                         shapes=None,
                          copied=torch.cuda.Event(), done=torch.cuda.Event(), out=torch.cuda.Event(), graph=None, busy=False)
                 self.slots.append(s)
             self.h2d_bytes_per_batch = self.slots[0]["x"].numel()
             self.d2h_bytes_per_batch = (self.world if self.collect_all else 1) * nrec * 8
+            if self.overlay:
+                self.d2h_bytes_per_batch += self.slots[0]["x"].numel()         # mixed mode copies only the bytes in use
             # warm up (plans, workspaces) and capture one graph per slot on the compute stream
             self.compute.wait_stream(torch.cuda.current_stream(dev))
             with torch.cuda.stream(self.compute):
@@ -95,7 +108,8 @@ class BatchPipeline:
         self._next = 0
 
     def _enqueue(self, s):
-        """The captured part of a step: (uniform resize ->) stem .. heads -> candidates -> greedy decode (-> coordinate scaling)."""
+        """The captured part of a step: (uniform resize ->) stem .. heads -> candidates -> greedy decode (-> coordinate scaling)
+        (-> overlay on the submitted frames)."""
         x = s["x"]
         lib = nat.load()
         if self.resize and not self.mixed:
@@ -110,6 +124,13 @@ class BatchPipeline:
                                                    C.c_void_p(s["scales"].data_ptr()) if self.mixed else None,
                                                    float(self.scale[0]), float(self.scale[1]), nat.stream_ptr()),
                       "pn_scale_keypoint_coords")
+        if self.overlay:
+            x = s["x"]
+            nat.check(lib.pn_draw_poses(C.c_void_p(x.data_ptr()), self.batch, self.h, self.w, self.h * self.w * 3,
+                                        C.c_void_p(s["hw"].data_ptr()) if self.mixed else None, C.c_void_p(ps.data_ptr()),
+                                        C.c_void_p(ks.data_ptr()), C.c_void_p(kc.data_ptr()), self.P, self.overlay[0],
+                                        self.overlay[1], nat.DRAW_KEYPOINTS | nat.DRAW_SKELETON, nat.stream_ptr()),
+                      "pn_draw_poses")
 
     def _resize_mixed(self, s, shapes):
         """Per-frame cv2-exact resize of frames stored at their own size (row i of the slot's input buffer holds frame i
@@ -147,11 +168,19 @@ class BatchPipeline:
             sc.fill_(1.0)
             for i, (h, w) in enumerate(shapes):
                 sc[i, 0], sc[i, 1] = h / self.th, w / self.tw                     # utils.py:19, per frame
+            if self.overlay:
+                hw = s["hw_host"]
+                hw.zero_()                                                        # rows without a frame are not drawn
+                if shapes:
+                    hw[:len(shapes)] = torch.tensor(shapes, dtype=torch.int32)
         else:
             assert shapes is None, "shapes are for mixed=True pipelines"
+        s["shapes"] = shapes
         with torch.cuda.device(self.dev):
             with torch.cuda.stream(self.h2d):
                 self.h2d.wait_event(s["done"])              # the previous use of this slot's input buffer has finished
+                if self.overlay:
+                    self.h2d.wait_event(s["out"])           # ... and its drawn frames have been copied back
                 if self.mixed and shapes:
                     used = max(h * w * 3 for h, w in shapes)                      # one strided copy of the bytes in use
                     s["x"].view(self.batch, -1)[:len(shapes), :used].copy_(host_batch.view(self.batch, -1)[:len(shapes), :used],
@@ -159,6 +188,8 @@ class BatchPipeline:
                     s["scales"].copy_(sc, non_blocking=True)
                 elif not self.mixed:
                     s["x"].copy_(host_batch.view(s["x"].shape), non_blocking=True)
+                if self.overlay and self.mixed:
+                    s["hw"].copy_(s["hw_host"], non_blocking=True)
                 s["copied"].record(self.h2d)
             with torch.cuda.stream(self.compute):
                 self.compute.wait_event(s["copied"])
@@ -178,6 +209,12 @@ class BatchPipeline:
                     import torch.distributed as dist
                     dist.all_gather_into_tensor(s["rec_all"], s["rec"], group=self.group)
                 s["rec_host"].copy_(s["rec_all"] if self.collect_all else s["rec"], non_blocking=True)
+                if self.overlay and self.mixed and shapes:
+                    used = max(h * w * 3 for h, w in shapes)
+                    s["frames_host"].view(self.batch, -1)[:len(shapes), :used].copy_(s["x"].view(self.batch, -1)[:len(shapes), :used],
+                                                                                   non_blocking=True)
+                elif self.overlay and not self.mixed:
+                    s["frames_host"].copy_(s["x"], non_blocking=True)
                 s["out"].record(self.d2h)
         s["busy"] = True
         ticket = self._next
@@ -186,7 +223,8 @@ class BatchPipeline:
 
     def result(self, ticket, copy=True, source_coords=None, gathered=False):
         """Block until the ticket's records are on the host; returns the reference's 4-tuple for this rank's batch
-        (numpy float64: [batch,P], [batch,P,17], [batch,P,17,2], [batch,P,17,2]).  ``gathered=True`` (rank 0 of a
+        (numpy float64: [batch,P], [batch,P,17], [batch,P,17,2], [batch,P,17,2]).  With ``overlay``, a fifth item holds this
+        rank's drawn frames: uint8 [batch,h,w,3], or in mixed mode a list of [h_i,w_i,3] arrays, one per submitted frame.  ``gathered=True`` (rank 0 of a
         ``gather=True`` pipeline): the records of ALL ranks' batches instead, leading dimension ``world * batch`` (rank-major).
         ``source_coords`` is a construction-time option (the scaling runs on the device); passing a different value here is an
         error."""
@@ -199,12 +237,21 @@ class BatchPipeline:
         flat = s["rec_host"].numpy()
         if copy:
             flat = flat.copy()
+        frames = ()
+        if self.overlay:
+            fr = s["frames_host"].numpy()
+            if self.mixed:
+                rows = fr.reshape(self.batch, -1)
+                fr = [rows[i, :h * w * 3].reshape(h, w, 3) for i, (h, w) in enumerate(s["shapes"])]
+                frames = ([f.copy() for f in fr] if copy else fr,)
+            else:
+                frames = (fr.copy() if copy else fr,)
         if not gathered:
             own = flat[self.rank * self.nrec:(self.rank + 1) * self.nrec] if self.collect_all else flat
-            return split_pose_records(own, self.batch, self.P)
+            return split_pose_records(own, self.batch, self.P) + frames
         assert self.collect_all, "gathered=True: only rank 0 of a gather=True pipeline reads every rank's records back"
         parts = [split_pose_records(flat[r * self.nrec:(r + 1) * self.nrec], self.batch, self.P) for r in range(self.world)]
-        return tuple(np.concatenate([p[j] for p in parts], axis=0) for j in range(4))
+        return tuple(np.concatenate([p[j] for p in parts], axis=0) for j in range(4)) + frames
 
     def time_gather(self, reps=20):
         """Device time (ms) of one all-gather of a step's record buffer, measured alone with CUDA events."""

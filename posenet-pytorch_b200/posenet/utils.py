@@ -4,7 +4,8 @@
 [1,3,H,W] numpy, source image, scale)`` out -- but the resize / colour swap / normalisation run in
 the fused CUDA kernel ``pn_preprocess_u8`` (bit-exact with cv2's INTER_LINEAR).  For device-resident
 pipelines use ``process_input_gpu``, which returns the CUDA tensor without the copy back.
-The drawing helpers are host-side visualisation (out of the accelerated path).
+The drawing helpers with the reference's names are host-side (cv2); ``draw_skel_and_kp_batch`` / ``draw_skeleton_batch`` draw
+the same pixels on device-resident frames with the CUDA kernel ``pn_draw_poses``.
 """
 import ctypes as C
 
@@ -127,3 +128,39 @@ def draw_skel_and_kp(img, instance_scores, keypoint_scores, keypoint_coords,
         out_img = cv2.drawKeypoints(out_img, pts, outImage=np.array([]), color=(255, 255, 0),
                                     flags=cv2.DRAW_MATCHES_FLAGS_DRAW_RICH_KEYPOINTS)
     return cv2.polylines(out_img, segments, isClosed=False, color=(255, 255, 0))
+
+
+# ---------------------------------------------------------------------------- overlays (device)
+def _draw_batch(frames, pose_scores, keypoint_scores, keypoint_coords, min_pose, min_part, what):
+    nat.require_device()
+    assert torch.is_tensor(frames) and frames.is_cuda and frames.dtype == torch.uint8 and frames.dim() == 4 and frames.shape[3] == 3, \
+        "expected uint8 CUDA frames [N,h,w,3]"
+    n, h, w = frames.shape[:3]
+    st = frames.stride()
+    assert st[3] == 1 and st[2] == 3 and st[1] == 3 * w and st[0] >= 3 * h * w, \
+        "each frame must be stored densely (rows of w*3 bytes); frames may be further apart"
+    dev = frames.device
+    ps, ks, kc = (torch.as_tensor(t, dtype=torch.float64, device=dev).contiguous()
+                  for t in (pose_scores, keypoint_scores, keypoint_coords))
+    P = ps.shape[-1]
+    assert tuple(ps.shape) == (n, P) and tuple(ks.shape) == (n, P, 17) and tuple(kc.shape) == (n, P, 17, 2), \
+        "expected records [N,P], [N,P,17], [N,P,17,2] for %d frames" % n
+    with torch.cuda.device(dev):
+        nat.check(nat.load().pn_draw_poses(C.c_void_p(frames.data_ptr()), n, h, w, st[0], None, C.c_void_p(ps.data_ptr()),
+                                           C.c_void_p(ks.data_ptr()), C.c_void_p(kc.data_ptr()), P, float(min_pose),
+                                           float(min_part), what, nat.stream_ptr()), "pn_draw_poses")
+    return frames
+
+
+def draw_skel_and_kp_batch(frames, pose_scores, keypoint_scores, keypoint_coords, min_pose_score=0.5, min_part_score=0.5):
+    """``draw_skel_and_kp`` of every frame of a batch, on the GPU and bit-exact with it.  ``frames``: uint8 CUDA [N,h,w,3]
+    (BGR), drawn IN PLACE and returned; the records are ``decode_multiple_poses_batch``'s (float64 CUDA [N,P], [N,P,17],
+    [N,P,17,2], coordinates in the frames' pixels)."""
+    return _draw_batch(frames, pose_scores, keypoint_scores, keypoint_coords, min_pose_score, min_part_score,
+                       nat.DRAW_KEYPOINTS | nat.DRAW_SKELETON)
+
+
+def draw_skeleton_batch(frames, pose_scores, keypoint_scores, keypoint_coords, min_pose_confidence=0.5, min_part_confidence=0.5):
+    """``draw_skeleton`` of every frame of a batch on the GPU (in place, bit-exact); arguments as ``draw_skel_and_kp_batch``."""
+    return _draw_batch(frames, pose_scores, keypoint_scores, keypoint_coords, min_pose_confidence, min_part_confidence,
+                       nat.DRAW_SKELETON)
