@@ -159,6 +159,71 @@ int pn_draw_poses(uint8_t *frames, int n_img, int h, int w, int64_t frame_stride
                   const double *kp_scores, const double *kp_coords, int max_poses, double min_pose_score, double min_part_score,
                   int what, pn_stream_t stream);
 
+/* ---- N2'': baseline JPEG files decoded ON THE DEVICE, bit-exact with cv2.imread / cv2.imdecode(IMREAD_COLOR) (libjpeg-turbo 3.1
+ * with its defaults: jdhuff.c, the accurate integer IDCT of jidctint.c, fancy upsampling of jdsample.c, jdcolor.c YCbCr -> BGR).
+ *
+ * pn_jpeg_parse (host only, no device needed) reads a file's headers into a descriptor and classifies it: PN_JPEG_SUPPORTED
+ * (1- or 3-component YCbCr / grayscale, 8-bit, baseline / extended Huffman, one interleaved scan, sampling factors 1..4 x 1..2 with
+ * integral ratios, EXIF orientation 1 or absent, ending in an EOI) or PN_JPEG_HOST with a PN_JPEG_WHY_* reason; host files are for
+ * cv2 to decode.  The descriptor carries everything the device needs: geometry, quantisation tables (natural order) and the derived
+ * Huffman tables (validated like jpeg_make_d_derived_tbl). */
+enum { PN_JPEG_SUPPORTED = 0, PN_JPEG_HOST = 1 };
+enum {
+    PN_JPEG_WHY_NONE = 0, PN_JPEG_WHY_NOT_JPEG, PN_JPEG_WHY_TRUNCATED, PN_JPEG_WHY_PROGRESSIVE, PN_JPEG_WHY_ARITHMETIC,
+    PN_JPEG_WHY_LOSSLESS, PN_JPEG_WHY_PRECISION, PN_JPEG_WHY_MULTI_SCAN, PN_JPEG_WHY_COMPONENTS, PN_JPEG_WHY_RGB,
+    PN_JPEG_WHY_NO_DHT, PN_JPEG_WHY_EXIF_ORIENTATION, PN_JPEG_WHY_SAMPLING, PN_JPEG_WHY_BAD_TABLE, PN_JPEG_WHY_UNKNOWN
+};
+/* pn_jpeg_decode's per-image status: 0 decoded, 1 skipped (a PN_JPEG_HOST descriptor: its frame is left untouched), < 0 the
+ * descriptor or the entropy-coded data is malformed (its frame is written as zeros; cv2's recovery is not reproduced). */
+enum { PN_JPEG_OK = 0, PN_JPEG_SKIPPED = 1, PN_JPEG_ERR_DESC = -1, PN_JPEG_ERR_NO_END = -2, PN_JPEG_ERR_RESTART = -3,
+       PN_JPEG_ERR_CODE = -4, PN_JPEG_ERR_LENGTH = -5 };
+#define PN_JPEG_MAX_BLOCKS 10 /* blocks per MCU (libjpeg's D_MAX_BLOCKS_IN_MCU) */
+
+typedef struct pn_jpeg_huff {
+    uint16_t lookup[256];  /* next 8 bits -> (code length << 8) | symbol; 0: the code is longer than 8 bits */
+    int32_t maxcode[18];   /* largest code of length l, -1 if none; maxcode[17] is a sentinel */
+    int32_t valoffset[18]; /* huffval index of a code of length l: code + valoffset[l] */
+    uint8_t huffval[256];
+} pn_jpeg_huff;
+
+typedef struct pn_jpeg_comp {
+    int32_t h, v;            /* sampling factors as coded in the MCU (1 x 1 for a single-component scan) */
+    int32_t hr, vr;          /* upsampling ratios max_h / h, max_v / v */
+    int32_t dc, ac;          /* pn_jpeg_desc.huff slots */
+    int32_t bw, bh;          /* coefficient plane size in blocks (MCU-padded) */
+    int32_t dw, dh;          /* downsampled_width / downsampled_height */
+} pn_jpeg_comp;
+
+typedef struct pn_jpeg_desc {
+    int32_t kind, why;       /* PN_JPEG_SUPPORTED | PN_JPEG_HOST, PN_JPEG_WHY_* */
+    int32_t height, width, ncomp;
+    int32_t mcus_x, mcus_y, blocks_per_mcu;
+    int32_t restart_interval; /* MCUs per restart interval (the whole scan when the file has no DRI) */
+    int32_t n_segments;       /* restart intervals in the scan */
+    int64_t file_offset;      /* set by the caller: byte offset of the file in pn_jpeg_decode's byte arena */
+    int64_t file_bytes;
+    int64_t scan_offset;      /* first entropy-coded byte, from the start of the file */
+    pn_jpeg_comp comp[3];     /* in frame (SOF) order: Y, Cb, Cr */
+    uint8_t mcu_comp[PN_JPEG_MAX_BLOCKS], mcu_bx[PN_JPEG_MAX_BLOCKS], mcu_by[PN_JPEG_MAX_BLOCKS], pad[2];
+    int16_t quant[3][64];     /* per component, natural order (libjpeg's ISLOW_MULT_TYPE) */
+    pn_jpeg_huff huff[4];
+} pn_jpeg_desc;
+
+/* Parse the headers of one file (HOST pointers).  PN_OK whatever the classification; PN_ERR_ARG for null pointers. */
+int pn_jpeg_parse(const uint8_t *file_host, int64_t nbytes, pn_jpeg_desc *desc_host);
+/* Device workspace (bytes, 256-byte aligned base) pn_jpeg_decode needs for up to n_img files of together at most arena_bytes
+ * bytes, none larger than max_h x max_w. */
+int pn_jpeg_workspace(int n_img, int64_t arena_bytes, int max_h, int max_w, size_t *bytes_host);
+/* Decode n_img files at once.  files: device byte arena (file i at descs[i].file_offset, arena_bytes in all); descs: DEVICE array
+ * of pn_jpeg_parse's descriptors with file_offset filled in.  Frame i is written as uint8 BGR HWC at its own size, contiguous
+ * from frames + i * frame_stride (frame_stride >= 3 * max_h * max_w); nothing else in a row and nothing outside the frames is
+ * written, and no byte outside a file's range is read, whatever the file contains.  frame_hw (optional, device int32 [n_img, 2])
+ * receives each decoded frame's (h, w), (0, 0) for the others; status: device int32 [n_img], PN_JPEG_OK / _SKIPPED / < 0.  The
+ * launch geometry depends only on the arguments, not on the descriptors' contents, so the call can be captured in a CUDA graph. */
+int pn_jpeg_decode(const uint8_t *files, int64_t arena_bytes, const pn_jpeg_desc *descs, int n_img, int max_h, int max_w,
+                   uint8_t *frames, int64_t frame_stride, int *frame_hw, void *workspace, size_t ws_bytes, int *status,
+                   pn_stream_t stream);
+
 /* ---- Whole-network plan: mobilenet_v1.py:130-162 (MobileNetV1.__init__/forward) --------------------
  * The layer table is computed by the caller (posenet/models/mobilenet_v1.py mirrors
  * _to_output_strided_layers, mobilenet_v1.py:8-39) and passed in explicitly. */

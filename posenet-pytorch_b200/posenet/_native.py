@@ -17,6 +17,11 @@ NUM_PARTS, NUM_EDGES, HEAD_CHANNELS, HEAD_ROWS = 17, 16, 115, 128
 ABI_VERSION = 5
 PLAN_UNFUSED = 1
 DRAW_KEYPOINTS, DRAW_SKELETON = 1, 2
+JPEG_SUPPORTED, JPEG_HOST = 0, 1
+JPEG_WHY = {name: i for i, name in enumerate((
+    "none", "not_jpeg", "truncated", "progressive", "arithmetic", "lossless", "precision", "multi_scan", "components", "rgb",
+    "no_dht", "exif_orientation", "sampling", "bad_table", "unknown"))}
+JPEG_OK, JPEG_SKIPPED = 0, 1
 
 
 class NativeError(RuntimeError):
@@ -42,6 +47,23 @@ class NetDesc(C.Structure):
     _fields_ = [("dtype", C.c_int), ("n", C.c_int), ("h", C.c_int), ("w", C.c_int), ("input_u8", C.c_int),
                 ("num_layers", C.c_int), ("layers", Layer * 16), ("head_w", C.c_void_p), ("head_b", C.c_void_p),
                 ("flags", C.c_int)]
+
+
+class JpegHuff(C.Structure):
+    _fields_ = [("lookup", C.c_uint16 * 256), ("maxcode", C.c_int32 * 18), ("valoffset", C.c_int32 * 18), ("huffval", C.c_uint8 * 256)]
+
+
+class JpegComp(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("h", "v", "hr", "vr", "dc", "ac", "bw", "bh", "dw", "dh")]
+
+
+class JpegDesc(C.Structure):
+    """pn_jpeg_desc: one file's headers as pn_jpeg_parse leaves them (file_offset is the caller's)."""
+    _fields_ = [(n, C.c_int32) for n in ("kind", "why", "height", "width", "ncomp", "mcus_x", "mcus_y", "blocks_per_mcu",
+                                         "restart_interval", "n_segments")] + \
+               [("file_offset", C.c_int64), ("file_bytes", C.c_int64), ("scan_offset", C.c_int64), ("comp", JpegComp * 3),
+                ("mcu_comp", C.c_uint8 * 10), ("mcu_bx", C.c_uint8 * 10), ("mcu_by", C.c_uint8 * 10), ("pad", C.c_uint8 * 2),
+                ("quant", (C.c_int16 * 64) * 3), ("huff", JpegHuff * 4)]
 
 
 _SIGNATURES = {
@@ -75,6 +97,10 @@ _SIGNATURES = {
     "pn_scale_keypoint_coords": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_double, C.c_double, C.c_void_p]),
     "pn_draw_poses": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_int, C.c_double, C.c_double, C.c_int, C.c_void_p]),
+    "pn_jpeg_parse": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(JpegDesc)]),
+    "pn_jpeg_workspace": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
+    "pn_jpeg_decode": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_void_p,
+                                 C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
     "pn_plan_query": (C.c_int, [C.POINTER(NetDesc), C.POINTER(C.c_size_t), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "pn_plan_create": (C.c_int, [C.POINTER(NetDesc), C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p)]),
     "pn_plan_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -15,17 +15,51 @@ A directory of images of DIFFERENT sizes (``benchmark.py:24-29`` pre-processes e
     pipe = posenet.BatchPipeline(model, 64, 720, 1280, mixed=True, source_coords=True, min_pose_score=0.25)
     for records in pipe.run((b, shapes) for b, _, shapes in stream.batches()):
         ...                                                       # coordinates already in each file's own pixel grid
+
+JPEG files decoded on the GPU instead (``posenet.jpeg``; the records are identical, the host only reads and parses files):
+
+    stream = posenet.ImageStream(paths, batch=64, decode="gpu")
+    pipe = posenet.BatchPipeline(model, 64, stream.height, stream.width, jpeg=True, min_pose_score=0.25)
+    for *records, status in pipe.run(b for b, _ in stream.batches()):
+        ...                                                       # status[i]: 0 GPU, 1 decoded by cv2 on the host, < 0 malformed
 """
 import concurrent.futures
+import ctypes as C
 import os
+import threading
 
 import cv2
 import numpy as np
 import torch
 
+from posenet import _native as nat
+
+
+class EncodedBatch:
+    """One batch of files as ``ImageStream(decode="gpu")`` hands it to ``BatchPipeline(jpeg=True)``: the bytes of the files the GPU
+    decodes packed into a pinned byte arena (``arena[:used]``), their descriptors (``descs``, pinned uint8, one pn_jpeg_desc per
+    row; rows the GPU does not decode are marked host), and the frames cv2 decoded on the host (``raw`` rows ``host_rows``)."""
+
+    def __init__(self, arena, descs, raw, batch):
+        self.arena, self.descs, self.raw, self.batch = arena, descs, raw, batch
+        self.used = 0
+        self.host_rows = []
+        self.shapes = [None] * batch
+        self.n_valid = 0
+        self.lock = threading.Lock()
+
+    def reset(self, n_valid):
+        self.used = 0
+        self.host_rows = []
+        self.shapes = [None] * self.batch
+        self.n_valid = n_valid
+        host = nat.JpegDesc()
+        host.kind = nat.JPEG_HOST
+        self.descs.numpy()[:] = np.frombuffer(bytes((nat.JpegDesc * self.batch)(*([host] * self.batch))), np.uint8)
+
 
 class ImageStream:
-    def __init__(self, paths, batch, height=None, width=None, workers=None, slots=4, keep=2, pinned=None, mixed=False):
+    def __init__(self, paths, batch, height=None, width=None, workers=None, slots=4, keep=2, pinned=None, mixed=False, decode="cv2"):
         """``mixed``: the files may have different sizes (each at most ``height`` x ``width``); a batch row then holds its frame
         contiguously at the frame's own size and ``batches()`` also yields the list of ``(h, w)`` -- the input format of a
         ``BatchPipeline(..., mixed=True)``, which resizes every frame on the GPU like ``_process_input`` (utils.py:13-26) does.
@@ -33,7 +67,13 @@ class ImageStream:
         ``slots`` batch buffers rotate.  A buffer handed out by ``batches()`` stays valid while the consumer takes ``keep``
         further batches and is decoded into again when it asks for the one after that; the remaining ``slots - 1 - keep``
         batches decode ahead on the thread pool.  ``BatchPipeline.run`` (depth d) copies batch i to the device asynchronously
-        and only blocks on it after taking batch i + d, so ``keep >= d`` is what makes the reuse safe (defaults: d = 2)."""
+        and only blocks on it after taking batch i + d, so ``keep >= d`` is what makes the reuse safe (defaults: d = 2).
+
+        ``decode="gpu"``: the workers only read each file into the batch's pinned byte arena (``batch * height * width * 3``
+        bytes, the size of a decoded batch) and parse its headers; ``batches()`` yields an ``EncodedBatch`` in place of the
+        uint8 tensor, for a ``BatchPipeline(..., jpeg=True)`` to decode on the GPU.  Files the GPU does not decode (not baseline
+        JPEG, EXIF-rotated, ...; ``posenet.jpeg``) or that do not fit the arena's remaining space are decoded by cv2.imread into
+        their row of a pinned side buffer.  Size checks and errors are those of ``decode="cv2"``."""
         self.paths = list(paths)
         assert self.paths, "no image files"
         self.batch = int(batch)
@@ -55,6 +95,15 @@ class ImageStream:
             self._bufs.append(t.pin_memory() if pinned else t)
         self._views = [b.numpy() for b in self._bufs]
         self._shapes = [[None] * self.batch for _ in self._bufs]
+        assert decode in ("cv2", "gpu"), "decode is 'cv2' or 'gpu'"
+        self.decode = decode
+        self._enc = []
+        if decode == "gpu":
+            for b in self._bufs:
+                arena = torch.empty(b.numel(), dtype=torch.uint8)
+                descs = torch.empty(self.batch * C.sizeof(nat.JpegDesc), dtype=torch.uint8)
+                self._enc.append(EncodedBatch(arena.pin_memory() if pinned else arena, descs.pin_memory() if pinned else descs, b,
+                                              self.batch))
 
     def __len__(self):
         return (len(self.paths) + self.batch - 1) // self.batch
@@ -63,6 +112,42 @@ class ImageStream:
         """Number of real images in every batch (the last one may be partial; its tail rows are zero images)."""
         n = len(self.paths)
         return [min(self.batch, n - i) for i in range(0, n, self.batch)]
+
+    def _check_size(self, path, h, w):
+        if self.mixed:
+            if h > self.height or w > self.width:
+                raise ValueError("%s is %dx%d, larger than the stream's %dx%d frames" % (path, w, h, self.width, self.height))
+        elif (h, w) != (self.height, self.width):
+            raise ValueError("%s is %dx%d, the stream carries %dx%d frames (mixed=True accepts different sizes)" % (
+                path, w, h, self.width, self.height))
+
+    def _load_encoded(self, path, enc, row):
+        """Read one file into the arena and parse it; cv2 decodes it into its raw row when the GPU cannot."""
+        try:
+            with open(path, "rb") as f:
+                size = os.fstat(f.fileno()).st_size
+                with enc.lock:
+                    off = enc.used
+                    fits = off + size <= enc.arena.numel()
+                    if fits:
+                        enc.used += size
+                view = enc.arena.numpy()[off:off + size] if fits else None
+                n = f.readinto(memoryview(view)) if fits else -1
+        except OSError:
+            raise IOError("Image file not found or unreadable: %s" % path)
+        if fits and n == size:
+            d = nat.JpegDesc()
+            nat.check(nat.load().pn_jpeg_parse(view.ctypes.data, size, C.byref(d)), "pn_jpeg_parse")
+            if d.kind == nat.JPEG_SUPPORTED:
+                self._check_size(path, d.height, d.width)
+                d.file_offset = off
+                k = C.sizeof(nat.JpegDesc)
+                enc.descs.numpy()[row * k:(row + 1) * k] = np.frombuffer(bytes(d), np.uint8)
+                enc.shapes[row] = (d.height, d.width)
+                return
+        self._load(path, enc.raw.numpy()[row], enc.shapes, row)
+        with enc.lock:
+            enc.host_rows.append(row)
 
     def _load(self, path, dst, shapes, row):
         img = cv2.imread(path)
@@ -89,6 +174,10 @@ class ImageStream:
                 buf, shapes = self._views[bi % len(self._views)], self._shapes[bi % len(self._views)]
                 lo = starts[bi]
                 hi = min(n, lo + self.batch)
+                if self.decode == "gpu":
+                    enc = self._enc[bi % len(self._enc)]
+                    enc.reset(hi - lo)
+                    return [ex.submit(self._load_encoded, self.paths[i], enc, i - lo) for i in range(lo, hi)]
                 if hi - lo < self.batch:
                     buf[hi - lo:] = 0
                 return [ex.submit(self._load, self.paths[i], buf[i - lo], shapes, i - lo) for i in range(lo, hi)]
@@ -103,7 +192,11 @@ class ImageStream:
                 if nxt < len(starts):
                     pending[nxt] = launch(nxt)
                 nv = min(self.batch, n - starts[bi])
-                if self.mixed:
+                if self.decode == "gpu":
+                    enc = self._enc[bi % len(self._enc)]
+                    enc.host_rows.sort()
+                    yield (enc, nv, list(enc.shapes[:nv])) if self.mixed else (enc, nv)
+                elif self.mixed:
                     yield self._bufs[bi % len(self._bufs)], nv, list(self._shapes[bi % len(self._bufs)][:nv])
                 else:
                     yield self._bufs[bi % len(self._bufs)], nv

@@ -26,7 +26,7 @@ from posenet.decode_multi import decode_multiple_poses_batch, split_pose_records
 
 class BatchPipeline:
     def __init__(self, model, batch, height, width, depth=2, use_graph=True, output_stride=None, scale_factor=1.0,
-                 source_coords=False, mixed=False, gather=False, group=None, overlay=None, **decode_kw):
+                 source_coords=False, mixed=False, gather=False, group=None, overlay=None, jpeg=False, **decode_kw):
         """``height`` x ``width``: size of the uint8 frames handed to ``submit`` (``mixed=True``: the LARGEST frame; each
         frame of a batch then comes with its own size).  The network runs at ``valid_resolution(width * scale_factor,
         height * scale_factor)`` (utils.py:7-10); frames of any other size go through the bit-exact cv2 resize
@@ -40,7 +40,11 @@ class BatchPipeline:
         ``overlay=(min_pose_score, min_part_score)``: the step also draws ``draw_skel_and_kp`` (image_demo.py:53) on the submitted
         frames at their own size, on the device (``pn_draw_poses``, bit-exact with cv2), and copies them back after the records;
         ``result`` then returns the frames as a fifth item.  Frames that are resized need ``source_coords=True`` (the overlay is
-        drawn in their coordinates).  With ``gather``, the frames stay on their rank."""
+        drawn in their coordinates).  With ``gather``, the frames stay on their rank.
+        ``jpeg``: ``submit`` takes the ``EncodedBatch`` of an ``ImageStream(..., decode="gpu")``.  The host-to-device copy carries
+        the bytes of the files in use, their descriptors and the rows cv2 decoded on the host; ``pn_jpeg_decode`` writes the
+        frames into the step's input buffer (same layout as the uint8 batches) on the compute stream, just before the step.
+        ``result`` appends the int32 decode status ``[batch]`` as its last item (0 GPU, 1 host, < 0 malformed: a zero frame)."""
         nat.require_device()
         assert depth >= 1
         self.model, self.batch, self.h, self.w = model, int(batch), int(height), int(width)
@@ -85,6 +89,13 @@ class BatchPipeline:
                          shapes=None,
                          copied=torch.cuda.Event(), done=torch.cuda.Event(), out=torch.cuda.Event(), graph=None, busy=False)
                 self.slots.append(s)
+            self.jpeg = bool(jpeg)
+            if self.jpeg:
+                from posenet.jpeg import Decoder
+                for s in self.slots:
+                    s["dec"] = Decoder(self.batch, s["x"].numel(), self.h, self.w, dev)
+                    s["status_host"] = torch.zeros(self.batch, dtype=torch.int32).pin_memory()
+                    s["h2d_bytes"] = 0
             self.h2d_bytes_per_batch = self.slots[0]["x"].numel()
             self.d2h_bytes_per_batch = (self.world if self.collect_all else 1) * nrec * 8
             if self.overlay:
@@ -150,6 +161,24 @@ class BatchPipeline:
             nat.check(lib.pn_resize_u8(base_in + i * row, n, h, w, self.th, self.tw, base_out + i * out_row, st), "pn_resize_u8")
             i += n
 
+    def _copy_encoded(self, s, enc, shapes):
+        """H2D part of a jpeg=True step (on the h2d stream): file bytes in use, descriptors, host-decoded rows."""
+        dec, x = s["dec"], s["x"].view(self.batch, -1)
+        n = 0
+        if enc.used:
+            dec.arena[:enc.used].copy_(enc.arena[:enc.used], non_blocking=True)
+            n += enc.used
+        dec.descs.copy_(enc.descs, non_blocking=True)
+        n += enc.descs.numel()
+        raw = enc.raw.view(self.batch, -1)
+        for i in enc.host_rows:
+            used = shapes[i][0] * shapes[i][1] * 3 if self.mixed else x.shape[1]
+            x[i, :used].copy_(raw[i, :used], non_blocking=True)
+            n += used
+        if not self.mixed and enc.n_valid < self.batch:
+            x[enc.n_valid:].zero_()                                    # rows without a file decode as black frames
+        s["h2d_bytes"] = n
+
     def submit(self, host_batch, shapes=None):
         """Enqueue one batch (uint8 [batch,h,w,3], ideally pinned).  Returns a ticket for ``result``; if the slot is
         still in flight its previous result must have been collected.
@@ -159,7 +188,16 @@ class BatchPipeline:
         (``len(shapes) < batch``) decode as black frames."""
         s = self.slots[self._next]
         assert not s["busy"], "pipeline full: collect result() of the oldest ticket first"
-        assert host_batch.numel() == s["x"].numel() and host_batch.dtype == torch.uint8
+        enc = None
+        if self.jpeg:
+            from posenet.ingest import EncodedBatch
+            assert isinstance(host_batch, EncodedBatch), "jpeg=True: submit the EncodedBatch of an ImageStream(decode='gpu')"
+            assert host_batch.arena.numel() <= s["dec"].arena_bytes and host_batch.batch == self.batch
+            enc = host_batch
+            if self.mixed and shapes is None:
+                shapes = list(enc.shapes[:enc.n_valid])
+        else:
+            assert host_batch.numel() == s["x"].numel() and host_batch.dtype == torch.uint8
         if self.mixed:
             assert shapes is not None and len(shapes) <= self.batch, "mixed=True: pass the (h, w) of every frame"
             shapes = [(int(h), int(w)) for h, w in shapes]
@@ -179,9 +217,13 @@ class BatchPipeline:
         with torch.cuda.device(self.dev):
             with torch.cuda.stream(self.h2d):
                 self.h2d.wait_event(s["done"])              # the previous use of this slot's input buffer has finished
-                if self.overlay:
-                    self.h2d.wait_event(s["out"])           # ... and its drawn frames have been copied back
-                if self.mixed and shapes:
+                if self.overlay or self.jpeg:
+                    self.h2d.wait_event(s["out"])           # ... and its drawn frames / decode status have been copied back
+                if enc is not None:
+                    self._copy_encoded(s, enc, shapes)
+                    if self.mixed:
+                        s["scales"].copy_(sc, non_blocking=True)
+                elif self.mixed and shapes:
                     used = max(h * w * 3 for h, w in shapes)                      # one strided copy of the bytes in use
                     s["x"].view(self.batch, -1)[:len(shapes), :used].copy_(host_batch.view(self.batch, -1)[:len(shapes), :used],
                                                                           non_blocking=True)
@@ -194,6 +236,8 @@ class BatchPipeline:
             with torch.cuda.stream(self.compute):
                 self.compute.wait_event(s["copied"])
                 self.compute.wait_event(s["out"])           # the previous records of this slot have left the device
+                if enc is not None:
+                    s["dec"].decode(s["x"], self.h * self.w * 3)
                 if self.mixed:
                     if len(shapes) < self.batch:
                         s["xr"][len(shapes):].zero_()
@@ -215,6 +259,8 @@ class BatchPipeline:
                                                                                    non_blocking=True)
                 elif self.overlay and not self.mixed:
                     s["frames_host"].copy_(s["x"], non_blocking=True)
+                if enc is not None:
+                    s["status_host"].copy_(s["dec"].status, non_blocking=True)
                 s["out"].record(self.d2h)
         s["busy"] = True
         ticket = self._next
@@ -224,7 +270,8 @@ class BatchPipeline:
     def result(self, ticket, copy=True, source_coords=None, gathered=False):
         """Block until the ticket's records are on the host; returns the reference's 4-tuple for this rank's batch
         (numpy float64: [batch,P], [batch,P,17], [batch,P,17,2], [batch,P,17,2]).  With ``overlay``, a fifth item holds this
-        rank's drawn frames: uint8 [batch,h,w,3], or in mixed mode a list of [h_i,w_i,3] arrays, one per submitted frame.  ``gathered=True`` (rank 0 of a
+        rank's drawn frames: uint8 [batch,h,w,3], or in mixed mode a list of [h_i,w_i,3] arrays, one per submitted frame.  With
+        ``jpeg``, the last item is the int32 decode status [batch].  ``gathered=True`` (rank 0 of a
         ``gather=True`` pipeline): the records of ALL ranks' batches instead, leading dimension ``world * batch`` (rank-major).
         ``source_coords`` is a construction-time option (the scaling runs on the device); passing a different value here is an
         error."""
@@ -246,6 +293,8 @@ class BatchPipeline:
                 frames = ([f.copy() for f in fr] if copy else fr,)
             else:
                 frames = (fr.copy() if copy else fr,)
+        if self.jpeg:
+            frames = frames + (s["status_host"].numpy().copy(),)
         if not gathered:
             own = flat[self.rank * self.nrec:(self.rank + 1) * self.nrec] if self.collect_all else flat
             return split_pose_records(own, self.batch, self.P) + frames
