@@ -224,6 +224,28 @@ int pn_jpeg_decode(const uint8_t *files, int64_t arena_bytes, const pn_jpeg_desc
                    uint8_t *frames, int64_t frame_stride, int *frame_hw, void *workspace, size_t ws_bytes, int *status,
                    pn_stream_t stream);
 
+/* ---- N5: image_demo.py:57 cv2.imwrite of the drawn frames: baseline JPEG files encoded ON THE DEVICE, bit-exact with
+ * cv2.imencode(".jpg", frame, params) (libjpeg-turbo 3.1 as cv2 4.13 calls it: jccolor.c, jcsample.c, the accurate integer FDCT
+ * of jfdctint.c, the Annex K Huffman tables, JFIF headers; no optimised tables, not progressive).
+ *
+ * sampling: cv2's IMWRITE_JPEG_SAMPLING_FACTOR_* value (0x411111, 0x221111, 0x211111, 0x121111, 0x111111); restart_interval:
+ * MCUs per interval, 0 for none (cv2's IMWRITE_JPEG_RST_INTERVAL).
+ *
+ * pn_jpeg_encode_bound (host only): a true worst case of one file of h x w (every block at its largest Huffman code length,
+ * every byte stuffed, markers and headers); 0 for 0 x 0. */
+int pn_jpeg_encode_bound(int h, int w, int sampling, int restart_interval, int64_t *bytes_host);
+/* Device workspace (bytes, 256-byte aligned base) pn_jpeg_encode needs for up to n_img frames of at most max_h x max_w. */
+int pn_jpeg_encode_workspace(int n_img, int max_h, int max_w, int sampling, int restart_interval, size_t *bytes_host);
+/* Encode n_img frames at once.  frames: device uint8 BGR HWC, frame i from frames + i * frame_stride (>= 3 * max_h * max_w), rows
+ * of w_i * 3 bytes; frame_hw: device int32 [n_img, 2] with each frame's (h_i, w_i), a size outside 1..max_h x 1..max_w giving an
+ * empty file, or NULL for max_h x max_w everywhere.  quality: 0..100 (0 behaves like 1, as in cv2).  out: device bytes, packed:
+ * file i is out[out_offsets[i] .. out_offsets[i + 1]) with out_offsets device int64 [n_img + 1]; out_capacity must be at least
+ * n_img * pn_jpeg_encode_bound(max_h, max_w, ..) and nothing at or past out_offsets[n_img] is written.  The frames are only read.
+ * The launch geometry depends only on the capacity, so the call can be captured in a CUDA graph (quality is fixed then). */
+int pn_jpeg_encode(const uint8_t *frames, int n_img, int max_h, int max_w, int64_t frame_stride, const int *frame_hw, int quality,
+                   int sampling, int restart_interval, uint8_t *out, int64_t out_capacity, int64_t *out_offsets, void *workspace,
+                   size_t ws_bytes, pn_stream_t stream);
+
 /* ---- Whole-network plan: mobilenet_v1.py:130-162 (MobileNetV1.__init__/forward) --------------------
  * The layer table is computed by the caller (posenet/models/mobilenet_v1.py mirrors
  * _to_output_strided_layers, mobilenet_v1.py:8-39) and passed in explicitly. */

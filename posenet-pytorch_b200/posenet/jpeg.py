@@ -1,11 +1,14 @@
-"""Baseline JPEG decode on the GPU, bit-exact with ``cv2.imdecode(buf, cv2.IMREAD_COLOR)`` (``pn_jpeg_parse`` / ``pn_jpeg_decode``).
+"""Baseline JPEG decode on the GPU, bit-exact with ``cv2.imdecode(buf, cv2.IMREAD_COLOR)`` (``pn_jpeg_parse`` / ``pn_jpeg_decode``),
+and encode, bit-exact with ``cv2.imencode(".jpg", frame, params)`` (``pn_jpeg_encode``).
 
     frames, status = posenet.imdecode_batch(buffers)                  # files of one size: CUDA uint8 [N, h, w, 3]
     rows, status, shapes = posenet.imdecode_batch(buffers)            # sizes differ: row i holds frame i at its own size
 
 ``status[i]``: 0 decoded on the GPU, 1 decoded by cv2 on the host (progressive, arithmetic-coded, 12-bit, CMYK / RGB-coded,
 EXIF-rotated or truncated files, anything the parser does not know) and uploaded, < 0 the file's entropy-coded data is
-malformed: its frame is zeros (cv2 decodes such files with a warning; its recovery is not reproduced)."""
+malformed: its frame is zeros (cv2 decodes such files with a warning; its recovery is not reproduced).
+
+    files = posenet.imencode_batch(frames, [cv2.IMWRITE_JPEG_QUALITY, 90])   # list of bytes, one per frame"""
 import ctypes as C
 
 import cv2
@@ -92,3 +95,103 @@ def imdecode_batch(buffers, device=None):
         return rows.view(len(bufs), H, W, 3), status
     return rows, status, shapes
 
+
+
+# ---- encode: pn_jpeg_encode_bound / pn_jpeg_encode -----------------------------------------------------------------------------------
+SAMPLINGS = (0x411111, 0x221111, 0x211111, 0x121111, 0x111111)     # cv2.IMWRITE_JPEG_SAMPLING_FACTOR_411 .. _444
+
+
+def encode_options(params=()):
+    """(quality, sampling, restart_interval) of a cv2 ``imencode`` params list, with cv2's defaults (95, 4:2:0, none) and its
+    clamping of the quality to 0..100.  ValueError for anything the device encoder does not do (optimised tables, progressive,
+    separate luma / chroma quality, other formats' flags): the caller can use cv2 for those."""
+    params = [int(p) for p in params]
+    if len(params) % 2:
+        raise ValueError("imencode params are (flag, value) pairs: %r" % (params,))
+    quality, sampling, rst = 95, cv2.IMWRITE_JPEG_SAMPLING_FACTOR_420, 0
+    for flag, value in zip(params[::2], params[1::2]):
+        if flag == cv2.IMWRITE_JPEG_QUALITY:
+            quality = min(max(value, 0), 100)
+        elif flag == cv2.IMWRITE_JPEG_SAMPLING_FACTOR:
+            if value not in SAMPLINGS:
+                raise ValueError("IMWRITE_JPEG_SAMPLING_FACTOR 0x%x is not one of cv2's five" % value)
+            sampling = value
+        elif flag == cv2.IMWRITE_JPEG_RST_INTERVAL:
+            rst = min(max(value, 0), 65535)
+        elif flag in (cv2.IMWRITE_JPEG_OPTIMIZE, cv2.IMWRITE_JPEG_PROGRESSIVE) and value == 0:
+            pass
+        else:
+            raise ValueError("imencode param %d = %d is not supported on the device (use cv2.imencode)" % (flag, value))
+    return quality, sampling, rst
+
+
+def encode_bound(h, w, sampling=cv2.IMWRITE_JPEG_SAMPLING_FACTOR_420, restart_interval=0):
+    """pn_jpeg_encode_bound: the largest file an h x w frame can encode to."""
+    n = C.c_int64()
+    nat.check(nat.load().pn_jpeg_encode_bound(int(h), int(w), int(sampling), int(restart_interval), C.byref(n)),
+              "pn_jpeg_encode_bound")
+    return n.value
+
+
+class Encoder:
+    """Device buffers for ``pn_jpeg_encode`` at a fixed capacity: ``batch`` frames of at most ``max_h`` x ``max_w``, encoded with
+    the cv2 ``params``.  ``encode`` enqueues on the current stream; file i is then ``out[offsets[i]:offsets[i + 1]]``."""
+
+    def __init__(self, batch, max_h, max_w, params=(), device=None):
+        self.quality, self.sampling, self.rst = encode_options(params)
+        self.batch, self.max_h, self.max_w = int(batch), int(max_h), int(max_w)
+        dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        n = C.c_size_t()
+        nat.check(nat.load().pn_jpeg_encode_workspace(self.batch, self.max_h, self.max_w, self.sampling, self.rst, C.byref(n)),
+                  "pn_jpeg_encode_workspace")
+        self.ws = torch.empty(n.value, dtype=torch.uint8, device=dev)
+        self.capacity = self.batch * encode_bound(self.max_h, self.max_w, self.sampling, self.rst)
+        self.out = torch.empty(self.capacity, dtype=torch.uint8, device=dev)
+        self.offsets = torch.zeros(self.batch + 1, dtype=torch.int64, device=dev)
+
+    def encode(self, frames, frame_stride, frame_hw=None):
+        """Enqueue pn_jpeg_encode of ``frames`` (frame i from byte ``i * frame_stride``; ``frame_hw``: CUDA int32 [batch, 2]
+        per-frame sizes, or None for max_h x max_w everywhere) into ``self.out`` / ``self.offsets``."""
+        nat.check(nat.load().pn_jpeg_encode(
+            C.c_void_p(frames.data_ptr()), self.batch, self.max_h, self.max_w, int(frame_stride),
+            C.c_void_p(frame_hw.data_ptr()) if frame_hw is not None else None, self.quality, self.sampling, self.rst,
+            C.c_void_p(self.out.data_ptr()), self.capacity, C.c_void_p(self.offsets.data_ptr()), C.c_void_p(self.ws.data_ptr()),
+            self.ws.numel(), nat.stream_ptr()), "pn_jpeg_encode")
+
+    def files(self):
+        """Synchronise and copy the files of the last ``encode`` back (the bytes in use only): a list of ``bytes``, one per
+        frame."""
+        off = self.offsets.cpu().numpy()
+        data = self.out[:int(off[-1])].cpu().numpy()
+        return [data[off[i]:off[i + 1]].tobytes() for i in range(self.batch)]
+
+
+def imencode_batch(frames, params=(), shapes=None):
+    """Encode every frame on the GPU; returns a list of ``bytes``, file i equal to ``cv2.imencode(".jpg", frame_i, params)[1]``.
+    ``frames``: CUDA uint8 [N, h, w, 3] (BGR), or with ``shapes`` the rows [N, H * W * 3] and sizes ``imdecode_batch`` returns
+    (frame i stored contiguously from the start of row i at its own size; a (0, 0) frame gives an empty file).  ``params``: cv2's
+    flat list; IMWRITE_JPEG_QUALITY, _SAMPLING_FACTOR and _RST_INTERVAL, and OPTIMIZE / PROGRESSIVE at 0.  Anything else raises
+    ValueError (see ``encode_options``)."""
+    encode_options(params)
+    nat.require_device()
+    assert frames.is_cuda and frames.dtype == torch.uint8, "frames: a CUDA uint8 tensor"
+    n = frames.shape[0]
+    hw = None
+    if shapes is None:
+        assert frames.dim() == 4 and frames.shape[3] == 3, "frames: [N, h, w, 3] (or rows with shapes)"
+        frames = frames.contiguous()
+        H, W = int(frames.shape[1]), int(frames.shape[2])
+        stride = H * W * 3
+    else:
+        shapes = [(int(h), int(w)) for h, w in shapes]
+        assert len(shapes) == n, "one (h, w) per row"
+        H, W = max(max(h for h, _ in shapes), 1), max(max(w for _, w in shapes), 1)
+        frames = frames.reshape(n, -1)
+        assert frames.stride(1) == 1 and all(h * w * 3 <= frames.shape[1] for h, w in shapes)
+        stride = frames.stride(0)
+        assert stride >= H * W * 3, "rows shorter than the largest frame's H * W * 3"
+        hw = torch.tensor(shapes, dtype=torch.int32).to(frames.device)
+    with torch.cuda.device(frames.device):
+        enc = Encoder(n, H, W, params, frames.device)
+        enc.encode(frames, stride, hw)
+        return enc.files()

@@ -9,7 +9,8 @@ This is the batched form of what the reference's ``benchmark.py:32-44`` does per
     for pose_scores, keypoint_scores, keypoint_coords, pose_offsets in pipe.run(batches):   # pinned uint8 [64,513,513,3]
         ...
 
-Options on top of that: ``source_coords=True`` maps the keypoint coordinates back to the submitted frames ON THE DEVICE
+Options on top of that (``overlay=`` draws the poses on the frames, ``encode=`` returns them as JPEG files, ``jpeg=True``
+takes JPEG files in): ``source_coords=True`` maps the keypoint coordinates back to the submitted frames ON THE DEVICE
 (``image_demo.py:50``), ``mixed=True`` accepts frames of different sizes in one batch (every file of a directory
 pre-processed at its own size, ``benchmark.py:24-29``), ``gather=True`` all-gathers the records of every rank's shard over
 NCCL inside the step (one process per GPU, ``posenet.sharding``).
@@ -26,7 +27,7 @@ from posenet.decode_multi import decode_multiple_poses_batch, split_pose_records
 
 class BatchPipeline:
     def __init__(self, model, batch, height, width, depth=2, use_graph=True, output_stride=None, scale_factor=1.0,
-                 source_coords=False, mixed=False, gather=False, group=None, overlay=None, jpeg=False, **decode_kw):
+                 source_coords=False, mixed=False, gather=False, group=None, overlay=None, jpeg=False, encode=None, **decode_kw):
         """``height`` x ``width``: size of the uint8 frames handed to ``submit`` (``mixed=True``: the LARGEST frame; each
         frame of a batch then comes with its own size).  The network runs at ``valid_resolution(width * scale_factor,
         height * scale_factor)`` (utils.py:7-10); frames of any other size go through the bit-exact cv2 resize
@@ -44,7 +45,13 @@ class BatchPipeline:
         ``jpeg``: ``submit`` takes the ``EncodedBatch`` of an ``ImageStream(..., decode="gpu")``.  The host-to-device copy carries
         the bytes of the files in use, their descriptors and the rows cv2 decoded on the host; ``pn_jpeg_decode`` writes the
         frames into the step's input buffer (same layout as the uint8 batches) on the compute stream, just before the step.
-        ``result`` appends the int32 decode status ``[batch]`` as its last item (0 GPU, 1 host, < 0 malformed: a zero frame)."""
+        ``result`` appends the int32 decode status ``[batch]`` as its last item (0 GPU, 1 host, < 0 malformed: a zero frame).
+        ``encode``: a cv2 ``imencode`` params list (``[]`` for cv2's defaults; needs ``overlay``).  The step's graph also encodes
+        the drawn frames as JPEG files (``pn_jpeg_encode``, bit-exact with ``cv2.imencode(".jpg", frame, encode)``), and the
+        in-graph device-to-host copy carries the files' offsets instead of the frames.  ``result`` copies exactly the bytes in use
+        on a stream of its own (the offsets are only known on the host then) and returns a list of ``bytes`` as the fifth item
+        instead of the frames: one per submitted frame in mixed mode, ``batch`` otherwise.  Params the device encoder does not
+        do raise ValueError here."""
         nat.require_device()
         assert depth >= 1
         self.model, self.batch, self.h, self.w = model, int(batch), int(height), int(width)
@@ -58,6 +65,11 @@ class BatchPipeline:
         self.overlay = None if overlay is None else (float(overlay[0]), float(overlay[1]))
         assert self.overlay is None or self.source_coords or not self.resize, \
             "overlay on resized frames needs source_coords=True (the records must be in the frames' coordinates)"
+        assert encode is None or self.overlay is not None, "encode= encodes the drawn frames: it needs overlay="
+        self.encode = None if encode is None else list(encode)
+        if self.encode is not None:
+            from posenet.jpeg import encode_options
+            encode_options(self.encode)
         self.decode_kw = dict(decode_kw)
         self.P = int(self.decode_kw.get("max_pose_detections", 10))
         dev = model._device()
@@ -83,7 +95,8 @@ class BatchPipeline:
                          rec_host=torch.zeros((self.world if self.collect_all else 1) * nrec, dtype=torch.float64).pin_memory(),
                          scales=torch.ones((self.batch, 2), dtype=torch.float64, device=dev) if self.mixed else None,
                          scales_host=torch.ones((self.batch, 2), dtype=torch.float64).pin_memory() if self.mixed else None,
-                         frames_host=torch.empty((self.batch, self.h, self.w, 3), dtype=torch.uint8).pin_memory() if self.overlay else None,
+                         frames_host=torch.empty((self.batch, self.h, self.w, 3), dtype=torch.uint8).pin_memory()
+                         if self.overlay and self.encode is None else None,
                          hw=torch.zeros((self.batch, 2), dtype=torch.int32, device=dev) if self.overlay and self.mixed else None,
                          hw_host=torch.zeros((self.batch, 2), dtype=torch.int32).pin_memory() if self.overlay and self.mixed else None,
                          shapes=None,
@@ -96,10 +109,22 @@ class BatchPipeline:
                     s["dec"] = Decoder(self.batch, s["x"].numel(), self.h, self.w, dev)
                     s["status_host"] = torch.zeros(self.batch, dtype=torch.int32).pin_memory()
                     s["h2d_bytes"] = 0
+            if self.encode is not None:
+                from posenet.jpeg import Encoder
+                self.files_stream = torch.cuda.Stream(dev)             # result()'s copy of the packed files
+                for s in self.slots:
+                    s["enc"] = Encoder(self.batch, self.h, self.w, self.encode, dev)
+                    s["offsets_host"] = torch.zeros(self.batch + 1, dtype=torch.int64).pin_memory()
+                    s["files_host"] = torch.empty(self.batch * self.h * self.w * 3 // 4, dtype=torch.uint8).pin_memory()
             self.h2d_bytes_per_batch = self.slots[0]["x"].numel()
             self.d2h_bytes_per_batch = (self.world if self.collect_all else 1) * nrec * 8
-            if self.overlay:
+            if self.overlay and self.encode is None:
                 self.d2h_bytes_per_batch += self.slots[0]["x"].numel()         # mixed mode copies only the bytes in use
+            elif self.encode is not None:
+                # the offsets, plus the files: an estimate of a tenth of the frames' raw size (drawn frames at q95 4:2:0 are
+                # 8-12 %); result() copies exactly the bytes in use and records them in last_file_bytes
+                self.d2h_bytes_per_batch += 8 * (self.batch + 1) + self.slots[0]["x"].numel() // 10
+            self.last_file_bytes = 0
             # warm up (plans, workspaces) and capture one graph per slot on the compute stream
             self.compute.wait_stream(torch.cuda.current_stream(dev))
             with torch.cuda.stream(self.compute):
@@ -142,6 +167,8 @@ class BatchPipeline:
                                         C.c_void_p(ks.data_ptr()), C.c_void_p(kc.data_ptr()), self.P, self.overlay[0],
                                         self.overlay[1], nat.DRAW_KEYPOINTS | nat.DRAW_SKELETON, nat.stream_ptr()),
                       "pn_draw_poses")
+            if self.encode is not None:
+                s["enc"].encode(x, self.h * self.w * 3, s["hw"] if self.mixed else None)
 
     def _resize_mixed(self, s, shapes):
         """Per-frame cv2-exact resize of frames stored at their own size (row i of the slot's input buffer holds frame i
@@ -253,7 +280,9 @@ class BatchPipeline:
                     import torch.distributed as dist
                     dist.all_gather_into_tensor(s["rec_all"], s["rec"], group=self.group)
                 s["rec_host"].copy_(s["rec_all"] if self.collect_all else s["rec"], non_blocking=True)
-                if self.overlay and self.mixed and shapes:
+                if self.encode is not None:
+                    s["offsets_host"].copy_(s["enc"].offsets, non_blocking=True)
+                elif self.overlay and self.mixed and shapes:
                     used = max(h * w * 3 for h, w in shapes)
                     s["frames_host"].view(self.batch, -1)[:len(shapes), :used].copy_(s["x"].view(self.batch, -1)[:len(shapes), :used],
                                                                                    non_blocking=True)
@@ -270,7 +299,8 @@ class BatchPipeline:
     def result(self, ticket, copy=True, source_coords=None, gathered=False):
         """Block until the ticket's records are on the host; returns the reference's 4-tuple for this rank's batch
         (numpy float64: [batch,P], [batch,P,17], [batch,P,17,2], [batch,P,17,2]).  With ``overlay``, a fifth item holds this
-        rank's drawn frames: uint8 [batch,h,w,3], or in mixed mode a list of [h_i,w_i,3] arrays, one per submitted frame.  With
+        rank's drawn frames: uint8 [batch,h,w,3], or in mixed mode a list of [h_i,w_i,3] arrays, one per submitted frame (with
+        ``encode``: their JPEG files, a list of ``bytes``).  With
         ``jpeg``, the last item is the int32 decode status [batch].  ``gathered=True`` (rank 0 of a
         ``gather=True`` pipeline): the records of ALL ranks' batches instead, leading dimension ``world * batch`` (rank-major).
         ``source_coords`` is a construction-time option (the scaling runs on the device); passing a different value here is an
@@ -285,7 +315,9 @@ class BatchPipeline:
         if copy:
             flat = flat.copy()
         frames = ()
-        if self.overlay:
+        if self.encode is not None:
+            frames = (self._files(s),)
+        elif self.overlay:
             fr = s["frames_host"].numpy()
             if self.mixed:
                 rows = fr.reshape(self.batch, -1)
@@ -301,6 +333,23 @@ class BatchPipeline:
         assert self.collect_all, "gathered=True: only rank 0 of a gather=True pipeline reads every rank's records back"
         parts = [split_pose_records(flat[r * self.nrec:(r + 1) * self.nrec], self.batch, self.P) for r in range(self.world)]
         return tuple(np.concatenate([p[j] for p in parts], axis=0) for j in range(4)) + frames
+
+    def _files(self, s):
+        """The slot's packed files, copied back on their own stream once the offsets are on the host (the d2h stream would
+        queue the copy behind later tickets' copies).  Returns only when the copy is done: the next step of this slot rewrites
+        the packed buffer."""
+        off = s["offsets_host"].numpy().copy()
+        n = int(off[-1])
+        if n > s["files_host"].numel():
+            s["files_host"] = torch.empty(n, dtype=torch.uint8).pin_memory()
+        if n:
+            with torch.cuda.device(self.dev), torch.cuda.stream(self.files_stream):
+                s["files_host"][:n].copy_(s["enc"].out[:n], non_blocking=True)
+            self.files_stream.synchronize()
+        self.last_file_bytes = n
+        data = s["files_host"].numpy()
+        count = len(s["shapes"]) if self.mixed else self.batch
+        return [data[off[i]:off[i + 1]].tobytes() for i in range(count)]
 
     def time_gather(self, reps=20):
         """Device time (ms) of one all-gather of a step's record buffer, measured alone with CUDA events."""
