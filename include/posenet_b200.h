@@ -246,6 +246,24 @@ int pn_jpeg_encode(const uint8_t *frames, int n_img, int max_h, int max_w, int64
                    int sampling, int restart_interval, uint8_t *out, int64_t out_capacity, int64_t *out_offsets, void *workspace,
                    size_t ws_bytes, pn_stream_t stream);
 
+/* ---- N6: image_demo.py:57 cv2.imwrite of the drawn frames to .png names: PNG files encoded ON THE DEVICE, bit-exact with
+ * cv2.imencode(".png", frame) without params (libpng 1.6 with cv2's SUB filter, zlib 1.3 deflate at level 1 with Z_RLE, IDAT
+ * chunks of 8192 bytes).
+ *
+ * pn_png_encode_bound (host only): a true worst case of one file of h x w (every block at its static coding, 9 bits a byte, or
+ * stored, with block, zlib and chunk overhead); 0 for 0 x 0. */
+int pn_png_encode_bound(int h, int w, int64_t *bytes_host);
+/* Device workspace (bytes, 256-byte aligned base) pn_png_encode needs for up to n_img frames of at most max_h x max_w. */
+int pn_png_encode_workspace(int n_img, int max_h, int max_w, size_t *bytes_host);
+/* Encode n_img frames at once.  frames: device uint8 BGR HWC, frame i from frames + i * frame_stride (>= 3 * max_h * max_w), rows
+ * of w_i * 3 bytes; frame_hw: device int32 [n_img, 2] with each frame's (h_i, w_i), a size outside 1..max_h x 1..max_w giving an
+ * empty file, or NULL for max_h x max_w everywhere.  out: device bytes, packed: file i is out[out_offsets[i] .. out_offsets[i + 1])
+ * with out_offsets device int64 [n_img + 1]; out_capacity must be at least n_img * pn_png_encode_bound(max_h, max_w) and nothing
+ * at or past out_offsets[n_img] is written.  The frames are only read.  The launch geometry depends only on the capacity, so the
+ * call can be captured in a CUDA graph. */
+int pn_png_encode(const uint8_t *frames, int n_img, int max_h, int max_w, int64_t frame_stride, const int *frame_hw, uint8_t *out,
+                  int64_t out_capacity, int64_t *out_offsets, void *workspace, size_t ws_bytes, pn_stream_t stream);
+
 /* ---- Whole-network plan: mobilenet_v1.py:130-162 (MobileNetV1.__init__/forward) --------------------
  * The layer table is computed by the caller (posenet/models/mobilenet_v1.py mirrors
  * _to_output_strided_layers, mobilenet_v1.py:8-39) and passed in explicitly. */

@@ -105,6 +105,10 @@ _SIGNATURES = {
     "pn_jpeg_encode_workspace": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
     "pn_jpeg_encode": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                  C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "pn_png_encode_bound": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_int64)]),
+    "pn_png_encode_workspace": (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
+    "pn_png_encode": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
+                                C.c_void_p, C.c_size_t, C.c_void_p]),
     "pn_plan_query": (C.c_int, [C.POINTER(NetDesc), C.POINTER(C.c_size_t), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "pn_plan_create": (C.c_int, [C.POINTER(NetDesc), C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p)]),
     "pn_plan_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

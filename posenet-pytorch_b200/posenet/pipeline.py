@@ -9,8 +9,8 @@ This is the batched form of what the reference's ``benchmark.py:32-44`` does per
     for pose_scores, keypoint_scores, keypoint_coords, pose_offsets in pipe.run(batches):   # pinned uint8 [64,513,513,3]
         ...
 
-Options on top of that (``overlay=`` draws the poses on the frames, ``encode=`` returns them as JPEG files, ``jpeg=True``
-takes JPEG files in): ``source_coords=True`` maps the keypoint coordinates back to the submitted frames ON THE DEVICE
+Options on top of that (``overlay=`` draws the poses on the frames, ``encode=`` returns them as JPEG files, or as PNG files
+with ``encode_ext=".png"``, ``jpeg=True`` takes JPEG files in): ``source_coords=True`` maps the keypoint coordinates back to the submitted frames ON THE DEVICE
 (``image_demo.py:50``), ``mixed=True`` accepts frames of different sizes in one batch (every file of a directory
 pre-processed at its own size, ``benchmark.py:24-29``), ``gather=True`` all-gathers the records of every rank's shard over
 NCCL inside the step (one process per GPU, ``posenet.sharding``).
@@ -27,7 +27,7 @@ from posenet.decode_multi import decode_multiple_poses_batch, split_pose_records
 
 class BatchPipeline:
     def __init__(self, model, batch, height, width, depth=2, use_graph=True, output_stride=None, scale_factor=1.0,
-                 source_coords=False, mixed=False, gather=False, group=None, overlay=None, jpeg=False, encode=None, **decode_kw):
+                 source_coords=False, mixed=False, gather=False, group=None, overlay=None, jpeg=False, encode=None, encode_ext=".jpg", **decode_kw):
         """``height`` x ``width``: size of the uint8 frames handed to ``submit`` (``mixed=True``: the LARGEST frame; each
         frame of a batch then comes with its own size).  The network runs at ``valid_resolution(width * scale_factor,
         height * scale_factor)`` (utils.py:7-10); frames of any other size go through the bit-exact cv2 resize
@@ -51,7 +51,9 @@ class BatchPipeline:
         in-graph device-to-host copy carries the files' offsets instead of the frames.  ``result`` copies exactly the bytes in use
         on a stream of its own (the offsets are only known on the host then) and returns a list of ``bytes`` as the fifth item
         instead of the frames: one per submitted frame in mixed mode, ``batch`` otherwise.  Params the device encoder does not
-        do raise ValueError here."""
+        do raise ValueError here.
+        ``encode_ext``: ``".jpg"`` (the default) or ``".png"``: the files are then PNG (``pn_png_encode``, bit-exact with
+        ``cv2.imencode(".png", frame)``; ``encode`` must be ``[]``)."""
         nat.require_device()
         assert depth >= 1
         self.model, self.batch, self.h, self.w = model, int(batch), int(height), int(width)
@@ -67,9 +69,15 @@ class BatchPipeline:
             "overlay on resized frames needs source_coords=True (the records must be in the frames' coordinates)"
         assert encode is None or self.overlay is not None, "encode= encodes the drawn frames: it needs overlay="
         self.encode = None if encode is None else list(encode)
+        if encode_ext not in (".jpg", ".png"):
+            raise ValueError("encode_ext %r: the device encoders write .jpg and .png" % (encode_ext,))
+        self.encode_ext = encode_ext
+        assert encode_ext == ".jpg" or self.encode is not None, "encode_ext= names the format of encode=: it needs encode="
         if self.encode is not None:
-            from posenet.jpeg import encode_options
-            encode_options(self.encode)
+            from posenet import jpeg as jpeg_codec, png as png_codec
+            codec = png_codec if encode_ext == ".png" else jpeg_codec
+            codec.encode_options(self.encode)
+            self.encoder = codec.Encoder
         self.decode_kw = dict(decode_kw)
         self.P = int(self.decode_kw.get("max_pose_detections", 10))
         dev = model._device()
@@ -110,20 +118,23 @@ class BatchPipeline:
                     s["status_host"] = torch.zeros(self.batch, dtype=torch.int32).pin_memory()
                     s["h2d_bytes"] = 0
             if self.encode is not None:
-                from posenet.jpeg import Encoder
+                # the share of the frames' raw size the files take, for the estimates below: drawn frames at q95 4:2:0 are
+                # 8-12 % as JPEG, smooth ones about 58 % as PNG (photographs more)
+                self.file_share = 0.6 if encode_ext == ".png" else 0.1
                 self.files_stream = torch.cuda.Stream(dev)             # result()'s copy of the packed files
                 for s in self.slots:
-                    s["enc"] = Encoder(self.batch, self.h, self.w, self.encode, dev)
+                    s["enc"] = self.encoder(self.batch, self.h, self.w, self.encode, dev)
                     s["offsets_host"] = torch.zeros(self.batch + 1, dtype=torch.int64).pin_memory()
-                    s["files_host"] = torch.empty(self.batch * self.h * self.w * 3 // 4, dtype=torch.uint8).pin_memory()
+                    s["files_host"] = torch.empty(int(self.batch * self.h * self.w * 3 * min(2.5 * self.file_share, 1)),
+                                                  dtype=torch.uint8).pin_memory()
             self.h2d_bytes_per_batch = self.slots[0]["x"].numel()
             self.d2h_bytes_per_batch = (self.world if self.collect_all else 1) * nrec * 8
             if self.overlay and self.encode is None:
                 self.d2h_bytes_per_batch += self.slots[0]["x"].numel()         # mixed mode copies only the bytes in use
             elif self.encode is not None:
-                # the offsets, plus the files: an estimate of a tenth of the frames' raw size (drawn frames at q95 4:2:0 are
-                # 8-12 %); result() copies exactly the bytes in use and records them in last_file_bytes
-                self.d2h_bytes_per_batch += 8 * (self.batch + 1) + self.slots[0]["x"].numel() // 10
+                # the offsets, plus the files: an estimate (file_share of the frames' raw size); result() copies exactly the
+                # bytes in use and records them in last_file_bytes
+                self.d2h_bytes_per_batch += 8 * (self.batch + 1) + int(self.slots[0]["x"].numel() * self.file_share)
             self.last_file_bytes = 0
             # warm up (plans, workspaces) and capture one graph per slot on the compute stream
             self.compute.wait_stream(torch.cuda.current_stream(dev))
@@ -300,7 +311,7 @@ class BatchPipeline:
         """Block until the ticket's records are on the host; returns the reference's 4-tuple for this rank's batch
         (numpy float64: [batch,P], [batch,P,17], [batch,P,17,2], [batch,P,17,2]).  With ``overlay``, a fifth item holds this
         rank's drawn frames: uint8 [batch,h,w,3], or in mixed mode a list of [h_i,w_i,3] arrays, one per submitted frame (with
-        ``encode``: their JPEG files, a list of ``bytes``).  With
+        ``encode``: their JPEG or PNG files, a list of ``bytes``).  With
         ``jpeg``, the last item is the int32 decode status [batch].  ``gathered=True`` (rank 0 of a
         ``gather=True`` pipeline): the records of ALL ranks' batches instead, leading dimension ``world * batch`` (rank-major).
         ``source_coords`` is a construction-time option (the scaling runs on the device); passing a different value here is an
