@@ -223,6 +223,15 @@ int pn_jpeg_workspace(int n_img, int64_t arena_bytes, int max_h, int max_w, size
 int pn_jpeg_decode(const uint8_t *files, int64_t arena_bytes, const pn_jpeg_desc *descs, int n_img, int max_h, int max_w,
                    uint8_t *frames, int64_t frame_stride, int *frame_hw, void *workspace, size_t ws_bytes, int *status,
                    pn_stream_t stream);
+/* The same at 1 / scale_denom (1, 2, 4 or 8; anything else is PN_ERR_ARG), bit-exact with cv2.imdecode(buf,
+ * IMREAD_REDUCED_COLOR_<scale_denom>): libjpeg's DCT-domain scaling (jidctred.c), no full-size intermediate.  Frame i is
+ * ceil(height / scale_denom) x ceil(width / scale_denom), and that is what frame_hw reports; max_h x max_w bound those reduced
+ * sizes (a file up to scale_denom * max_h x scale_denom * max_w).  With scale_denom 1 these are pn_jpeg_workspace /
+ * pn_jpeg_decode. */
+int pn_jpeg_workspace_scaled(int n_img, int64_t arena_bytes, int max_h, int max_w, int scale_denom, size_t *bytes_host);
+int pn_jpeg_decode_scaled(const uint8_t *files, int64_t arena_bytes, const pn_jpeg_desc *descs, int n_img, int max_h, int max_w,
+                          int scale_denom, uint8_t *frames, int64_t frame_stride, int *frame_hw, void *workspace, size_t ws_bytes,
+                          int *status, pn_stream_t stream);
 
 /* ---- N5: image_demo.py:57 cv2.imwrite of the drawn frames: baseline JPEG files encoded ON THE DEVICE, bit-exact with
  * cv2.imencode(".jpg", frame, params) (libjpeg-turbo 3.1 as cv2 4.13 calls it: jccolor.c, jcsample.c, the accurate integer FDCT

@@ -14,8 +14,11 @@
 //             up to m[0], then path m[0], ...  Every chain element gets its true exit state and block count
 //   write     every subsequence decodes from its true entry and stores the blocks that begin in it (DC as a difference)
 //   dc        one warp per segment: per-component prefix sums of the DC differences (reset at every restart marker)
-//   idct      jpeg_idct_islow, eight threads per block, into per-component sample planes
-//   color     upsampling + YCbCr -> BGR, one thread per pixel, straight into the frame's row
+//   idct      eight threads per block, into per-component sample planes: jpeg_idct_islow, or at 1/2, 1/4, 1/8 (scale_denom,
+//             cv2's IMREAD_REDUCED_COLOR_*) the component's scaled IDCT (jidctred.c), ssize x ssize samples per block
+//   color     upsampling + YCbCr -> BGR, one thread per output pixel, straight into the frame's row (ceil(h / d) x ceil(w / d))
+// Everything up to dc is independent of the scale.  The workspace is sized for files of scale_denom * max_h x scale_denom * max_w
+// (a file whose reduced frame fits max_h x max_w is at most that large).
 // (Weissenberger & Schmidt, "Massively Parallel Huffman Decoding on GPUs", ICPP 2018, for the self-synchronisation.)
 #include "common.cuh"
 #include "jpeg_decode.cuh"
@@ -101,7 +104,7 @@ struct Args {
     const uint8_t *files;
     int64_t arena;
     const pn_jpeg_desc *descs;
-    int n_img, max_h, max_w;
+    int n_img, max_h, max_w, denom;    // max_h x max_w: the largest OUTPUT frame (at 1 / denom)
     uint8_t *frames;
     int64_t stride;
     int *frame_hw, *status;
@@ -127,7 +130,8 @@ __global__ void __launch_bounds__(32) plan_kernel(Args a, Ws ws) {
         bool ok = d.kind == PN_JPEG_SUPPORTED;
         const bool skipped = !ok;
         ok = ok && d.file_offset >= 0 && d.file_bytes > 0 && d.file_offset + d.file_bytes <= a.arena && d.scan_offset >= 0 &&
-             d.scan_offset < d.file_bytes && d.height >= 1 && d.height <= a.max_h && d.width >= 1 && d.width <= a.max_w &&
+             d.scan_offset < d.file_bytes && d.height >= 1 && (d.height + a.denom - 1) / a.denom <= a.max_h && d.width >= 1 &&
+             (d.width + a.denom - 1) / a.denom <= a.max_w &&
              (d.ncomp == 1 || d.ncomp == 3) && d.blocks_per_mcu >= 1 && d.blocks_per_mcu <= PN_JPEG_MAX_BLOCKS &&
              d.mcus_x >= 1 && d.mcus_y >= 1 && d.restart_interval >= 1;
         const long long mcus = ok ? (long long)d.mcus_x * d.mcus_y : 0;
@@ -145,6 +149,14 @@ __global__ void __launch_bounds__(32) plan_kernel(Args a, Ws ws) {
             ok = c < d.ncomp && d.mcu_bx[b] < d.comp[c].h && d.mcu_by[b] < d.comp[c].v;
         }
         ok = ok && planes == mcus * d.blocks_per_mcu;
+        Scaled g;                              // the reduced planes and the upsampler's reads stay inside the blocks
+        ok = ok && scaled_geometry(d, a.denom, &g);
+        for (int c = 0; ok && c < d.ncomp; ++c) {
+            const pn_jpeg_comp &k = d.comp[c];
+            const CompScale &s = g.comp[c];
+            ok = s.dw >= 1 && s.dh >= 1 && s.dw <= s.ssize * k.bw && s.dh <= s.ssize * k.bh && (g.w - 1) / s.hr < s.dw &&
+                 (g.h - 1) / s.vr < s.dh;
+        }
         // DC symbols are extra-bit counts: at most 15 (what jpeg_make_d_derived_tbl enforces)
         bool tables_ok = true;
         for (int c = 0; ok && c < d.ncomp; ++c) {
@@ -574,7 +586,7 @@ __global__ void __launch_bounds__(THREADS) dc_kernel(Args a, Ws ws) {
     }
 }
 
-// ---- IDCT: eight threads per block ------------------------------------------------------------------------------------------------
+// ---- IDCT: eight threads per block (pass 1: a column each; pass 2: a row each, the first ssize threads) --------------------------
 __global__ void __launch_bounds__(THREADS) idct_kernel(Args a, Ws ws) {
     __shared__ int wsm[THREADS / 8][64];
     const int grp = threadIdx.x >> 3, r = threadIdx.x & 7;
@@ -591,21 +603,26 @@ __global__ void __launch_bounds__(THREADS) idct_kernel(Args a, Ws ws) {
             img = ws.img[lo].status == PN_JPEG_OK ? lo : -1;
         }
         const pn_jpeg_desc *d = img >= 0 ? a.descs + img : nullptr;
-        int comp = 0, bx = 0, by = 0;
-        long long g = 0;
+        int comp = 0, bx = 0, by = 0, ss = 8;
         if (d) {
-            g = gb - ws.img[img].blk_base;
-            block_place(*d, g, &comp, &bx, &by);
-            idct_column(ws.coef + gb * 64, d->quant[comp], r, wsm[grp]);
+            block_place(*d, gb - ws.img[img].blk_base, &comp, &bx, &by);
+            ss = comp_ssize(*d, a.denom, comp);
+            idct_column_scaled(ws.coef + gb * 64, d->quant[comp], ss, r, wsm[grp]);
         }
         __syncwarp();
-        if (d) {
+        if (d && ss == 8) {
             const int pitch = d->comp[comp].bw * 8;
             uint8_t o[8];
             idct_row(wsm[grp], r, o);
             uint8_t *dst = ws.planes + ws.img[img].plane_base[comp] + ((long long)by * 8 + r) * pitch + bx * 8;
             *reinterpret_cast<uint2 *>(dst) = make_uint2(o[0] | (o[1] << 8) | (o[2] << 16) | ((uint32_t)o[3] << 24),
                                                          o[4] | (o[5] << 8) | (o[6] << 16) | ((uint32_t)o[7] << 24));
+        } else if (d && r < ss) {
+            const int pitch = d->comp[comp].bw * ss;
+            uint8_t o[4];
+            idct_row_scaled(ws.coef + gb * 64, d->quant[comp], wsm[grp], ss, r, o);
+            uint8_t *dst = ws.planes + ws.img[img].plane_base[comp] + ((long long)by * ss + r) * pitch + (long long)bx * ss;
+            for (int c = 0; c < ss; ++c) dst[c] = o[c];
         }
         __syncwarp();
     }
@@ -618,26 +635,28 @@ __global__ void __launch_bounds__(THREADS) color_kernel(Args a, Ws ws) {
     const int st = w.status;
     if (blockIdx.x == 0 && threadIdx.x == 0) {
         a.status[i] = st;
-        if (a.frame_hw) {
-            a.frame_hw[2 * i] = st == PN_JPEG_OK ? a.descs[i].height : 0;
-            a.frame_hw[2 * i + 1] = st == PN_JPEG_OK ? a.descs[i].width : 0;
+        if (a.frame_hw) {                   // the frame at 1 / denom
+            a.frame_hw[2 * i] = st == PN_JPEG_OK ? (a.descs[i].height + a.denom - 1) / a.denom : 0;
+            a.frame_hw[2 * i + 1] = st == PN_JPEG_OK ? (a.descs[i].width + a.denom - 1) / a.denom : 0;
         }
     }
     if (st == PN_JPEG_SKIPPED || st == PN_JPEG_ERR_DESC) return;     // untouched: the host's frame, or no trusted size
     const pn_jpeg_desc &d = a.descs[i];
-    const int H = d.height, W = d.width;
+    Scaled g;
+    scaled_geometry(d, a.denom, &g);       // plan_kernel checked it
+    const int H = g.h, W = g.w;
     uint8_t *frame = a.frames + (long long)i * a.stride;
     const uint8_t *plane[3];
     int pitch[3];
 #pragma unroll
     for (int c = 0; c < 3; ++c) {           // components past ncomp are never read
         plane[c] = ws.planes + w.plane_base[c];
-        pitch[c] = d.comp[c].bw * 8;
+        pitch[c] = d.comp[c].bw * g.comp[c].ssize;
     }
     const long long npx = (long long)H * W;
     for (long long p = blockIdx.x * (long long)THREADS + threadIdx.x; p < npx; p += (long long)gridDim.x * THREADS) {
         uint8_t bgr[3] = {0, 0, 0};
-        if (st == PN_JPEG_OK) pixel_bgr(d, plane, pitch, (int)(p / W), (int)(p % W), bgr);
+        if (st == PN_JPEG_OK) pixel_bgr(d, g, plane, pitch, (int)(p / W), (int)(p % W), bgr);
         frame[3 * p] = bgr[0];
         frame[3 * p + 1] = bgr[1];
         frame[3 * p + 2] = bgr[2];
@@ -667,7 +686,8 @@ Ws bind(void *base, const Layout &L) {
     return w;
 }
 
-bool caps_ok(int n_img, int64_t arena_bytes, int max_h, int max_w) {
+// max_h x max_w: the full-size capacity (scale_denom times the output capacity)
+bool caps_ok(int n_img, int64_t arena_bytes, long long max_h, long long max_w) {
     return n_img > 0 && n_img <= 65535 && arena_bytes > 0 && arena_bytes < (1ll << 40) && max_h > 0 && max_w > 0 &&
            max_h <= 65500 && max_w <= 65500;
 }
@@ -677,26 +697,36 @@ bool caps_ok(int n_img, int64_t arena_bytes, int max_h, int max_w) {
 
 using namespace pn;
 
-extern "C" int pn_jpeg_workspace(int n_img, int64_t arena_bytes, int max_h, int max_w, size_t *bytes_host) {
-    PN_CHECK_ARG(bytes_host, "pn_jpeg_workspace: null pointer");
-    PN_CHECK_ARG(caps_ok(n_img, arena_bytes, max_h, max_w), "pn_jpeg_workspace: bad capacity (%d images, %lld bytes, %d x %d)",
-                 n_img, (long long)arena_bytes, max_h, max_w);
-    *bytes_host = layout(n_img, arena_bytes, max_h, max_w).bytes;
+extern "C" int pn_jpeg_workspace_scaled(int n_img, int64_t arena_bytes, int max_h, int max_w, int scale_denom,
+                                        size_t *bytes_host) {
+    PN_CHECK_ARG(bytes_host, "pn_jpeg_workspace_scaled: null pointer");
+    PN_CHECK_ARG(valid_denom(scale_denom), "pn_jpeg_workspace_scaled: scale_denom %d is not 1, 2, 4 or 8", scale_denom);
+    PN_CHECK_ARG(caps_ok(n_img, arena_bytes, (long long)max_h * scale_denom, (long long)max_w * scale_denom),
+                 "pn_jpeg_workspace_scaled: bad capacity (%d images, %lld bytes, %d x %d at 1/%d)", n_img, (long long)arena_bytes,
+                 max_h, max_w, scale_denom);
+    *bytes_host = layout(n_img, arena_bytes, max_h * scale_denom, max_w * scale_denom).bytes;
     return PN_OK;
 }
 
-extern "C" int pn_jpeg_decode(const uint8_t *files, int64_t arena_bytes, const pn_jpeg_desc *descs, int n_img, int max_h, int max_w,
-                              uint8_t *frames, int64_t frame_stride, int *frame_hw, void *workspace, size_t ws_bytes, int *status,
-                              pn_stream_t stream) {
-    PN_CHECK_ARG(files && descs && frames && workspace && status, "pn_jpeg_decode: null pointer");
-    PN_CHECK_ARG(caps_ok(n_img, arena_bytes, max_h, max_w), "pn_jpeg_decode: bad capacity (%d images, %lld bytes, %d x %d)", n_img,
-                 (long long)arena_bytes, max_h, max_w);
-    PN_CHECK_ARG(frame_stride >= 3ll * max_h * max_w, "pn_jpeg_decode: frame_stride %lld < 3 * max_h * max_w",
+extern "C" int pn_jpeg_workspace(int n_img, int64_t arena_bytes, int max_h, int max_w, size_t *bytes_host) {
+    return pn_jpeg_workspace_scaled(n_img, arena_bytes, max_h, max_w, 1, bytes_host);
+}
+
+extern "C" int pn_jpeg_decode_scaled(const uint8_t *files, int64_t arena_bytes, const pn_jpeg_desc *descs, int n_img, int max_h,
+                                     int max_w, int scale_denom, uint8_t *frames, int64_t frame_stride, int *frame_hw,
+                                     void *workspace, size_t ws_bytes, int *status, pn_stream_t stream) {
+    PN_CHECK_ARG(files && descs && frames && workspace && status, "pn_jpeg_decode_scaled: null pointer");
+    PN_CHECK_ARG(valid_denom(scale_denom), "pn_jpeg_decode_scaled: scale_denom %d is not 1, 2, 4 or 8", scale_denom);
+    PN_CHECK_ARG(caps_ok(n_img, arena_bytes, (long long)max_h * scale_denom, (long long)max_w * scale_denom),
+                 "pn_jpeg_decode_scaled: bad capacity (%d images, %lld bytes, %d x %d at 1/%d)", n_img, (long long)arena_bytes,
+                 max_h, max_w, scale_denom);
+    PN_CHECK_ARG(frame_stride >= 3ll * max_h * max_w, "pn_jpeg_decode_scaled: frame_stride %lld < 3 * max_h * max_w",
                  (long long)frame_stride);
-    PN_CHECK_ARG(((uintptr_t)workspace & 255) == 0, "pn_jpeg_decode: workspace must be 256-byte aligned");
-    const Layout L = layout(n_img, arena_bytes, max_h, max_w);
-    PN_CHECK_ARG(ws_bytes >= L.bytes, "pn_jpeg_decode: workspace %zu < %zu bytes (pn_jpeg_workspace)", ws_bytes, L.bytes);
-    Args a{files, arena_bytes, descs, n_img, max_h, max_w, frames, frame_stride, frame_hw, status};
+    PN_CHECK_ARG(((uintptr_t)workspace & 255) == 0, "pn_jpeg_decode_scaled: workspace must be 256-byte aligned");
+    const Layout L = layout(n_img, arena_bytes, max_h * scale_denom, max_w * scale_denom);
+    PN_CHECK_ARG(ws_bytes >= L.bytes, "pn_jpeg_decode_scaled: workspace %zu < %zu bytes (pn_jpeg_workspace_scaled)", ws_bytes,
+                 L.bytes);
+    Args a{files, arena_bytes, descs, n_img, max_h, max_w, scale_denom, frames, frame_stride, frame_hw, status};
     const Ws w = bind(workspace, L);
     const cudaStream_t st = as_stream(stream);
     const int grid = 4 * num_sms();
@@ -724,4 +754,11 @@ extern "C" int pn_jpeg_decode(const uint8_t *files, int64_t arena_bytes, const p
     color_kernel<<<dim3((unsigned)gx, (unsigned)n_img), THREADS, 0, st>>>(a, w);
     PN_CHECK_LAUNCH();
     return PN_OK;
+}
+
+extern "C" int pn_jpeg_decode(const uint8_t *files, int64_t arena_bytes, const pn_jpeg_desc *descs, int n_img, int max_h, int max_w,
+                              uint8_t *frames, int64_t frame_stride, int *frame_hw, void *workspace, size_t ws_bytes, int *status,
+                              pn_stream_t stream) {
+    return pn_jpeg_decode_scaled(files, arena_bytes, descs, n_img, max_h, max_w, 1, frames, frame_stride, frame_hw, workspace,
+                                 ws_bytes, status, stream);
 }

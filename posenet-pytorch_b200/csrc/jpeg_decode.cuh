@@ -4,8 +4,11 @@
 //
 //   entropy data:  byte de-stuffing and markers (jdhuff.c fill_bit_buffer), Huffman symbols (HUFF_DECODE / jpeg_huff_decode),
 //                  HUFF_EXTEND, zig-zag runs landing on coefficient 63 past the end (jpeg_natural_order's 16 extra entries)
-//   IDCT:          jpeg_idct_islow (jidctint.c): CONST_BITS 13, PASS1_BITS 2, range_limit[x & RANGE_MASK]
-//   upsampling:    jdsample.c h2v1 / h1v2 / h2v2 fancy, replication otherwise; context rows as jdmainct.c supplies them
+//   IDCT:          jpeg_idct_islow (jidctint.c): CONST_BITS 13, PASS1_BITS 2, range_limit[x & RANGE_MASK]; at 1/2, 1/4, 1/8
+//                  (cv2's IMREAD_REDUCED_COLOR_*) jpeg_idct_4x4 / 2x2 / 1x1 (jidctred.c) with the per-component scaled sizes
+//                  of jdmaster.c
+//   upsampling:    jdsample.c h2v1 / h1v2 / h2v2 fancy, replication otherwise, chosen from the scaled group ratios; context
+//                  rows as jdmainct.c supplies them
 //   colour:        jdcolor.c ycc_rgb_convert (build_ycc_rgb_table, SCALEBITS 16) into B, G, R; grayscale replicated
 #pragma once
 #include <stdint.h>
@@ -285,24 +288,173 @@ PN_JHD void idct_row(const int *ws, int row, uint8_t *outp) {
     for (int c = 0; c < 8; ++c) outp[c] = idct_limit(descale(out[c], CONST_BITS + PASS1_BITS + 3));
 }
 
+// ---- reduced IDCTs: jidctred.c (cv2's IMREAD_REDUCED_*: libjpeg's DCT-domain scaling) ------------------------------------------
+// jpeg_idct_4x4 and jpeg_idct_2x2 are their own transforms, not truncations of islow: they read the odd coefficients 1, 3, 5, 7
+// (and 2, 6 for 4x4) and never coefficient 4.  Both passes split like idct_column / idct_row: pass 1 fills ws[r * 8 + col] for
+// r < n (columns the second pass does not read are skipped), pass 2 turns row `row` of ws into n samples.
+constexpr int64_t FIX_0_211164243 = 1730, FIX_0_509795579 = 4176, FIX_0_601344887 = 4926, FIX_0_720959822 = 5906,
+                  FIX_0_850430095 = 6967, FIX_1_061594337 = 8697, FIX_1_272758580 = 10426, FIX_1_451774981 = 11893,
+                  FIX_2_172734803 = 17799, FIX_3_624509785 = 29692;
+
+// The 4-point odd part both passes of jpeg_idct_4x4 share (z1..z4: inputs 7, 5, 3, 1).
+PN_JHD void idct4_odd(int64_t z1, int64_t z2, int64_t z3, int64_t z4, int64_t *tmp0, int64_t *tmp2) {
+    *tmp0 = z1 * -FIX_0_211164243 + z2 * FIX_1_451774981 + z3 * -FIX_2_172734803 + z4 * FIX_1_061594337;
+    *tmp2 = z1 * -FIX_0_509795579 + z2 * -FIX_0_601344887 + z3 * FIX_0_899976223 + z4 * FIX_2_562915447;
+}
+
+PN_JHD void idct4x4_column(const int16_t *coef, const int16_t *quant, int col, int *ws) {
+    if (col == 4) return;
+    auto dq = [&](int r) { return (int64_t)((int)coef[r * 8 + col] * (int)quant[r * 8 + col]); };
+    const int64_t tmp0e = dq(0) * ((int64_t)1 << (CONST_BITS + 1));
+    const int64_t tmp2e = dq(2) * FIX_1_847759065 + dq(6) * -FIX_0_765366865;
+    const int64_t tmp10 = tmp0e + tmp2e, tmp12 = tmp0e - tmp2e;
+    int64_t tmp0, tmp2;
+    idct4_odd(dq(7), dq(5), dq(3), dq(1), &tmp0, &tmp2);
+    const int sh = CONST_BITS - PASS1_BITS + 1;   // the all-AC-zero shortcut of jidctred.c computes the same values
+    ws[0 * 8 + col] = (int)descale(tmp10 + tmp2, sh);
+    ws[3 * 8 + col] = (int)descale(tmp10 - tmp2, sh);
+    ws[1 * 8 + col] = (int)descale(tmp12 + tmp0, sh);
+    ws[2 * 8 + col] = (int)descale(tmp12 - tmp0, sh);
+}
+
+PN_JHD void idct4x4_row(const int *ws, int row, uint8_t *outp) {
+    const int *w = ws + row * 8;
+    const int64_t tmp0e = (int64_t)w[0] * ((int64_t)1 << (CONST_BITS + 1));
+    const int64_t tmp2e = (int64_t)w[2] * FIX_1_847759065 + (int64_t)w[6] * -FIX_0_765366865;
+    const int64_t tmp10 = tmp0e + tmp2e, tmp12 = tmp0e - tmp2e;
+    int64_t tmp0, tmp2;
+    idct4_odd(w[7], w[5], w[3], w[1], &tmp0, &tmp2);
+    const int sh = CONST_BITS + PASS1_BITS + 3 + 1;
+    outp[0] = idct_limit(descale(tmp10 + tmp2, sh));
+    outp[3] = idct_limit(descale(tmp10 - tmp2, sh));
+    outp[1] = idct_limit(descale(tmp12 + tmp0, sh));
+    outp[2] = idct_limit(descale(tmp12 - tmp0, sh));
+}
+
+PN_JHD void idct2x2_column(const int16_t *coef, const int16_t *quant, int col, int *ws) {
+    if (col == 2 || col == 4 || col == 6) return;
+    auto dq = [&](int r) { return (int64_t)((int)coef[r * 8 + col] * (int)quant[r * 8 + col]); };
+    const int64_t tmp10 = dq(0) * ((int64_t)1 << (CONST_BITS + 2));
+    const int64_t tmp0 = dq(7) * -FIX_0_720959822 + dq(5) * FIX_0_850430095 + dq(3) * -FIX_1_272758580 + dq(1) * FIX_3_624509785;
+    ws[0 * 8 + col] = (int)descale(tmp10 + tmp0, CONST_BITS - PASS1_BITS + 2);
+    ws[1 * 8 + col] = (int)descale(tmp10 - tmp0, CONST_BITS - PASS1_BITS + 2);
+}
+
+PN_JHD void idct2x2_row(const int *ws, int row, uint8_t *outp) {
+    const int *w = ws + row * 8;
+    const int64_t tmp10 = (int64_t)w[0] * ((int64_t)1 << (CONST_BITS + 2));
+    const int64_t tmp0 = (int64_t)w[7] * -FIX_0_720959822 + (int64_t)w[5] * FIX_0_850430095 +
+                         (int64_t)w[3] * -FIX_1_272758580 + (int64_t)w[1] * FIX_3_624509785;
+    outp[0] = idct_limit(descale(tmp10 + tmp0, CONST_BITS + PASS1_BITS + 3 + 2));
+    outp[1] = idct_limit(descale(tmp10 - tmp0, CONST_BITS + PASS1_BITS + 3 + 2));
+}
+
+// jpeg_idct_1x1: the DC term alone, descaled by 3
+PN_JHD uint8_t idct1x1(const int16_t *coef, const int16_t *quant) {
+    return idct_limit(descale((int64_t)((int)coef[0] * (int)quant[0]), 3));
+}
+
+// The IDCT of scaled size n (8: islow, 4, 2, 1), split in passes as above; idct_row_scaled writes n samples.
+PN_JHD void idct_column_scaled(const int16_t *coef, const int16_t *quant, int n, int col, int *ws) {
+    if (n == 8) idct_column(coef, quant, col, ws);
+    else if (n == 4) idct4x4_column(coef, quant, col, ws);
+    else if (n == 2) idct2x2_column(coef, quant, col, ws);
+}
+PN_JHD void idct_row_scaled(const int16_t *coef, const int16_t *quant, const int *ws, int n, int row, uint8_t *outp) {
+    if (n == 8) idct_row(ws, row, outp);
+    else if (n == 4) idct4x4_row(ws, row, outp);
+    else if (n == 2) idct2x2_row(ws, row, outp);
+    else outp[0] = idct1x1(coef, quant);
+}
+
+// ---- output geometry at 1 / scale_denom (jdmaster.c jpeg_core_output_dimensions, jdsample.c jinit_upsampler) ----------------------
+// The frame is ceil(h / d) x ceil(w / d).  Luma's IDCT is 8 / d; a component whose samples are coarser than the largest factor
+// doubles its IDCT size while that keeps the ratio to the minimum integral in both directions, so (e.g.) 4:2:0 chroma at 1/2 is
+// decoded with the full 8x8 IDCT and needs no upsampling.  What is left to upsample is the ratio of max_h x max_v output samples
+// to the component's h_in_group x v_in_group; fancy filters only when the minimum scaled size is above 1.
+enum { UP_FULL = 0, UP_H2V1_FANCY, UP_H1V2_FANCY, UP_H2V2_FANCY, UP_REPLICATE };
+struct CompScale {
+    int ssize;        // DCT_scaled_size: samples per block side
+    int hr, vr;       // upsampling ratios (output samples per component sample)
+    int dw, dh;       // downsampled_width / downsampled_height: the component's real samples at this scale
+    int up;           // UP_*
+};
+struct Scaled {
+    int h, w;         // output frame size
+    CompScale comp[3];
+};
+
+PN_JHD bool valid_denom(int denom) { return denom == 1 || denom == 2 || denom == 4 || denom == 8; }
+
+// DCT_scaled_size of component c (sampling factors >= 1, denom valid)
+PN_JHD int comp_ssize(const pn_jpeg_desc &d, int denom, int c) {
+    const int mn = 8 / denom;
+    if (mn == 8) return 8;
+    int max_h = 1, max_v = 1;
+    for (int k = 0; k < d.ncomp; ++k) {
+        max_h = d.comp[k].h > max_h ? d.comp[k].h : max_h;
+        max_v = d.comp[k].v > max_v ? d.comp[k].v : max_v;
+    }
+    const int h = d.comp[c].h, v = d.comp[c].v;
+    int ss = mn;
+    while (ss < 8 && (max_h * mn) % (h * ss * 2) == 0 && (max_v * mn) % (v * ss * 2) == 0) ss *= 2;
+    return ss;
+}
+
+// False for a scale_denom other than 1, 2, 4, 8 or a ratio that is not integral (JERR_FRACT_SAMPLE_NOTIMPL).
+PN_JHD bool scaled_geometry(const pn_jpeg_desc &d, int denom, Scaled *g) {
+    if (!valid_denom(denom)) return false;
+    const int mn = 8 / denom;
+    int max_h = 1, max_v = 1;
+    for (int c = 0; c < d.ncomp; ++c) {
+        if (d.comp[c].h < 1 || d.comp[c].v < 1) return false;
+        max_h = d.comp[c].h > max_h ? d.comp[c].h : max_h;
+        max_v = d.comp[c].v > max_v ? d.comp[c].v : max_v;
+    }
+    g->h = (d.height + denom - 1) / denom;
+    g->w = (d.width + denom - 1) / denom;
+    for (int c = 0; c < 3; ++c) {
+        CompScale &s = g->comp[c];
+        s = CompScale{mn, 1, 1, 1, 1, UP_FULL};
+        if (c >= d.ncomp) continue;
+        const int h = d.comp[c].h, v = d.comp[c].v;
+        const int ss = comp_ssize(d, denom, c);
+        s.ssize = ss;
+        s.dw = (int)(((int64_t)d.width * h * ss + max_h * 8 - 1) / (max_h * 8));
+        s.dh = (int)(((int64_t)d.height * v * ss + max_v * 8 - 1) / (max_v * 8));
+        const int hin = h * ss / mn, vin = v * ss / mn;
+        if (max_h % hin || max_v % vin) return false;
+        s.hr = max_h / hin;
+        s.vr = max_v / vin;
+        const bool fancy = mn > 1;
+        if (s.hr == 1 && s.vr == 1) s.up = UP_FULL;
+        else if (s.hr == 2 && s.vr == 1) s.up = fancy && s.dw > 2 ? UP_H2V1_FANCY : UP_REPLICATE;
+        else if (s.hr == 1 && s.vr == 2) s.up = fancy ? UP_H1V2_FANCY : UP_REPLICATE;
+        else if (s.hr == 2 && s.vr == 2) s.up = fancy && s.dw > 2 ? UP_H2V2_FANCY : UP_REPLICATE;
+        else s.up = UP_REPLICATE;
+    }
+    return true;
+}
+
 // ---- upsampling (jdsample.c) -------------------------------------------------------------------------------------------------------
-// Sample (y, x) of the full-resolution component, from its downsampled plane (pitch bytes per row, dw x dh real samples).
+// Sample (y, x) of the output-resolution component, from its downsampled plane (pitch bytes per row, dw x dh real samples).
 // Rows above the first and below row dh - 1 are that row repeated (jdmainct.c context rows).
-PN_JHD int upsample(const uint8_t *pl, int pitch, const pn_jpeg_comp &c, int y, int x) {
-    const int hr = c.hr, vr = c.vr, dw = c.dw, dh = c.dh;
-    if (hr == 1 && vr == 1) return pl[(int64_t)y * pitch + x];
-    if (hr == 1 && vr == 2) {                                                        // h1v2_fancy_upsample
+PN_JHD int upsample(const uint8_t *pl, int pitch, const CompScale &c, int y, int x) {
+    const int dw = c.dw, dh = c.dh;
+    switch (c.up) {
+    case UP_FULL: return pl[(int64_t)y * pitch + x];
+    case UP_H1V2_FANCY: {                                                            // h1v2_fancy_upsample
         const int iy = y >> 1, v = y & 1;
         const int nb = v ? (iy + 1 < dh ? iy + 1 : dh - 1) : (iy > 0 ? iy - 1 : 0);
         return (3 * pl[(int64_t)iy * pitch + x] + pl[(int64_t)nb * pitch + x] + (v ? 2 : 1)) >> 2;
     }
-    if (hr == 2 && vr == 1 && dw > 2) {                                              // h2v1_fancy_upsample
+    case UP_H2V1_FANCY: {                                                            // h2v1_fancy_upsample
         const uint8_t *row = pl + (int64_t)y * pitch;
         const int ix = x >> 1;
         if (!(x & 1)) return ix == 0 ? row[0] : (3 * row[ix] + row[ix - 1] + 1) >> 2;
         return ix == dw - 1 ? row[dw - 1] : (3 * row[ix] + row[ix + 1] + 2) >> 2;
     }
-    if (hr == 2 && vr == 2 && dw > 2) {                                              // h2v2_fancy_upsample
+    case UP_H2V2_FANCY: {                                                            // h2v2_fancy_upsample
         const int iy = y >> 1, v = y & 1;
         const int nb = v ? (iy + 1 < dh ? iy + 1 : dh - 1) : (iy > 0 ? iy - 1 : 0);
         const uint8_t *r0 = pl + (int64_t)iy * pitch, *r1 = pl + (int64_t)nb * pitch;
@@ -311,7 +463,8 @@ PN_JHD int upsample(const uint8_t *pl, int pitch, const pn_jpeg_comp &c, int y, 
         if (!(x & 1)) return ix == 0 ? (4 * cs + 8) >> 4 : (3 * cs + 3 * r0[ix - 1] + r1[ix - 1] + 8) >> 4;
         return ix == dw - 1 ? (4 * cs + 7) >> 4 : (3 * cs + 3 * r0[ix + 1] + r1[ix + 1] + 7) >> 4;
     }
-    return pl[(int64_t)(y / vr) * pitch + x / hr];                                   // h2v1 / h2v2 / int_upsample: replication
+    default: return pl[(int64_t)(y / c.vr) * pitch + x / c.hr];                      // h2v1 / h2v2 / int_upsample: replication
+    }
 }
 
 // ---- colour (jdcolor.c) --------------------------------------------------------------------------------------------------------------
@@ -327,14 +480,23 @@ PN_JHD void ycc_to_bgr(int y, int cb, int cr, uint8_t *bgr) {
     bgr[2] = clamp255(y + r);
 }
 
-// Pixel (y, x) of the image as BGR, from the component planes (plane[c] has pitch[c] bytes per row).
-PN_JHD void pixel_bgr(const pn_jpeg_desc &d, const uint8_t *const plane[3], const int pitch[3], int y, int x, uint8_t *bgr) {
-    const int Y = upsample(plane[0], pitch[0], d.comp[0], y, x);
+// Pixel (y, x) of the output frame as BGR, from the component planes at scale g (plane[c] has pitch[c] bytes per row).
+PN_JHD void pixel_bgr(const pn_jpeg_desc &d, const Scaled &g, const uint8_t *const plane[3], const int pitch[3], int y, int x,
+                      uint8_t *bgr) {
+    const int Y = upsample(plane[0], pitch[0], g.comp[0], y, x);
     if (d.ncomp == 1) {
         bgr[0] = bgr[1] = bgr[2] = (uint8_t)Y;
         return;
     }
-    ycc_to_bgr(Y, upsample(plane[1], pitch[1], d.comp[1], y, x), upsample(plane[2], pitch[2], d.comp[2], y, x), bgr);
+    ycc_to_bgr(Y, upsample(plane[1], pitch[1], g.comp[1], y, x), upsample(plane[2], pitch[2], g.comp[2], y, x), bgr);
+}
+
+// The same at full size, for the serial host decoder of tests/test_jpeg_cpu.py: it derives the geometry per pixel, so a loop over
+// pixels (csrc/jpeg.cu's color_kernel) calls scaled_geometry once and the overload above.
+PN_JHD void pixel_bgr(const pn_jpeg_desc &d, const uint8_t *const plane[3], const int pitch[3], int y, int x, uint8_t *bgr) {
+    Scaled g;
+    scaled_geometry(d, 1, &g);
+    pixel_bgr(d, g, plane, pitch, y, x, bgr);
 }
 
 // Where block g (decode order) of an image lands: component and block coordinates in that component's plane.

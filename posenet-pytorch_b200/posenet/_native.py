@@ -101,6 +101,9 @@ _SIGNATURES = {
     "pn_jpeg_workspace": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
     "pn_jpeg_decode": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_void_p,
                                  C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
+    "pn_jpeg_workspace_scaled": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
+    "pn_jpeg_decode_scaled": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                        C.c_int64, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
     "pn_jpeg_encode_bound": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int64)]),
     "pn_jpeg_encode_workspace": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
     "pn_jpeg_encode": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_void_p, C.c_int, C.c_int, C.c_int,

@@ -22,6 +22,13 @@ JPEG files decoded on the GPU instead (``posenet.jpeg``; the records are identic
     pipe = posenet.BatchPipeline(model, 64, stream.height, stream.width, jpeg=True, min_pose_score=0.25)
     for *records, status in pipe.run(b for b, _ in stream.batches()):
         ...                                                       # status[i]: 0 GPU, 1 decoded by cv2 on the host, < 0 malformed
+
+Camera photos decoded at 1/2, 1/4 or 1/8 (``cv2.imread(path, cv2.IMREAD_REDUCED_COLOR_4)``; JPEG files scaled in the DCT domain,
+without a full-size frame anywhere):
+
+    stream = posenet.ImageStream(paths, batch=64, decode="gpu", reduce=4)        # height x width: the REDUCED frame size
+    pipe = posenet.BatchPipeline(model, 64, stream.height, stream.width, jpeg=True, reduce=4, arena_bytes=stream.arena_bytes)
+    ...                                                           # coordinates refer to the reduced frames
 """
 import concurrent.futures
 import ctypes as C
@@ -33,15 +40,17 @@ import numpy as np
 import torch
 
 from posenet import _native as nat
+from posenet.jpeg import imread_flag, reduced_size
 
 
 class EncodedBatch:
     """One batch of files as ``ImageStream(decode="gpu")`` hands it to ``BatchPipeline(jpeg=True)``: the bytes of the files the GPU
     decodes packed into a pinned byte arena (``arena[:used]``), their descriptors (``descs``, pinned uint8, one pn_jpeg_desc per
-    row; rows the GPU does not decode are marked host), and the frames cv2 decoded on the host (``raw`` rows ``host_rows``)."""
+    row; rows the GPU does not decode are marked host), and the frames cv2 decoded on the host (``raw`` rows ``host_rows``).
+    ``reduce``: the scale the frames are decoded at (1 / reduce), the stream's."""
 
-    def __init__(self, arena, descs, raw, batch):
-        self.arena, self.descs, self.raw, self.batch = arena, descs, raw, batch
+    def __init__(self, arena, descs, raw, batch, reduce=1):
+        self.arena, self.descs, self.raw, self.batch, self.reduce = arena, descs, raw, batch, reduce
         self.used = 0
         self.host_rows = []
         self.shapes = [None] * batch
@@ -59,7 +68,8 @@ class EncodedBatch:
 
 
 class ImageStream:
-    def __init__(self, paths, batch, height=None, width=None, workers=None, slots=4, keep=2, pinned=None, mixed=False, decode="cv2"):
+    def __init__(self, paths, batch, height=None, width=None, workers=None, slots=4, keep=2, pinned=None, mixed=False, decode="cv2",
+                 reduce=1, arena_bytes=None):
         """``mixed``: the files may have different sizes (each at most ``height`` x ``width``); a batch row then holds its frame
         contiguously at the frame's own size and ``batches()`` also yields the list of ``(h, w)`` -- the input format of a
         ``BatchPipeline(..., mixed=True)``, which resizes every frame on the GPU like ``_process_input`` (utils.py:13-26) does.
@@ -69,17 +79,27 @@ class ImageStream:
         batches decode ahead on the thread pool.  ``BatchPipeline.run`` (depth d) copies batch i to the device asynchronously
         and only blocks on it after taking batch i + d, so ``keep >= d`` is what makes the reuse safe (defaults: d = 2).
 
-        ``decode="gpu"``: the workers only read each file into the batch's pinned byte arena (``batch * height * width * 3``
-        bytes, the size of a decoded batch) and parse its headers; ``batches()`` yields an ``EncodedBatch`` in place of the
+        ``decode="gpu"``: the workers only read each file into the batch's pinned byte arena (``arena_bytes``, below) and parse
+        its headers; ``batches()`` yields an ``EncodedBatch`` in place of the
         uint8 tensor, for a ``BatchPipeline(..., jpeg=True)`` to decode on the GPU.  Files the GPU does not decode (not baseline
         JPEG, EXIF-rotated, ...; ``posenet.jpeg``) or that do not fit the arena's remaining space are decoded by cv2.imread into
-        their row of a pinned side buffer.  Size checks and errors are those of ``decode="cv2"``."""
+        their row of a pinned side buffer.  Size checks and errors are those of ``decode="cv2"``.
+
+        ``reduce`` (1, 2, 4 or 8): every file is decoded at 1 / reduce, as ``cv2.imread(path, cv2.IMREAD_REDUCED_COLOR_<reduce>)``
+        does (JPEG files: ceil(h / reduce) x ceil(w / reduce), scaled in the DCT domain).  ``height`` / ``width`` are then the
+        REDUCED frame size (taken from the first file read with that flag when not given), and size checks apply to it; pose
+        coordinates downstream refer to the reduced frames.  With ``decode="gpu"`` the decode runs at that scale on the device.
+        ``arena_bytes``: the pinned byte arena per batch of ``decode="gpu"`` (``self.arena_bytes``; a ``BatchPipeline`` needs a
+        decoder arena at least as large).  Default: ``batch * height * width * 3`` at ``reduce=1``; otherwise ``batch *
+        (reduce * height) * (reduce * width)``, room for full-size camera files of about a byte per pixel."""
+        self.flag = imread_flag(reduce)
+        self.reduce = int(reduce)
         self.paths = list(paths)
         assert self.paths, "no image files"
         self.batch = int(batch)
         assert not (mixed and (height is None or width is None)), "mixed=True needs the largest frame size (height, width)"
         if height is None or width is None:
-            first = cv2.imread(self.paths[0])
+            first = cv2.imread(self.paths[0], self.flag)
             if first is None:
                 raise IOError("Image file not found or unreadable: %s" % self.paths[0])     # utils.py:36-37
             height, width = first.shape[:2]
@@ -97,13 +117,18 @@ class ImageStream:
         self._shapes = [[None] * self.batch for _ in self._bufs]
         assert decode in ("cv2", "gpu"), "decode is 'cv2' or 'gpu'"
         self.decode = decode
+        if arena_bytes is None:
+            r = self.reduce
+            arena_bytes = self._bufs[0].numel() if r == 1 else self.batch * (r * self.height) * (r * self.width)
+        self.arena_bytes = int(arena_bytes)
+        assert self.arena_bytes > 0, "arena_bytes must be positive"
         self._enc = []
         if decode == "gpu":
             for b in self._bufs:
-                arena = torch.empty(b.numel(), dtype=torch.uint8)
+                arena = torch.empty(self.arena_bytes, dtype=torch.uint8)
                 descs = torch.empty(self.batch * C.sizeof(nat.JpegDesc), dtype=torch.uint8)
                 self._enc.append(EncodedBatch(arena.pin_memory() if pinned else arena, descs.pin_memory() if pinned else descs, b,
-                                              self.batch))
+                                              self.batch, self.reduce))
 
     def __len__(self):
         return (len(self.paths) + self.batch - 1) // self.batch
@@ -139,18 +164,19 @@ class ImageStream:
             d = nat.JpegDesc()
             nat.check(nat.load().pn_jpeg_parse(view.ctypes.data, size, C.byref(d)), "pn_jpeg_parse")
             if d.kind == nat.JPEG_SUPPORTED:
-                self._check_size(path, d.height, d.width)
+                h, w = reduced_size(d.height, d.width, self.reduce)
+                self._check_size(path, h, w)
                 d.file_offset = off
                 k = C.sizeof(nat.JpegDesc)
                 enc.descs.numpy()[row * k:(row + 1) * k] = np.frombuffer(bytes(d), np.uint8)
-                enc.shapes[row] = (d.height, d.width)
+                enc.shapes[row] = (h, w)
                 return
         self._load(path, enc.raw.numpy()[row], enc.shapes, row)
         with enc.lock:
             enc.host_rows.append(row)
 
     def _load(self, path, dst, shapes, row):
-        img = cv2.imread(path)
+        img = cv2.imread(path, self.flag)
         if img is None:
             raise IOError("Image file not found or unreadable: %s" % path)
         if self.mixed:

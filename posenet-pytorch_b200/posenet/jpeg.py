@@ -1,8 +1,9 @@
-"""Baseline JPEG decode on the GPU, bit-exact with ``cv2.imdecode(buf, cv2.IMREAD_COLOR)`` (``pn_jpeg_parse`` / ``pn_jpeg_decode``),
-and encode, bit-exact with ``cv2.imencode(".jpg", frame, params)`` (``pn_jpeg_encode``).
+"""Baseline JPEG decode on the GPU, bit-exact with ``cv2.imdecode(buf, cv2.IMREAD_COLOR)`` (``pn_jpeg_parse`` / ``pn_jpeg_decode``)
+and, at 1/2, 1/4, 1/8, with ``cv2.IMREAD_REDUCED_COLOR_*`` (``pn_jpeg_decode_scaled``), and encode, bit-exact with ``cv2.imencode(".jpg", frame, params)`` (``pn_jpeg_encode``).
 
     frames, status = posenet.imdecode_batch(buffers)                  # files of one size: CUDA uint8 [N, h, w, 3]
     rows, status, shapes = posenet.imdecode_batch(buffers)            # sizes differ: row i holds frame i at its own size
+    frames, status = posenet.imdecode_batch(buffers, reduce=4)        # at 1/4 (cv2.IMREAD_REDUCED_COLOR_4), ceil(h/4) x ceil(w/4)
 
 ``status[i]``: 0 decoded on the GPU, 1 decoded by cv2 on the host (progressive, arithmetic-coded, 12-bit, CMYK / RGB-coded,
 EXIF-rotated or truncated files, anything the parser does not know) and uploaded, < 0 the file's entropy-coded data is
@@ -17,6 +18,22 @@ import torch
 
 from posenet import _native as nat
 from posenet.imencode import encode_files
+
+
+REDUCE_FLAGS = {1: cv2.IMREAD_COLOR, 2: cv2.IMREAD_REDUCED_COLOR_2, 4: cv2.IMREAD_REDUCED_COLOR_4,
+                8: cv2.IMREAD_REDUCED_COLOR_8}
+
+
+def imread_flag(reduce):
+    """The cv2 imread / imdecode flag of a ``reduce`` factor (1, 2, 4 or 8); ValueError for any other."""
+    if isinstance(reduce, bool) or reduce not in REDUCE_FLAGS:
+        raise ValueError("reduce=%r: the decoders scale by 1, 2, 4 or 8 (cv2.IMREAD_REDUCED_COLOR_*)" % (reduce,))
+    return REDUCE_FLAGS[reduce]
+
+
+def reduced_size(h, w, reduce):
+    """The frame size of an h x w JPEG file decoded at 1 / reduce: ceil(h / reduce) x ceil(w / reduce)."""
+    return -(-int(h) // reduce), -(-int(w) // reduce)
 
 
 def parse(buf):
@@ -34,33 +51,42 @@ def desc_bytes(descs):
 
 
 class Decoder:
-    """Device buffers for ``pn_jpeg_decode`` at a fixed capacity: ``batch`` files of together at most ``arena_bytes`` bytes,
-    none larger than ``max_h`` x ``max_w``.  ``decode`` enqueues on the current stream."""
+    """Device buffers for ``pn_jpeg_decode_scaled`` at a fixed capacity: ``batch`` files of together at most ``arena_bytes``
+    bytes, decoded at 1 / ``reduce`` to frames of at most ``max_h`` x ``max_w`` (files up to ``reduce * max_h`` x
+    ``reduce * max_w``).  ``decode`` enqueues on the current stream."""
 
-    def __init__(self, batch, arena_bytes, max_h, max_w, device=None):
+    def __init__(self, batch, arena_bytes, max_h, max_w, device=None, reduce=1):
+        imread_flag(reduce)
         self.batch, self.arena_bytes, self.max_h, self.max_w = int(batch), int(arena_bytes), int(max_h), int(max_w)
+        self.reduce = int(reduce)
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         n = C.c_size_t()
-        nat.check(nat.load().pn_jpeg_workspace(self.batch, self.arena_bytes, self.max_h, self.max_w, C.byref(n)), "pn_jpeg_workspace")
+        nat.check(nat.load().pn_jpeg_workspace_scaled(self.batch, self.arena_bytes, self.max_h, self.max_w, self.reduce, C.byref(n)),
+                  "pn_jpeg_workspace_scaled")
         self.ws = torch.empty(n.value, dtype=torch.uint8, device=dev)
         self.arena = torch.empty(self.arena_bytes, dtype=torch.uint8, device=dev)
         self.descs = torch.empty(self.batch * C.sizeof(nat.JpegDesc), dtype=torch.uint8, device=dev)
         self.status = torch.empty(self.batch, dtype=torch.int32, device=dev)
 
     def decode(self, frames, frame_stride, frame_hw=None):
-        """Enqueue pn_jpeg_decode of ``self.arena`` / ``self.descs`` (filled by the caller) into ``frames``."""
-        nat.check(nat.load().pn_jpeg_decode(
+        """Enqueue pn_jpeg_decode_scaled of ``self.arena`` / ``self.descs`` (filled by the caller) into ``frames``."""
+        nat.check(nat.load().pn_jpeg_decode_scaled(
             C.c_void_p(self.arena.data_ptr()), self.arena_bytes, C.c_void_p(self.descs.data_ptr()), self.batch, self.max_h,
-            self.max_w, C.c_void_p(frames.data_ptr()), int(frame_stride),
+            self.max_w, self.reduce, C.c_void_p(frames.data_ptr()), int(frame_stride),
             C.c_void_p(frame_hw.data_ptr()) if frame_hw is not None else None, C.c_void_p(self.ws.data_ptr()), self.ws.numel(),
-            C.c_void_p(self.status.data_ptr()), nat.stream_ptr()), "pn_jpeg_decode")
+            C.c_void_p(self.status.data_ptr()), nat.stream_ptr()), "pn_jpeg_decode_scaled")
 
 
-def imdecode_batch(buffers, device=None):
+def imdecode_batch(buffers, device=None, reduce=1):
     """Decode the JPEG files in ``buffers`` (bytes / uint8 arrays) on the GPU.  Returns ``(frames, status)`` when all frames
     share one size (frames: CUDA uint8 [N, h, w, 3]), else ``(rows, status, shapes)``: rows is CUDA uint8 [N, H * W * 3] (H x W
     the largest frame) with frame i stored contiguously from the start of row i, shapes the list of (h_i, w_i).  status: CUDA
-    int32 [N].  Files cv2 cannot decode at all raise ValueError."""
+    int32 [N].  Files cv2 cannot decode at all raise ValueError.
+
+    ``reduce`` (1, 2, 4 or 8; anything else is a ValueError): decode at 1 / reduce, frame i equal to ``cv2.imdecode(buf,
+    cv2.IMREAD_REDUCED_COLOR_<reduce>)`` -- ceil(h / reduce) x ceil(w / reduce) for JPEG files, scaled in the DCT domain.  Rows
+    cv2 decodes on the host (status 1: progressive, EXIF-rotated, PNG, ...) are cv2's reduced decode too."""
+    flag = imread_flag(reduce)
     nat.require_device()
     bufs = [np.frombuffer(b, np.uint8) if not isinstance(b, np.ndarray) else np.ascontiguousarray(b, np.uint8).reshape(-1)
             for b in buffers]
@@ -72,16 +98,16 @@ def imdecode_batch(buffers, device=None):
         if d.kind == nat.JPEG_SUPPORTED:
             d.file_offset = offset
             offset += b.size
-            shapes.append((d.height, d.width))
+            shapes.append(reduced_size(d.height, d.width, reduce))
         else:
-            img = cv2.imdecode(b, cv2.IMREAD_COLOR)
+            img = cv2.imdecode(b, flag)
             if img is None:
                 raise ValueError("buffer %d is not an image cv2 can decode" % i)
             host_imgs[i] = img
             shapes.append(img.shape[:2])
         descs.append(d)
     H, W = max(s[0] for s in shapes), max(s[1] for s in shapes)
-    dec = Decoder(len(bufs), max(offset, 1), H, W, device)
+    dec = Decoder(len(bufs), max(offset, 1), H, W, device, reduce)
     dev = dec.arena.device
     if offset:
         arena = torch.from_numpy(np.concatenate([b for b, d in zip(bufs, descs) if d.kind == nat.JPEG_SUPPORTED]))

@@ -27,7 +27,8 @@ from posenet.decode_multi import decode_multiple_poses_batch, split_pose_records
 
 class BatchPipeline:
     def __init__(self, model, batch, height, width, depth=2, use_graph=True, output_stride=None, scale_factor=1.0,
-                 source_coords=False, mixed=False, gather=False, group=None, overlay=None, jpeg=False, encode=None, encode_ext=".jpg", **decode_kw):
+                 source_coords=False, mixed=False, gather=False, group=None, overlay=None, jpeg=False, encode=None, encode_ext=".jpg",
+                 reduce=1, arena_bytes=None, **decode_kw):
         """``height`` x ``width``: size of the uint8 frames handed to ``submit`` (``mixed=True``: the LARGEST frame; each
         frame of a batch then comes with its own size).  The network runs at ``valid_resolution(width * scale_factor,
         height * scale_factor)`` (utils.py:7-10); frames of any other size go through the bit-exact cv2 resize
@@ -46,6 +47,12 @@ class BatchPipeline:
         the bytes of the files in use, their descriptors and the rows cv2 decoded on the host; ``pn_jpeg_decode`` writes the
         frames into the step's input buffer (same layout as the uint8 batches) on the compute stream, just before the step.
         ``result`` appends the int32 decode status ``[batch]`` as its last item (0 GPU, 1 host, < 0 malformed: a zero frame).
+        ``reduce`` (with ``jpeg``; 1, 2, 4 or 8): the stream's ``reduce``.  The files are decoded at 1 / reduce
+        (``pn_jpeg_decode_scaled``, bit-exact with ``cv2.imread(path, cv2.IMREAD_REDUCED_COLOR_<reduce>)``) and ``height`` x
+        ``width`` are the reduced frame size.  Everything downstream -- resize, records, ``source_coords``, overlay, encode --
+        works on the reduced frames: coordinates refer to them, not to the full-size files.  ``arena_bytes``: the decoder's
+        byte arena, at least the stream's ``arena_bytes`` (default: what ``ImageStream`` allocates for the same batch, size and
+        ``reduce``).  ``submit`` checks both against the ``EncodedBatch``.
         ``encode``: a cv2 ``imencode`` params list (``[]`` for cv2's defaults; needs ``overlay``).  The step's graph also encodes
         the drawn frames as JPEG files (``pn_jpeg_encode``, bit-exact with ``cv2.imencode(".jpg", frame, encode)``), and the
         in-graph device-to-host copy carries the files' offsets instead of the frames.  ``result`` copies exactly the bytes in use
@@ -111,10 +118,16 @@ class BatchPipeline:
                          copied=torch.cuda.Event(), done=torch.cuda.Event(), out=torch.cuda.Event(), graph=None, busy=False)
                 self.slots.append(s)
             self.jpeg = bool(jpeg)
+            assert self.jpeg or (reduce == 1 and arena_bytes is None), "reduce= and arena_bytes= are for jpeg=True pipelines"
             if self.jpeg:
-                from posenet.jpeg import Decoder
+                from posenet.jpeg import Decoder, imread_flag
+                imread_flag(reduce)
+                self.reduce = int(reduce)
+                r = self.reduce
+                if arena_bytes is None:
+                    arena_bytes = self.slots[0]["x"].numel() if r == 1 else self.batch * (r * self.h) * (r * self.w)
                 for s in self.slots:
-                    s["dec"] = Decoder(self.batch, s["x"].numel(), self.h, self.w, dev)
+                    s["dec"] = Decoder(self.batch, int(arena_bytes), self.h, self.w, dev, r)
                     s["status_host"] = torch.zeros(self.batch, dtype=torch.int32).pin_memory()
                     s["h2d_bytes"] = 0
             if self.encode is not None:
@@ -230,7 +243,12 @@ class BatchPipeline:
         if self.jpeg:
             from posenet.ingest import EncodedBatch
             assert isinstance(host_batch, EncodedBatch), "jpeg=True: submit the EncodedBatch of an ImageStream(decode='gpu')"
-            assert host_batch.arena.numel() <= s["dec"].arena_bytes and host_batch.batch == self.batch
+            assert host_batch.batch == self.batch
+            assert host_batch.reduce == self.reduce, \
+                "the stream decodes at 1/%d, the pipeline at 1/%d (reduce=)" % (host_batch.reduce, self.reduce)
+            assert host_batch.arena.numel() <= s["dec"].arena_bytes, \
+                "the stream's arena (%d bytes) exceeds the decoder's (%d): pass arena_bytes=stream.arena_bytes" % (
+                    host_batch.arena.numel(), s["dec"].arena_bytes)
             enc = host_batch
             if self.mixed and shapes is None:
                 shapes = list(enc.shapes[:enc.n_valid])
