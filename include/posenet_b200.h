@@ -273,6 +273,27 @@ int pn_png_encode_workspace(int n_img, int max_h, int max_w, size_t *bytes_host)
 int pn_png_encode(const uint8_t *frames, int n_img, int max_h, int max_w, int64_t frame_stride, const int *frame_hw, uint8_t *out,
                   int64_t out_capacity, int64_t *out_offsets, void *workspace, size_t ws_bytes, pn_stream_t stream);
 
+/* ---- N7: webcam_demo.py read_cap of video frames that arrive as YUV (software decoders give I420, hardware decoders and capture
+ * devices NV12, UVC webcams YUY2): a batch converted to BGR ON THE DEVICE, bit-exact with cv2.cvtColor(frame,
+ * cv2.COLOR_YUV2BGR_<layout>) (BT.601 limited range in 20-bit fixed point, nearest chroma).
+ *
+ * Frame i is read from src + i * src_stride in cv2's own layout (4:2:0: [h * 3 / 2, w], the Y plane then the chroma; 4:2:2:
+ * [h, w, 2]) and written as uint8 BGR HWC [h, w, 3] at dst + i * dst_stride.  w must be even, and h too for 4:2:0 (what cv2
+ * accepts).  src_stride is at least the frame's bytes (h * w * 3 / 2 or h * w * 2), dst_stride at least h * w * 3.  No byte
+ * outside the frames is read or written.
+ * The launch geometry depends only on the arguments, so the call can be captured in a CUDA graph. */
+typedef enum pn_yuv_layout {
+    PN_YUV_I420 = 0, /* Y, U (h/2 x w/2), V; COLOR_YUV2BGR_I420 / _IYUV */
+    PN_YUV_YV12 = 1, /* Y, V, U; COLOR_YUV2BGR_YV12 */
+    PN_YUV_NV12 = 2, /* Y, interleaved UV (h/2 x w); COLOR_YUV2BGR_NV12 */
+    PN_YUV_NV21 = 3, /* Y, interleaved VU; COLOR_YUV2BGR_NV21 */
+    PN_YUV_YUY2 = 4, /* Y0 U Y1 V; COLOR_YUV2BGR_YUY2 / _YUYV / _YUNV */
+    PN_YUV_UYVY = 5, /* U Y0 V Y1; COLOR_YUV2BGR_UYVY / _Y422 / _UYNV */
+    PN_YUV_YVYU = 6  /* Y0 V Y1 U; COLOR_YUV2BGR_YVYU */
+} pn_yuv_layout;
+int pn_yuv_to_bgr(const uint8_t *src, int n_img, int h, int w, int64_t src_stride, int layout, uint8_t *dst, int64_t dst_stride,
+                  pn_stream_t stream);
+
 /* ---- Whole-network plan: mobilenet_v1.py:130-162 (MobileNetV1.__init__/forward) --------------------
  * The layer table is computed by the caller (posenet/models/mobilenet_v1.py mirrors
  * _to_output_strided_layers, mobilenet_v1.py:8-39) and passed in explicitly. */

@@ -17,6 +17,7 @@ from posenet.pipeline import BatchPipeline  # noqa: F401  (streaming batches: co
 from posenet.ingest import ImageStream  # noqa: F401  (threaded image-file decode into pinned batches)
 from posenet.jpeg import imdecode_batch, imencode_batch  # noqa: F401  (baseline JPEG decode / encode on the GPU, bit-exact with cv2)
 from posenet.png import imencode_png_batch  # noqa: F401  (PNG encode on the GPU, bit-exact with cv2)
+from posenet.yuv import yuv_to_bgr_batch  # noqa: F401  (YUV video frames to BGR on the GPU, bit-exact with cv2.cvtColor)
 from posenet.utils import *  # noqa: F401,F403
 from posenet.utils import _process_input, process_input_gpu, resize_u8_gpu  # noqa: F401
 from posenet.utils import draw_skel_and_kp_batch, draw_skeleton_batch  # noqa: F401  (overlays drawn on the GPU)

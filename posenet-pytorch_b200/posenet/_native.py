@@ -22,6 +22,7 @@ JPEG_WHY = {name: i for i, name in enumerate((
     "none", "not_jpeg", "truncated", "progressive", "arithmetic", "lossless", "precision", "multi_scan", "components", "rgb",
     "no_dht", "exif_orientation", "sampling", "bad_table", "unknown"))}
 JPEG_OK, JPEG_SKIPPED = 0, 1
+YUV_I420, YUV_YV12, YUV_NV12, YUV_NV21, YUV_YUY2, YUV_UYVY, YUV_YVYU = range(7)
 
 
 class NativeError(RuntimeError):
@@ -112,6 +113,7 @@ _SIGNATURES = {
     "pn_png_encode_workspace": (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
     "pn_png_encode": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p,
                                 C.c_void_p, C.c_size_t, C.c_void_p]),
+    "pn_yuv_to_bgr": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]),
     "pn_plan_query": (C.c_int, [C.POINTER(NetDesc), C.POINTER(C.c_size_t), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "pn_plan_create": (C.c_int, [C.POINTER(NetDesc), C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p)]),
     "pn_plan_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

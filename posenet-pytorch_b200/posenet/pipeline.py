@@ -10,7 +10,7 @@ This is the batched form of what the reference's ``benchmark.py:32-44`` does per
         ...
 
 Options on top of that (``overlay=`` draws the poses on the frames, ``encode=`` returns them as JPEG files, or as PNG files
-with ``encode_ext=".png"``, ``jpeg=True`` takes JPEG files in): ``source_coords=True`` maps the keypoint coordinates back to the submitted frames ON THE DEVICE
+with ``encode_ext=".png"``, ``jpeg=True`` takes JPEG files in, ``yuv=code`` video frames in YUV): ``source_coords=True`` maps the keypoint coordinates back to the submitted frames ON THE DEVICE
 (``image_demo.py:50``), ``mixed=True`` accepts frames of different sizes in one batch (every file of a directory
 pre-processed at its own size, ``benchmark.py:24-29``), ``gather=True`` all-gathers the records of every rank's shard over
 NCCL inside the step (one process per GPU, ``posenet.sharding``).
@@ -28,7 +28,7 @@ from posenet.decode_multi import decode_multiple_poses_batch, split_pose_records
 class BatchPipeline:
     def __init__(self, model, batch, height, width, depth=2, use_graph=True, output_stride=None, scale_factor=1.0,
                  source_coords=False, mixed=False, gather=False, group=None, overlay=None, jpeg=False, encode=None, encode_ext=".jpg",
-                 reduce=1, arena_bytes=None, **decode_kw):
+                 reduce=1, arena_bytes=None, yuv=None, **decode_kw):
         """``height`` x ``width``: size of the uint8 frames handed to ``submit`` (``mixed=True``: the LARGEST frame; each
         frame of a batch then comes with its own size).  The network runs at ``valid_resolution(width * scale_factor,
         height * scale_factor)`` (utils.py:7-10); frames of any other size go through the bit-exact cv2 resize
@@ -53,6 +53,12 @@ class BatchPipeline:
         works on the reduced frames: coordinates refer to them, not to the full-size files.  ``arena_bytes``: the decoder's
         byte arena, at least the stream's ``arena_bytes`` (default: what ``ImageStream`` allocates for the same batch, size and
         ``reduce``).  ``submit`` checks both against the ``EncodedBatch``.
+        ``yuv``: a ``cv2.COLOR_YUV2BGR_*`` code of a 4:2:0 or 4:2:2 layout (I420 / IYUV, YV12, NV12, NV21, YUY2 / YUYV / YUNV,
+        UYVY / Y422 / UYNV, YVYU).  ``submit`` then takes uint8 batches of video frames in cv2's input layout of that code
+        (``[batch, h*3/2, w]`` or ``[batch, h, w, 2]``; ``height`` x ``width`` stay the BGR frame size, both even).  The host-to-device
+        copy carries only those 1.5 or 2 bytes a pixel, and the step's first launch converts them into the BGR frames
+        (``pn_yuv_to_bgr``, bit-exact with ``cv2.cvtColor(frame, yuv)``).  Everything downstream -- resize, records,
+        ``source_coords``, overlay, encode, gather -- works on the converted frames.  Not with ``jpeg`` or ``mixed``.
         ``encode``: a cv2 ``imencode`` params list (``[]`` for cv2's defaults; needs ``overlay``).  The step's graph also encodes
         the drawn frames as JPEG files (``pn_jpeg_encode``, bit-exact with ``cv2.imencode(".jpg", frame, encode)``), and the
         in-graph device-to-host copy carries the files' offsets instead of the frames.  ``result`` copies exactly the bytes in use
@@ -61,6 +67,13 @@ class BatchPipeline:
         do raise ValueError here.
         ``encode_ext``: ``".jpg"`` (the default) or ``".png"``: the files are then PNG (``pn_png_encode``, bit-exact with
         ``cv2.imencode(".png", frame)``; ``encode`` must be ``[]``)."""
+        self.yuv = None
+        if yuv is not None:
+            from posenet import yuv as yuv_mod
+            self.yuv = yuv_mod.layout_of(yuv)
+            if jpeg or mixed:
+                raise ValueError("yuv= takes video frames of one size: not with jpeg=True or mixed=True")
+            self.yuv_bytes = int(np.prod(yuv_mod.frame_shape(self.yuv, int(height), int(width))))
         nat.require_device()
         assert depth >= 1
         self.model, self.batch, self.h, self.w = model, int(batch), int(height), int(width)
@@ -114,6 +127,7 @@ class BatchPipeline:
                          if self.overlay and self.encode is None else None,
                          hw=torch.zeros((self.batch, 2), dtype=torch.int32, device=dev) if self.overlay and self.mixed else None,
                          hw_host=torch.zeros((self.batch, 2), dtype=torch.int32).pin_memory() if self.overlay and self.mixed else None,
+                         yuv=torch.empty(self.batch * self.yuv_bytes, dtype=torch.uint8, device=dev) if self.yuv is not None else None,
                          shapes=None,
                          copied=torch.cuda.Event(), done=torch.cuda.Event(), out=torch.cuda.Event(), graph=None, busy=False)
                 self.slots.append(s)
@@ -140,7 +154,7 @@ class BatchPipeline:
                     s["offsets_host"] = torch.zeros(self.batch + 1, dtype=torch.int64).pin_memory()
                     s["files_host"] = torch.empty(int(self.batch * self.h * self.w * 3 * min(2.5 * self.file_share, 1)),
                                                   dtype=torch.uint8).pin_memory()
-            self.h2d_bytes_per_batch = self.slots[0]["x"].numel()
+            self.h2d_bytes_per_batch = self.slots[0]["x"].numel() if self.yuv is None else self.slots[0]["yuv"].numel()
             self.d2h_bytes_per_batch = (self.world if self.collect_all else 1) * nrec * 8
             if self.overlay and self.encode is None:
                 self.d2h_bytes_per_batch += self.slots[0]["x"].numel()         # mixed mode copies only the bytes in use
@@ -154,6 +168,8 @@ class BatchPipeline:
             with torch.cuda.stream(self.compute):
                 for s in self.slots:
                     s["x"].zero_()
+                    if self.yuv is not None:
+                        s["yuv"].zero_()
                     if self.mixed:
                         s["xr"].zero_()
                     self._enqueue(s)
@@ -168,10 +184,13 @@ class BatchPipeline:
         self._next = 0
 
     def _enqueue(self, s):
-        """The captured part of a step: (uniform resize ->) stem .. heads -> candidates -> greedy decode (-> coordinate scaling)
-        (-> overlay on the submitted frames)."""
+        """The captured part of a step: (YUV -> BGR ->) (uniform resize ->) stem .. heads -> candidates -> greedy decode
+        (-> coordinate scaling) (-> overlay on the submitted frames)."""
         x = s["x"]
         lib = nat.load()
+        if self.yuv is not None:
+            from posenet.yuv import convert
+            convert(s["yuv"], self.batch, self.h, self.w, self.yuv, x)
         if self.resize and not self.mixed:
             nat.check(lib.pn_resize_u8(x.data_ptr(), self.batch, self.h, self.w, self.th, self.tw, s["xr"].data_ptr(),
                                        nat.stream_ptr()), "pn_resize_u8")
@@ -231,8 +250,8 @@ class BatchPipeline:
         s["h2d_bytes"] = n
 
     def submit(self, host_batch, shapes=None):
-        """Enqueue one batch (uint8 [batch,h,w,3], ideally pinned).  Returns a ticket for ``result``; if the slot is
-        still in flight its previous result must have been collected.
+        """Enqueue one batch (uint8 [batch,h,w,3], ideally pinned; with ``yuv``, the frames in cv2's YUV layout).  Returns a
+        ticket for ``result``; if the slot is still in flight its previous result must have been collected.
 
         ``mixed=True``: ``host_batch`` is uint8 ``[batch, h*w*3]`` (or ``[batch,h,w,3]``) whose row i starts with frame i
         stored contiguously at its own size ``shapes[i] = (h_i, w_i)`` (``h_i <= h``, ``w_i <= w``); rows without a frame
@@ -253,7 +272,7 @@ class BatchPipeline:
             if self.mixed and shapes is None:
                 shapes = list(enc.shapes[:enc.n_valid])
         else:
-            assert host_batch.numel() == s["x"].numel() and host_batch.dtype == torch.uint8
+            assert host_batch.numel() == (s["x"] if self.yuv is None else s["yuv"]).numel() and host_batch.dtype == torch.uint8
         if self.mixed:
             assert shapes is not None and len(shapes) <= self.batch, "mixed=True: pass the (h, w) of every frame"
             shapes = [(int(h), int(w)) for h, w in shapes]
@@ -284,6 +303,8 @@ class BatchPipeline:
                     s["x"].view(self.batch, -1)[:len(shapes), :used].copy_(host_batch.view(self.batch, -1)[:len(shapes), :used],
                                                                           non_blocking=True)
                     s["scales"].copy_(sc, non_blocking=True)
+                elif self.yuv is not None:
+                    s["yuv"].copy_(host_batch.view(-1), non_blocking=True)
                 elif not self.mixed:
                     s["x"].copy_(host_batch.view(s["x"].shape), non_blocking=True)
                 if self.overlay and self.mixed:
