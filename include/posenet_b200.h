@@ -164,8 +164,8 @@ int pn_draw_poses(uint8_t *frames, int n_img, int h, int w, int64_t frame_stride
  *
  * pn_jpeg_parse (host only, no device needed) reads a file's headers into a descriptor and classifies it: PN_JPEG_SUPPORTED
  * (1- or 3-component YCbCr / grayscale, 8-bit, baseline / extended Huffman, one interleaved scan, sampling factors 1..4 x 1..2 with
- * integral ratios, EXIF orientation 1 or absent, ending in an EOI) or PN_JPEG_HOST with a PN_JPEG_WHY_* reason; host files are for
- * cv2 to decode.  The descriptor carries everything the device needs: geometry, quantisation tables (natural order) and the derived
+ * integral ratios, EXIF orientation 1 or absent -- or certain, with pn_jpeg_parse_oriented --, ending in an EOI) or PN_JPEG_HOST
+ * with a PN_JPEG_WHY_* reason; host files are for cv2 to decode.  The descriptor carries everything the device needs: geometry, quantisation tables (natural order) and the derived
  * Huffman tables (validated like jpeg_make_d_derived_tbl). */
 enum { PN_JPEG_SUPPORTED = 0, PN_JPEG_HOST = 1 };
 enum {
@@ -204,13 +204,24 @@ typedef struct pn_jpeg_desc {
     int64_t file_bytes;
     int64_t scan_offset;      /* first entropy-coded byte, from the start of the file */
     pn_jpeg_comp comp[3];     /* in frame (SOF) order: Y, Cb, Cr */
-    uint8_t mcu_comp[PN_JPEG_MAX_BLOCKS], mcu_bx[PN_JPEG_MAX_BLOCKS], mcu_by[PN_JPEG_MAX_BLOCKS], pad[2];
+    uint8_t mcu_comp[PN_JPEG_MAX_BLOCKS], mcu_bx[PN_JPEG_MAX_BLOCKS], mcu_by[PN_JPEG_MAX_BLOCKS];
+    uint8_t orientation;      /* EXIF orientation the decode applies (cv2's): 0 or 1 none, 2..8 (pn_jpeg_parse_oriented) */
+    uint8_t pad[1];
     int16_t quant[3][64];     /* per component, natural order (libjpeg's ISLOW_MULT_TYPE) */
     pn_jpeg_huff huff[4];
 } pn_jpeg_desc;
 
-/* Parse the headers of one file (HOST pointers).  PN_OK whatever the classification; PN_ERR_ARG for null pointers. */
+/* Parse the headers of one file (HOST pointers).  PN_OK whatever the classification; PN_ERR_ARG for null pointers.  A file with an
+ * Exif APP1 segment that cannot be read or gives an orientation other than 1 is PN_JPEG_HOST (PN_JPEG_WHY_EXIF_ORIENTATION);
+ * desc->orientation is 0. */
 int pn_jpeg_parse(const uint8_t *file_host, int64_t nbytes, pn_jpeg_desc *desc_host);
+/* The same, except that a file whose EXIF orientation o in 2..8 is certain is PN_JPEG_SUPPORTED with desc->orientation = o, and
+ * is decoded rotated / flipped as cv2.imread does (out(y, x) of the H x W frame r: 2 r(y, W-1-x), 3 r(H-1-y, W-1-x), 4 r(H-1-y, x),
+ * 5 r(x, y), 6 r(H-1-x, y), 7 r(H-1-x, W-1-y), 8 r(x, W-1-y); 5..8 are W x H).  Certain: every Exif segment is readable (II / MM,
+ * 42, IFD0 and all its entries inside the segment), each has at most one 0x0112 entry, a SHORT with count 1 whose preceding
+ * entries are in TIFF order, of known types, with their data inside the segment, and all such entries agree.  Other files with an
+ * orientation other than 1 stay PN_JPEG_HOST as with pn_jpeg_parse. */
+int pn_jpeg_parse_oriented(const uint8_t *file_host, int64_t nbytes, pn_jpeg_desc *desc_host);
 /* Device workspace (bytes, 256-byte aligned base) pn_jpeg_decode needs for up to n_img files of together at most arena_bytes
  * bytes, none larger than max_h x max_w. */
 int pn_jpeg_workspace(int n_img, int64_t arena_bytes, int max_h, int max_w, size_t *bytes_host);
@@ -218,7 +229,7 @@ int pn_jpeg_workspace(int n_img, int64_t arena_bytes, int max_h, int max_w, size
  * of pn_jpeg_parse's descriptors with file_offset filled in.  Frame i is written as uint8 BGR HWC at its own size, contiguous
  * from frames + i * frame_stride (frame_stride >= 3 * max_h * max_w); nothing else in a row and nothing outside the frames is
  * written, and no byte outside a file's range is read, whatever the file contains.  frame_hw (optional, device int32 [n_img, 2])
- * receives each decoded frame's (h, w), (0, 0) for the others; status: device int32 [n_img], PN_JPEG_OK / _SKIPPED / < 0.  The
+ * receives each decoded frame's (h, w) -- after the descriptor's orientation, which max_h x max_w also bound --, (0, 0) for the others; status: device int32 [n_img], PN_JPEG_OK / _SKIPPED / < 0.  The
  * launch geometry depends only on the arguments, not on the descriptors' contents, so the call can be captured in a CUDA graph. */
 int pn_jpeg_decode(const uint8_t *files, int64_t arena_bytes, const pn_jpeg_desc *descs, int n_img, int max_h, int max_w,
                    uint8_t *frames, int64_t frame_stride, int *frame_hw, void *workspace, size_t ws_bytes, int *status,

@@ -16,9 +16,11 @@
 //   dc        one warp per segment: per-component prefix sums of the DC differences (reset at every restart marker)
 //   idct      eight threads per block, into per-component sample planes: jpeg_idct_islow, or at 1/2, 1/4, 1/8 (scale_denom,
 //             cv2's IMREAD_REDUCED_COLOR_*) the component's scaled IDCT (jidctred.c), ssize x ssize samples per block
-//   color     upsampling + YCbCr -> BGR, one thread per output pixel, straight into the frame's row (ceil(h / d) x ceil(w / d))
-// Everything up to dc is independent of the scale.  The workspace is sized for files of scale_denom * max_h x scale_denom * max_w
-// (a file whose reduced frame fits max_h x max_w is at most that large).
+//   color     upsampling + YCbCr -> BGR, one thread per output pixel, straight into the frame's row (ceil(h / d) x ceil(w / d)),
+//             with the descriptor's EXIF orientation applied: flips map each output pixel to its source pixel, transposes stage
+//             32 x 32 tiles through shared memory so that both the planes and the frame are walked along their rows
+// Everything up to dc is independent of the scale and the orientation.  The workspace is sized for files of scale_denom * max_h x
+// scale_denom * max_w in either order (a file whose reduced, oriented frame fits max_h x max_w is at most that large).
 // (Weissenberger & Schmidt, "Massively Parallel Huffman Decoding on GPUs", ICPP 2018, for the self-synchronisation.)
 #include "common.cuh"
 #include "jpeg_decode.cuh"
@@ -66,7 +68,8 @@ Layout layout(int n_img, int64_t arena, int max_h, int max_w) {
     const long long bx = (max_w + 7) / 8, by = (max_h + 7) / 8;
     L.nseg_cap = (long long)n_img * bx * by;
     L.nsub_cap = L.nseg_cap + arena * 8 / SUB_BITS + n_img;
-    L.nblk_cap = (long long)n_img * 3 * (bx + 3) * (by + 1);   // MCU padding of sampling factors up to 4 x 2
+    // MCU padding of sampling factors up to 4 x 2, for a file of max_h x max_w or (transposed orientations) max_w x max_h
+    L.nblk_cap = (long long)n_img * 3 * ((bx + 3) * (by + 1) > (by + 3) * (bx + 1) ? (bx + 3) * (by + 1) : (by + 3) * (bx + 1));
     size_t o = 0;
     auto take = [&](size_t bytes) { const size_t at = o; o = align256(o + bytes); return at; };
     L.totals = take(sizeof(Totals));
@@ -129,9 +132,11 @@ __global__ void __launch_bounds__(32) plan_kernel(Args a, Ws ws) {
         const pn_jpeg_desc &d = a.descs[i];
         bool ok = d.kind == PN_JPEG_SUPPORTED;
         const bool skipped = !ok;
+        const long long rh = ((long long)d.height + a.denom - 1) / a.denom, rw = ((long long)d.width + a.denom - 1) / a.denom;
+        const bool tr = orient_transposes(d.orientation);          // the oriented frame is rw x rh
         ok = ok && d.file_offset >= 0 && d.file_bytes > 0 && d.file_offset + d.file_bytes <= a.arena && d.scan_offset >= 0 &&
-             d.scan_offset < d.file_bytes && d.height >= 1 && (d.height + a.denom - 1) / a.denom <= a.max_h && d.width >= 1 &&
-             (d.width + a.denom - 1) / a.denom <= a.max_w &&
+             d.scan_offset < d.file_bytes && d.height >= 1 && d.width >= 1 && d.orientation <= 8 && (tr ? rw : rh) <= a.max_h &&
+             (tr ? rh : rw) <= a.max_w &&
              (d.ncomp == 1 || d.ncomp == 3) && d.blocks_per_mcu >= 1 && d.blocks_per_mcu <= PN_JPEG_MAX_BLOCKS &&
              d.mcus_x >= 1 && d.mcus_y >= 1 && d.restart_interval >= 1;
         const long long mcus = ok ? (long long)d.mcus_x * d.mcus_y : 0;
@@ -628,23 +633,31 @@ __global__ void __launch_bounds__(THREADS) idct_kernel(Args a, Ws ws) {
     }
 }
 
-// ---- colour: upsampling + YCbCr -> BGR into the frame rows -------------------------------------------------------------------------
+// ---- colour: upsampling + YCbCr -> BGR into the frame rows, in the descriptor's orientation ---------------------------------------
+constexpr int OT = 32;   // transposed orientations: OT x OT output tiles
+
 __global__ void __launch_bounds__(THREADS) color_kernel(Args a, Ws ws) {
+    __shared__ uint32_t tile[OT][OT + 1];
     const int i = blockIdx.y;
     const ImgWs &w = ws.img[i];
     const int st = w.status;
+    const pn_jpeg_desc &d = a.descs[i];
     if (blockIdx.x == 0 && threadIdx.x == 0) {
         a.status[i] = st;
-        if (a.frame_hw) {                   // the frame at 1 / denom
-            a.frame_hw[2 * i] = st == PN_JPEG_OK ? (a.descs[i].height + a.denom - 1) / a.denom : 0;
-            a.frame_hw[2 * i + 1] = st == PN_JPEG_OK ? (a.descs[i].width + a.denom - 1) / a.denom : 0;
+        if (a.frame_hw) {                   // the frame at 1 / denom, oriented
+            int oh = 0, ow = 0;
+            if (st == PN_JPEG_OK)
+                oriented_size(d.orientation, (d.height + a.denom - 1) / a.denom, (d.width + a.denom - 1) / a.denom, &oh, &ow);
+            a.frame_hw[2 * i] = oh;
+            a.frame_hw[2 * i + 1] = ow;
         }
     }
     if (st == PN_JPEG_SKIPPED || st == PN_JPEG_ERR_DESC) return;     // untouched: the host's frame, or no trusted size
-    const pn_jpeg_desc &d = a.descs[i];
     Scaled g;
-    scaled_geometry(d, a.denom, &g);       // plan_kernel checked it
-    const int H = g.h, W = g.w;
+    scaled_geometry(d, a.denom, &g);       // plan_kernel checked it and the orientation
+    const int H = g.h, W = g.w, o = d.orientation;                 // H x W: the decoded frame
+    int OH, OW;
+    oriented_size(o, H, W, &OH, &OW);
     uint8_t *frame = a.frames + (long long)i * a.stride;
     const uint8_t *plane[3];
     int pitch[3];
@@ -653,10 +666,45 @@ __global__ void __launch_bounds__(THREADS) color_kernel(Args a, Ws ws) {
         plane[c] = ws.planes + w.plane_base[c];
         pitch[c] = d.comp[c].bw * g.comp[c].ssize;
     }
-    const long long npx = (long long)H * W;
+    if (st == PN_JPEG_OK && orient_transposes(o)) {
+        // An output row is a source column.  Phase 1 walks the tile's source rows (a warp on 32 consecutive source pixels, i.e. one
+        // output column) into tile[output row][output column]; phase 2 writes the output rows.  Row stride OT + 1: no bank conflicts.
+        const int tiles_x = (OW + OT - 1) / OT, ntiles = tiles_x * ((OH + OT - 1) / OT);
+        for (int t = blockIdx.x; t < ntiles; t += gridDim.x) {
+            const int ty0 = (t / tiles_x) * OT, tx0 = (t % tiles_x) * OT;
+            for (int k = threadIdx.x; k < OT * OT; k += THREADS) {
+                const int ty = k % OT, tx = k / OT, y = ty0 + ty, x = tx0 + tx;
+                if (y < OH && x < OW) {
+                    int sy, sx;
+                    uint8_t bgr[3];
+                    orient_source(o, H, W, y, x, &sy, &sx);
+                    pixel_bgr(d, g, plane, pitch, sy, sx, bgr);
+                    tile[ty][tx] = bgr[0] | (bgr[1] << 8) | ((uint32_t)bgr[2] << 16);
+                }
+            }
+            __syncthreads();
+            for (int k = threadIdx.x; k < OT * OT; k += THREADS) {
+                const int ty = k / OT, tx = k % OT, y = ty0 + ty, x = tx0 + tx;
+                if (y < OH && x < OW) {
+                    const uint32_t v = tile[ty][tx];
+                    uint8_t *px = frame + 3 * ((long long)y * OW + x);
+                    px[0] = (uint8_t)v;
+                    px[1] = (uint8_t)(v >> 8);
+                    px[2] = (uint8_t)(v >> 16);
+                }
+            }
+            __syncthreads();
+        }
+        return;
+    }
+    const long long npx = (long long)OH * OW;
     for (long long p = blockIdx.x * (long long)THREADS + threadIdx.x; p < npx; p += (long long)gridDim.x * THREADS) {
         uint8_t bgr[3] = {0, 0, 0};
-        if (st == PN_JPEG_OK) pixel_bgr(d, g, plane, pitch, (int)(p / W), (int)(p % W), bgr);
+        if (st == PN_JPEG_OK) {
+            int y = (int)(p / OW), x = (int)(p % OW);
+            if (o > 1) orient_source(o, H, W, y, x, &y, &x);   // flips keep the row order
+            pixel_bgr(d, g, plane, pitch, y, x, bgr);
+        }
         frame[3 * p] = bgr[0];
         frame[3 * p + 1] = bgr[1];
         frame[3 * p + 2] = bgr[2];

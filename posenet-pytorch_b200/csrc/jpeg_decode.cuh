@@ -10,6 +10,7 @@
 //   upsampling:    jdsample.c h2v1 / h1v2 / h2v2 fancy, replication otherwise, chosen from the scaled group ratios; context
 //                  rows as jdmainct.c supplies them
 //   colour:        jdcolor.c ycc_rgb_convert (build_ycc_rgb_table, SCALEBITS 16) into B, G, R; grayscale replicated
+//   orientation:   the EXIF flips / transposes cv2.imread applies to the decoded frame, as a map of output to source pixels
 #pragma once
 #include <stdint.h>
 
@@ -497,6 +498,29 @@ PN_JHD void pixel_bgr(const pn_jpeg_desc &d, const uint8_t *const plane[3], cons
     Scaled g;
     scaled_geometry(d, 1, &g);
     pixel_bgr(d, g, plane, pitch, y, x, bgr);
+}
+
+// ---- EXIF orientation (what cv2.imread applies after the decode, at the reduced size too) ------------------------------------------
+// o: pn_jpeg_desc.orientation; 0 and 1 are the identity, 2..4 flips, 5..8 transposes (the frame becomes w x h).
+PN_JHD bool orient_transposes(int o) { return o >= 5 && o <= 8; }
+
+PN_JHD void oriented_size(int o, int h, int w, int *oh, int *ow) {
+    *oh = orient_transposes(o) ? w : h;
+    *ow = orient_transposes(o) ? h : w;
+}
+
+// Pixel (y, x) of the oriented frame -> pixel (*sy, *sx) of the decoded H x W frame.
+PN_JHD void orient_source(int o, int H, int W, int y, int x, int *sy, int *sx) {
+    switch (o) {
+    case 2: *sy = y; *sx = W - 1 - x; break;                  // flip(1)
+    case 3: *sy = H - 1 - y; *sx = W - 1 - x; break;          // flip(-1)
+    case 4: *sy = H - 1 - y; *sx = x; break;                  // flip(0)
+    case 5: *sy = x; *sx = y; break;                          // transpose
+    case 6: *sy = H - 1 - x; *sx = y; break;                  // transpose, flip(1)
+    case 7: *sy = H - 1 - x; *sx = W - 1 - y; break;          // transpose, flip(-1)
+    case 8: *sy = x; *sx = W - 1 - y; break;                  // transpose, flip(0)
+    default: *sy = y; *sx = x;
+    }
 }
 
 // Where block g (decode order) of an image lands: component and block coordinates in that component's plane.

@@ -1,7 +1,8 @@
 // pn_jpeg_parse: the header walk of libjpeg-turbo's jdmarker.c / jdinput.c for the files csrc/jpeg.cu decodes, in host code (no
 // device needed).  Everything that would make libjpeg-turbo (or cv2 around it) do something other than a plain baseline decode --
 // progressive or arithmetic coding, other precisions, several scans, CMYK / RGB colour, EXIF rotation, a warning -- classifies the
-// file PN_JPEG_HOST, so that the GPU path only ever decodes files cv2 reads without comment.
+// file PN_JPEG_HOST, so that the GPU path only ever decodes files cv2 reads without comment.  pn_jpeg_parse_oriented also accepts
+// files whose EXIF rotation is certain (read_exif) and records it for the decode to apply.
 #include <string.h>
 
 #include "common.cuh"
@@ -73,30 +74,57 @@ bool derive(const uint8_t bits[17], const uint8_t *vals, bool is_dc, pn_jpeg_huf
     return true;
 }
 
-// EXIF orientation of an APP1 "Exif\0\0" payload: 1 when absent, 0 when the TIFF structure cannot be read.
-int exif_orientation(const uint8_t *p, int64_t n) {
-    if (n < 14) return 0;
+// What one APP1 "Exif\0\0" payload says about the orientation (tag 0x0112 of IFD0).
+struct Exif {
+    bool readable;   // II / MM, 42, IFD0 and all of its entries inside the payload
+    int tags;        // 0x0112 entries in IFD0
+    int value;       // the first one's value (SHORT), 0 when it has another type; 1 without the tag
+    bool strict;     // every 0x0112 entry is a SHORT with count 1, and cv2 reads up to it (below)
+};
+
+// Bytes of a TIFF field type (1..12), 0 for an unknown type.
+int type_bytes(int type) {
+    static const int kBytes[13] = {0, 1, 1, 2, 4, 8, 1, 1, 2, 4, 8, 4, 8};
+    return type >= 1 && type <= 12 ? kBytes[type] : 0;
+}
+
+Exif read_exif(const uint8_t *p, int64_t n) {
+    Exif e{false, 0, 1, true};
+    if (n < 14) return e;
     const uint8_t *t = p + 6;
     const int64_t tn = n - 6;
     bool le;
     if (t[0] == 'I' && t[1] == 'I') le = true;
     else if (t[0] == 'M' && t[1] == 'M') le = false;
-    else return 0;
+    else return e;
     auto r16 = [&](int64_t o) -> int { return le ? t[o] | (t[o + 1] << 8) : (t[o] << 8) | t[o + 1]; };
     auto r32 = [&](int64_t o) -> int64_t {
         return le ? (int64_t)t[o] | ((int64_t)t[o + 1] << 8) | ((int64_t)t[o + 2] << 16) | ((int64_t)t[o + 3] << 24)
                   : ((int64_t)t[o] << 24) | ((int64_t)t[o + 1] << 16) | ((int64_t)t[o + 2] << 8) | (int64_t)t[o + 3];
     };
-    if (r16(2) != 42) return 0;
+    if (r16(2) != 42) return e;
     const int64_t ifd = r32(4);
-    if (ifd < 8 || ifd + 2 > tn) return 0;
+    if (ifd < 8 || ifd + 2 > tn) return e;
     const int cnt = r16(ifd);
-    if (ifd + 2 + 12ll * cnt > tn) return 0;
+    if (ifd + 2 + 12ll * cnt > tn) return e;
+    e.readable = true;
+    // cv2 reads the entries in order and gives up on the segment at the first one whose data it cannot read.  An entry ahead of
+    // the orientation is taken as read when it is in TIFF order (tag below 0x0112), of a known type, and its data is in the value
+    // field or inside the segment.
+    bool reached = true;
     for (int i = 0; i < cnt; ++i) {
-        const int64_t e = ifd + 2 + 12ll * i;
-        if (r16(e) == 0x0112) return r16(e + 2) == 3 ? r16(e + 8) : 0;
+        const int64_t q = ifd + 2 + 12ll * i;
+        const int tag = r16(q);
+        if (tag != 0x0112) {
+            const int64_t bytes = type_bytes(r16(q + 2)) * r32(q + 4);
+            reached = reached && tag < 0x0112 && type_bytes(r16(q + 2)) && (bytes <= 4 || r32(q + 8) + bytes <= tn);
+            continue;
+        }
+        const bool shrt = r16(q + 2) == 3;
+        if (e.tags++ == 0) e.value = shrt ? r16(q + 8) : 0;
+        e.strict = e.strict && reached && shrt && r32(q + 4) == 1;
     }
-    return 1;
+    return e;
 }
 
 }  // namespace
@@ -104,8 +132,8 @@ int exif_orientation(const uint8_t *p, int64_t n) {
 
 using namespace pn;
 
-extern "C" int pn_jpeg_parse(const uint8_t *file_host, int64_t nbytes, pn_jpeg_desc *d) {
-    PN_CHECK_ARG(file_host && d && nbytes >= 0, "pn_jpeg_parse: null pointer or negative size");
+// oriented: a file whose EXIF orientation o (2..8) is certain is PN_JPEG_SUPPORTED with desc->orientation = o (pn_jpeg_parse_oriented)
+static int parse(const uint8_t *file_host, int64_t nbytes, pn_jpeg_desc *d, bool oriented) {
     memset(d, 0, sizeof(*d));
     d->file_bytes = nbytes;
     const Reader R{file_host, nbytes};
@@ -117,7 +145,12 @@ extern "C" int pn_jpeg_parse(const uint8_t *file_host, int64_t nbytes, pn_jpeg_d
     bool qdef[4] = {};
     int comp_id[3] = {}, comp_h[3] = {}, comp_v[3] = {}, comp_tq[3] = {};
     bool sof = false, jfif = false, adobe = false;
-    int adobe_transform = -1, orientation = 1;
+    int adobe_transform = -1;
+    // EXIF: any Exif segment that is unreadable or says other than 1 sends the file to the host (cv2 takes the first segment with
+    // a readable orientation, looser than read_exif).  The oriented parse keeps a file whose Exif segments are all readable, whose
+    // 0x0112 entries are single SHORTs that cv2 reaches, one per segment, and agree on one value o.
+    bool exif_rotates = false, exif_certain = true;
+    int exif_o = -1;                       // the value of the 0x0112 entries, -1 before the first
     int64_t p = 2;
     for (;;) {
         if (R.u8(p) != 0xFF) return host(d, R.u8(p) < 0 ? PN_JPEG_WHY_TRUNCATED : PN_JPEG_WHY_UNKNOWN);   // extraneous bytes
@@ -185,7 +218,13 @@ extern "C" int pn_jpeg_parse(const uint8_t *file_host, int64_t nbytes, pn_jpeg_d
         } else if (m == 0xE0) {
             if (len - 2 >= 14 && !memcmp(file_host + q, "JFIF\0", 5)) jfif = true;
         } else if (m == 0xE1) {
-            if (len - 2 >= 6 && !memcmp(file_host + q, "Exif\0\0", 6)) orientation = exif_orientation(file_host + q, len - 2);
+            if (len - 2 >= 6 && !memcmp(file_host + q, "Exif\0\0", 6)) {
+                const Exif e = read_exif(file_host + q, len - 2);
+                exif_rotates = exif_rotates || !e.readable || e.value != 1;
+                exif_certain = exif_certain && e.readable && e.strict && e.tags <= 1;
+                if (e.tags && exif_o >= 0 && exif_o != e.value) exif_certain = false;
+                if (e.tags) exif_o = e.value;
+            }
         } else if (m == 0xEE) {
             if (len - 2 >= 12 && !memcmp(file_host + q, "Adobe", 5)) {
                 adobe = true;
@@ -200,7 +239,9 @@ extern "C" int pn_jpeg_parse(const uint8_t *file_host, int64_t nbytes, pn_jpeg_d
             if (ns != d->ncomp) return host(d, PN_JPEG_WHY_MULTI_SCAN);
             if (R.u8(q + 1 + 2 * ns) != 0 || R.u8(q + 2 + 2 * ns) != 63 || R.u8(q + 3 + 2 * ns) != 0)
                 return host(d, PN_JPEG_WHY_UNKNOWN);                                      // Ss, Se, Ah/Al of a sequential scan
-            if (orientation != 1) return host(d, PN_JPEG_WHY_EXIF_ORIENTATION);
+            const int orientation = exif_rotates ? exif_o : 0;
+            if (exif_rotates && !(oriented && exif_certain && orientation >= 2 && orientation <= 8))
+                return host(d, PN_JPEG_WHY_EXIF_ORIENTATION);
             if (d->ncomp == 3) {
                 if (jfif) {
                 } else if (adobe) {
@@ -294,10 +335,21 @@ extern "C" int pn_jpeg_parse(const uint8_t *file_host, int64_t nbytes, pn_jpeg_d
             if (!eoi) return host(d, PN_JPEG_WHY_TRUNCATED);
             d->kind = PN_JPEG_SUPPORTED;
             d->why = PN_JPEG_WHY_NONE;
+            d->orientation = (uint8_t)orientation;
             return PN_OK;
         } else {
             return host(d, PN_JPEG_WHY_UNKNOWN);                                          // DNL, DHP, EXP, JPG, ...
         }
         p = end;
     }
+}
+
+extern "C" int pn_jpeg_parse(const uint8_t *file_host, int64_t nbytes, pn_jpeg_desc *d) {
+    PN_CHECK_ARG(file_host && d && nbytes >= 0, "pn_jpeg_parse: null pointer or negative size");
+    return parse(file_host, nbytes, d, false);
+}
+
+extern "C" int pn_jpeg_parse_oriented(const uint8_t *file_host, int64_t nbytes, pn_jpeg_desc *d) {
+    PN_CHECK_ARG(file_host && d && nbytes >= 0, "pn_jpeg_parse_oriented: null pointer or negative size");
+    return parse(file_host, nbytes, d, true);
 }

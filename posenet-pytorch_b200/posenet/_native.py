@@ -59,11 +59,13 @@ class JpegComp(C.Structure):
 
 
 class JpegDesc(C.Structure):
-    """pn_jpeg_desc: one file's headers as pn_jpeg_parse leaves them (file_offset is the caller's)."""
+    """pn_jpeg_desc: one file's headers as pn_jpeg_parse leaves them (file_offset is the caller's; orientation: the EXIF
+    orientation the decode applies, 0 for none, 2..8 from pn_jpeg_parse_oriented)."""
     _fields_ = [(n, C.c_int32) for n in ("kind", "why", "height", "width", "ncomp", "mcus_x", "mcus_y", "blocks_per_mcu",
                                          "restart_interval", "n_segments")] + \
                [("file_offset", C.c_int64), ("file_bytes", C.c_int64), ("scan_offset", C.c_int64), ("comp", JpegComp * 3),
-                ("mcu_comp", C.c_uint8 * 10), ("mcu_bx", C.c_uint8 * 10), ("mcu_by", C.c_uint8 * 10), ("pad", C.c_uint8 * 2),
+                ("mcu_comp", C.c_uint8 * 10), ("mcu_bx", C.c_uint8 * 10), ("mcu_by", C.c_uint8 * 10), ("orientation", C.c_uint8),
+                ("pad", C.c_uint8 * 1),
                 ("quant", (C.c_int16 * 64) * 3), ("huff", JpegHuff * 4)]
 
 
@@ -99,6 +101,7 @@ _SIGNATURES = {
     "pn_draw_poses": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_int, C.c_double, C.c_double, C.c_int, C.c_void_p]),
     "pn_jpeg_parse": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(JpegDesc)]),
+    "pn_jpeg_parse_oriented": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(JpegDesc)]),
     "pn_jpeg_workspace": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
     "pn_jpeg_decode": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_void_p,
                                  C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),

@@ -29,6 +29,13 @@ without a full-size frame anywhere):
     stream = posenet.ImageStream(paths, batch=64, decode="gpu", reduce=4)        # height x width: the REDUCED frame size
     pipe = posenet.BatchPipeline(model, 64, stream.height, stream.width, jpeg=True, reduce=4, arena_bytes=stream.arena_bytes)
     ...                                                           # coordinates refer to the reduced frames
+
+Phone photos with an EXIF orientation (portraits are stored as landscape scans with orientation 6) rotated on the GPU too, as
+cv2.imread rotates them; a directory of portraits and landscapes has both frame orientations, so it is a mixed stream:
+
+    stream = posenet.ImageStream(paths, batch=64, height=1008, width=1008, mixed=True, decode="gpu", reduce=4, orientation="gpu")
+    pipe = posenet.BatchPipeline(model, 64, 1008, 1008, jpeg=True, mixed=True, reduce=4, arena_bytes=stream.arena_bytes,
+                                 source_coords=True)
 """
 import concurrent.futures
 import ctypes as C
@@ -40,7 +47,7 @@ import numpy as np
 import torch
 
 from posenet import _native as nat
-from posenet.jpeg import imread_flag, reduced_size
+from posenet.jpeg import frame_size, imread_flag, parser
 
 
 class EncodedBatch:
@@ -69,7 +76,7 @@ class EncodedBatch:
 
 class ImageStream:
     def __init__(self, paths, batch, height=None, width=None, workers=None, slots=4, keep=2, pinned=None, mixed=False, decode="cv2",
-                 reduce=1, arena_bytes=None):
+                 reduce=1, arena_bytes=None, orientation="cv2"):
         """``mixed``: the files may have different sizes (each at most ``height`` x ``width``); a batch row then holds its frame
         contiguously at the frame's own size and ``batches()`` also yields the list of ``(h, w)`` -- the input format of a
         ``BatchPipeline(..., mixed=True)``, which resizes every frame on the GPU like ``_process_input`` (utils.py:13-26) does.
@@ -82,8 +89,11 @@ class ImageStream:
         ``decode="gpu"``: the workers only read each file into the batch's pinned byte arena (``arena_bytes``, below) and parse
         its headers; ``batches()`` yields an ``EncodedBatch`` in place of the
         uint8 tensor, for a ``BatchPipeline(..., jpeg=True)`` to decode on the GPU.  Files the GPU does not decode (not baseline
-        JPEG, EXIF-rotated, ...; ``posenet.jpeg``) or that do not fit the arena's remaining space are decoded by cv2.imread into
-        their row of a pinned side buffer.  Size checks and errors are those of ``decode="cv2"``.
+        JPEG, EXIF-rotated unless ``orientation="gpu"``, ...; ``posenet.jpeg``) or that do not fit the arena's remaining space
+        are decoded by cv2.imread into their row of a pinned side buffer.  Size checks and errors are those of ``decode="cv2"``.
+        ``orientation="gpu"`` (with ``decode="gpu"`` only): files whose EXIF orientation is certain are decoded on the GPU and
+        rotated there as cv2.imread rotates them (``pn_jpeg_parse_oriented``); shapes and size checks use the rotated size, so
+        portraits and landscapes need ``mixed=True`` as with ``decode="cv2"``.
 
         ``reduce`` (1, 2, 4 or 8): every file is decoded at 1 / reduce, as ``cv2.imread(path, cv2.IMREAD_REDUCED_COLOR_<reduce>)``
         does (JPEG files: ceil(h / reduce) x ceil(w / reduce), scaled in the DCT domain).  ``height`` / ``width`` are then the
@@ -117,6 +127,10 @@ class ImageStream:
         self._shapes = [[None] * self.batch for _ in self._bufs]
         assert decode in ("cv2", "gpu"), "decode is 'cv2' or 'gpu'"
         self.decode = decode
+        parser(orientation)
+        if orientation == "gpu" and decode != "gpu":
+            raise ValueError("orientation='gpu' rotates files in the GPU decode: it needs decode='gpu'")
+        self.orientation = orientation
         if arena_bytes is None:
             r = self.reduce
             arena_bytes = self._bufs[0].numel() if r == 1 else self.batch * (r * self.height) * (r * self.width)
@@ -162,9 +176,9 @@ class ImageStream:
             raise IOError("Image file not found or unreadable: %s" % path)
         if fits and n == size:
             d = nat.JpegDesc()
-            nat.check(nat.load().pn_jpeg_parse(view.ctypes.data, size, C.byref(d)), "pn_jpeg_parse")
+            nat.check(parser(self.orientation)(view.ctypes.data, size, C.byref(d)), "pn_jpeg_parse")
             if d.kind == nat.JPEG_SUPPORTED:
-                h, w = reduced_size(d.height, d.width, self.reduce)
+                h, w = frame_size(d, self.reduce)
                 self._check_size(path, h, w)
                 d.file_offset = off
                 k = C.sizeof(nat.JpegDesc)

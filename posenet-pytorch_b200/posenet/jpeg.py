@@ -4,10 +4,11 @@ and, at 1/2, 1/4, 1/8, with ``cv2.IMREAD_REDUCED_COLOR_*`` (``pn_jpeg_decode_sca
     frames, status = posenet.imdecode_batch(buffers)                  # files of one size: CUDA uint8 [N, h, w, 3]
     rows, status, shapes = posenet.imdecode_batch(buffers)            # sizes differ: row i holds frame i at its own size
     frames, status = posenet.imdecode_batch(buffers, reduce=4)        # at 1/4 (cv2.IMREAD_REDUCED_COLOR_4), ceil(h/4) x ceil(w/4)
+    out = posenet.imdecode_batch(buffers, orientation="gpu")          # EXIF-rotated files (phone portraits) rotated on the GPU too
 
-``status[i]``: 0 decoded on the GPU, 1 decoded by cv2 on the host (progressive, arithmetic-coded, 12-bit, CMYK / RGB-coded,
-EXIF-rotated or truncated files, anything the parser does not know) and uploaded, < 0 the file's entropy-coded data is
-malformed: its frame is zeros (cv2 decodes such files with a warning; its recovery is not reproduced).
+``status[i]``: 0 decoded on the GPU, 1 decoded by cv2 on the host (progressive, arithmetic-coded, 12-bit, CMYK / RGB-coded or
+truncated files, EXIF-rotated ones unless ``orientation="gpu"``, anything the parser does not know) and uploaded, < 0 the file's
+entropy-coded data is malformed: its frame is zeros (cv2 decodes such files with a warning; its recovery is not reproduced).
 
     files = posenet.imencode_batch(frames, [cv2.IMWRITE_JPEG_QUALITY, 90])   # list of bytes, one per frame"""
 import ctypes as C
@@ -36,11 +37,31 @@ def reduced_size(h, w, reduce):
     return -(-int(h) // reduce), -(-int(w) // reduce)
 
 
-def parse(buf):
-    """pn_jpeg_parse on the bytes of one file: a ``_native.JpegDesc`` (``kind`` JPEG_SUPPORTED / JPEG_HOST, ``why``)."""
+ORIENTATIONS = ("cv2", "gpu")
+
+
+def parser(orientation):
+    """The C parser of an ``orientation`` option: "cv2" (EXIF-rotated files are cv2's, on the host) -> pn_jpeg_parse, "gpu" (files
+    whose EXIF orientation is certain are rotated by the GPU decode, as cv2.imread rotates them) -> pn_jpeg_parse_oriented."""
+    if orientation not in ORIENTATIONS:
+        raise ValueError("orientation=%r: 'cv2' (rotated files decoded on the host) or 'gpu'" % (orientation,))
+    lib = nat.load()
+    return lib.pn_jpeg_parse_oriented if orientation == "gpu" else lib.pn_jpeg_parse
+
+
+def frame_size(desc, reduce):
+    """The frame a SUPPORTED descriptor decodes to at 1 / reduce: the reduced size, transposed for EXIF orientations 5..8."""
+    h, w = reduced_size(desc.height, desc.width, reduce)
+    return (w, h) if 5 <= desc.orientation <= 8 else (h, w)
+
+
+def parse(buf, orientation="cv2"):
+    """pn_jpeg_parse (``orientation="gpu"``: pn_jpeg_parse_oriented) on the bytes of one file: a ``_native.JpegDesc`` (``kind``
+    JPEG_SUPPORTED / JPEG_HOST, ``why``, ``orientation``)."""
+    fn = parser(orientation)
     a = np.frombuffer(buf, np.uint8) if not isinstance(buf, np.ndarray) else np.ascontiguousarray(buf, np.uint8).reshape(-1)
     d = nat.JpegDesc()
-    nat.check(nat.load().pn_jpeg_parse(a.ctypes.data if a.size else C.c_void_p(1), a.size, C.byref(d)), "pn_jpeg_parse")
+    nat.check(fn(a.ctypes.data if a.size else C.c_void_p(1), a.size, C.byref(d)), "pn_jpeg_parse")
     return d
 
 
@@ -77,7 +98,7 @@ class Decoder:
             C.c_void_p(self.status.data_ptr()), nat.stream_ptr()), "pn_jpeg_decode_scaled")
 
 
-def imdecode_batch(buffers, device=None, reduce=1):
+def imdecode_batch(buffers, device=None, reduce=1, orientation="cv2"):
     """Decode the JPEG files in ``buffers`` (bytes / uint8 arrays) on the GPU.  Returns ``(frames, status)`` when all frames
     share one size (frames: CUDA uint8 [N, h, w, 3]), else ``(rows, status, shapes)``: rows is CUDA uint8 [N, H * W * 3] (H x W
     the largest frame) with frame i stored contiguously from the start of row i, shapes the list of (h_i, w_i).  status: CUDA
@@ -85,8 +106,13 @@ def imdecode_batch(buffers, device=None, reduce=1):
 
     ``reduce`` (1, 2, 4 or 8; anything else is a ValueError): decode at 1 / reduce, frame i equal to ``cv2.imdecode(buf,
     cv2.IMREAD_REDUCED_COLOR_<reduce>)`` -- ceil(h / reduce) x ceil(w / reduce) for JPEG files, scaled in the DCT domain.  Rows
-    cv2 decodes on the host (status 1: progressive, EXIF-rotated, PNG, ...) are cv2's reduced decode too."""
+    cv2 decodes on the host (status 1: progressive, EXIF-rotated, PNG, ...) are cv2's reduced decode too.
+
+    ``orientation``: "cv2" (default) leaves files with an EXIF orientation other than 1 to cv2 on the host; "gpu" decodes those
+    whose orientation is certain on the GPU, flipped / rotated as cv2 does (frame i is then the rotated frame, w x h for
+    orientations 5..8; the rest stay cv2's).  Anything else is a ValueError."""
     flag = imread_flag(reduce)
+    parser(orientation)
     nat.require_device()
     bufs = [np.frombuffer(b, np.uint8) if not isinstance(b, np.ndarray) else np.ascontiguousarray(b, np.uint8).reshape(-1)
             for b in buffers]
@@ -94,11 +120,11 @@ def imdecode_batch(buffers, device=None, reduce=1):
     descs, host_imgs, shapes = [], {}, []
     offset = 0
     for i, b in enumerate(bufs):
-        d = parse(b)
+        d = parse(b, orientation)
         if d.kind == nat.JPEG_SUPPORTED:
             d.file_offset = offset
             offset += b.size
-            shapes.append(reduced_size(d.height, d.width, reduce))
+            shapes.append(frame_size(d, reduce))
         else:
             img = cv2.imdecode(b, flag)
             if img is None:
