@@ -231,10 +231,8 @@ int pn_plan_create(const pn_net_desc *desc, void *arena, size_t arena_bytes, pn_
             snprintf(p->names[p->launches++], sizeof(p->names[0]), "stem");
             continue;
         }
-        // Fuse a block when the depthwise work is done once per tile (sep_fuse_recommended; PN_SEP_ALL=1 fuses every
-        // supported block)
-        S.fused = desc->dtype == PN_BF16 && !(desc->flags & PN_PLAN_UNFUSED) && sep_supported(L.cin, L.cout, L.stride, L.dilation) &&
-                  (sep_fuse_recommended(L.cin, L.cout, L.stride, L.dilation) || getenv("PN_SEP_ALL") != nullptr);
+        // Fuse a block when the depthwise work is done once per tile (sep_fuse_recommended)
+        S.fused = desc->dtype == PN_BF16 && !(desc->flags & PN_PLAN_UNFUSED) && sep_fuse_recommended(L.cin, L.cout, L.stride, L.dilation);
         if (S.fused) {
             rc = sep_prepare(&S.sep, p->buf[cur], L.dw_w, L.dw_b, L.pw_w, p->buf[cur ^ 1], desc->n, S.h_in, S.w_in, L.cin, L.cout,
                              L.stride, L.dilation);

@@ -186,16 +186,14 @@ int sepwarp_launch(const SepWarpOp *op, const float *dw_w, const float *dw_b, co
                    cudaStream_t s);
 void sepwarp_describe(const SepWarpOp *op, char *out, size_t cap);
 
-// fused block with the depthwise on the tensor pipe (septc.cu): stride 1, dilation 1 / 2, cin / cout multiples of 64 (<= 512)
+// fused block with the depthwise on the tensor pipe (septc.cu): stride 1, dilation 1 / 2, cin = cout = 256
 struct SepTcOp {
     alignas(64) unsigned char tmap_x[128];
     alignas(64) unsigned char tmap_w[128];
     alignas(8) unsigned char geom[256];
     int smem_bytes;
 };
-bool septc_supported(int k, int nc, int stride, int dil);
-bool septc_enabled();      // PN_SEP_TC=0 turns the path off
-bool septc_preferred(int k, int nc, int stride, int dil);   // default: the 256 -> 256 blocks only (measured); PN_SEP_TC=1: every supported block
+bool septc_supported(int k, int nc, int stride, int dil);   // the 256 -> 256 blocks at stride 1, dilation 1 or 2 (measured)
 int septc_geometry(SepTcOp *op, int n, int h, int wd, int k, int nc, int dil);
 int septc_prepare(SepTcOp *op, const void *x, const void *pw_w, int n, int h, int wd, int k, int nc, int dil);
 int septc_launch(const SepTcOp *op, const float *dw_w, const float *dw_b, const float *pw_b, void *y, cudaStream_t s);

@@ -180,7 +180,7 @@ dwwarp_kernel(const __grid_constant__ CUtensorMap tmap_x, const float *__restric
 
 // ---- host side ---------------------------------------------------------------------------------------------
 bool dwwarp_supported(int c, int stride, int dil, int dtype) {
-    return dtype == PN_BF16 && stride == 1 && (dil == 1 || dil == 2) && c % 8 == 0 && getenv("PN_NO_DWWARP") == nullptr;
+    return dtype == PN_BF16 && stride == 1 && (dil == 1 || dil == 2) && c % 8 == 0;
 }
 
 int dwwarp_prepare(DwWarpOp *op, const void *x, int n, int h, int wd, int c, int dil) {
@@ -196,38 +196,31 @@ int dwwarp_prepare(DwWarpOp *op, const void *x, int n, int h, int wd, int c, int
     const long long per_q = (long long)n * dil * g.strips * g.cblocks;
     const int max_nq = ceil_div(rows_c, 8);                               // row blocks of at least 8 rows
     long long nq = 1;
-    const char *e_items = getenv("PN_DWW_ITEMS");
-    if (e_items && atoi(e_items) > 0) {                                   // the rule of round 1: about PN_DWW_ITEMS (2) items per warp
-        nq = ((long long)atoi(e_items) * warps + per_q - 1) / per_q;
-        if (nq > max_nq) nq = max_nq;
-        if (nq < 1) nq = 1;
-    } else {
-        // as in sepwarp.cu: items go to the warps round-robin (channel blocks fastest), so the row-block count is the one that
-        // leaves the busiest warp the fewest input rows in a simulation of that assignment
-        std::vector<long long> load((size_t)warps);
-        long long best = -1;
-        for (int cand = 1; cand <= max_nq; ++cand) {
-            const int rb = ceil_div(rows_c, cand);
-            if (ceil_div(rows_c, rb) != cand) continue;
-            const long long items_c = per_q * cand;
-            if (items_c > (1ll << 22)) break;
-            std::fill(load.begin(), load.end(), 0ll);
-            const long long per_cls = (long long)g.strips * g.cblocks;    // items per (image, row block, class)
-            long long it = 0;
-            int wi = 0;
-            for (int img = 0; img < n; ++img)
-                for (int q = 0; q < cand; ++q)
-                    for (int cls = 0; cls < dil; ++cls) {
-                        const int rows_cls = (h - cls + dil - 1) / dil, rows_out = rows_cls - q * rb < rb ? rows_cls - q * rb : rb;
-                        const long long cost = rows_out > 0 ? rows_out + 2 : 0;
-                        for (long long j = 0; j < per_cls; ++j, ++it) {
-                            load[(size_t)wi] += cost;
-                            if (++wi == (int)warps) wi = 0;
-                        }
+    // as in sepwarp.cu: items go to the warps round-robin (channel blocks fastest), so the row-block count is the one that
+    // leaves the busiest warp the fewest input rows in a simulation of that assignment
+    std::vector<long long> load((size_t)warps);
+    long long best = -1;
+    for (int cand = 1; cand <= max_nq; ++cand) {
+        const int rb = ceil_div(rows_c, cand);
+        if (ceil_div(rows_c, rb) != cand) continue;
+        const long long items_c = per_q * cand;
+        if (items_c > (1ll << 22)) break;
+        std::fill(load.begin(), load.end(), 0ll);
+        const long long per_cls = (long long)g.strips * g.cblocks;        // items per (image, row block, class)
+        long long it = 0;
+        int wi = 0;
+        for (int img = 0; img < n; ++img)
+            for (int q = 0; q < cand; ++q)
+                for (int cls = 0; cls < dil; ++cls) {
+                    const int rows_cls = (h - cls + dil - 1) / dil, rows_out = rows_cls - q * rb < rb ? rows_cls - q * rb : rb;
+                    const long long cost = rows_out > 0 ? rows_out + 2 : 0;
+                    for (long long j = 0; j < per_cls; ++j, ++it) {
+                        load[(size_t)wi] += cost;
+                        if (++wi == (int)warps) wi = 0;
                     }
-            const long long worst = *std::max_element(load.begin(), load.end());
-            if (best < 0 || worst < best) { best = worst; nq = cand; }
-        }
+                }
+        const long long worst = *std::max_element(load.begin(), load.end());
+        if (best < 0 || worst < best) { best = worst; nq = cand; }
     }
     g.rb = ceil_div(rows_c, (int)nq);
     g.nq = ceil_div(rows_c, g.rb);

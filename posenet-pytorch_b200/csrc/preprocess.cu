@@ -1,14 +1,12 @@
 // P1 -- fused uint8 HWC BGR -> resize -> RGB -> x*(2/255)-1 -> f32 NCHW.
 // Replaces posenet/utils.py:13-26 (_process_input) of the reference, i.e. cv2.resize(INTER_LINEAR) on
 // uint8 + cvtColor + two rounded fp32 ops.  Integer/fixed-point work: bit-exact with OpenCV.
-// HBM-bound: reads 3 B and writes 12 B per output pixel; one thread per output pixel, x fastest.
-#include <stdlib.h>
-
+// HBM-bound: reads 3 B and writes 12 B per output pixel, x fastest.
 #include "common.cuh"
 
 namespace pn {
 
-enum { MODE_COPY = 0, MODE_AREA2 = 1, MODE_LINEAR = 2 };
+enum { MODE_COPY = 0, MODE_AREA2 = 1 };
 
 // cv2: f = (float)((d + 0.5) * scale - 0.5) in double, s = floor(f), f -= s in fp32.  Explicit _rn
 // intrinsics keep nvcc from contracting mul+add into an FMA (which rounds differently).
@@ -26,10 +24,10 @@ __device__ __forceinline__ float normalise(int v) {
 
 // OUT_U8: stop after the resize and keep uint8 BGR HWC (the tensor-core stem consumes that and normalises itself), so
 // frames of any size can feed the uint8 fast path; otherwise the reference's normalised f32 RGB NCHW tensor.
+// This kernel covers the same-size copy and the exact 2x decimation, one thread per output pixel; resize_linear_kernel the rest.
 template <int MODE, bool OUT_U8>
-__global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t *__restrict__ src, void *__restrict__ dst_,
-                                                          int sh, int sw, int dh, int dw, double scale_x,
-                                                          double scale_y) {
+__global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t *__restrict__ src, void *__restrict__ dst_, int sh, int sw,
+                                                          int dh, int dw) {
     const int x = blockIdx.x * blockDim.x + threadIdx.x;
     const int y = blockIdx.y;
     const int img = blockIdx.z;
@@ -39,35 +37,12 @@ __global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t *__restri
     if (MODE == MODE_COPY) {
         const uint8_t *p = s + ((size_t)y * sw + x) * 3;
         bgr[0] = p[0]; bgr[1] = p[1]; bgr[2] = p[2];
-    } else if (MODE == MODE_AREA2) {
+    } else {
         // exact 2x decimation takes cv2's INTER_AREA 2x2 box path
         const uint8_t *p0 = s + ((size_t)(2 * y) * sw + 2 * x) * 3;
         const uint8_t *p1 = p0 + (size_t)sw * 3;
 #pragma unroll
         for (int c = 0; c < 3; ++c) bgr[c] = (p0[c] + p0[3 + c] + p1[c] + p1[3 + c] + 2) >> 2;
-    } else {
-        int sx, sy;
-        float fx, fy;
-        axis_coeff(x, scale_x, sx, fx);
-        if (sx < 0) { sx = 0; fx = 0.f; }
-        if (sx >= sw - 1) { sx = sw - 1; fx = 0.f; }
-        const int x1 = min(sx + 1, sw - 1);
-        axis_coeff(y, scale_y, sy, fy);              // rows: index clipped, weights kept
-        const int y0 = min(max(sy, 0), sh - 1);
-        const int y1 = min(max(sy + 1, 0), sh - 1);
-        const int a1 = __float2int_rn(__fmul_rn(fx, 2048.f));
-        const int a0 = __float2int_rn(__fmul_rn(__fsub_rn(1.f, fx), 2048.f));
-        const int b1 = __float2int_rn(__fmul_rn(fy, 2048.f));
-        const int b0 = __float2int_rn(__fmul_rn(__fsub_rn(1.f, fy), 2048.f));
-        const uint8_t *r0 = s + (size_t)y0 * sw * 3;
-        const uint8_t *r1 = s + (size_t)y1 * sw * 3;
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-            const int h0 = r0[sx * 3 + c] * a0 + r0[x1 * 3 + c] * a1;
-            const int h1 = r1[sx * 3 + c] * a0 + r1[x1 * 3 + c] * a1;
-            int v = (((b0 * (h0 >> 4)) >> 16) + ((b1 * (h1 >> 4)) >> 16) + 2) >> 2;
-            bgr[c] = min(max(v, 0), 255);
-        }
     }
     if (OUT_U8) {
         uint8_t *o8 = reinterpret_cast<uint8_t *>(dst_) + (((size_t)img * dh + y) * dw + x) * 3;
@@ -81,9 +56,9 @@ __global__ void __launch_bounds__(256) preprocess_kernel(const uint8_t *__restri
     o[2 * plane] = normalise(bgr[0]);
 }
 
-// MODE_LINEAR with the coefficient arithmetic hoisted: a block covers 256 output columns x PRE_RB output rows; the row
-// coefficients (float64 -> fixed point, the expensive part of a pixel) are computed once per block row into shared memory and
-// the column coefficients once per thread, then reused down the rows.  Same operations per coefficient as above -> same bits.
+// cv2.resize INTER_LINEAR: a block covers 256 output columns x PRE_RB output rows; the row coefficients (float64 -> fixed point,
+// the expensive part of a pixel) are computed once per block row into shared memory and the column coefficients once per thread,
+// then reused down the rows.
 constexpr int PRE_RB = 16;
 template <bool OUT_U8>
 __global__ void __launch_bounds__(256) resize_linear_kernel(const uint8_t *__restrict__ src, void *__restrict__ dst_, int sh, int sw,
@@ -161,11 +136,9 @@ static int launch_preprocess_t(const uint8_t *src, int n, int sh, int sw, int dh
     const double scale_x = 1.0 / ((double)dw / (double)sw);
     const double scale_y = 1.0 / ((double)dh / (double)sh);
     if (dh == sh && dw == sw)
-        preprocess_kernel<MODE_COPY, OUT_U8><<<grid, block, 0, st>>>(src, dst, sh, sw, dh, dw, scale_x, scale_y);
+        preprocess_kernel<MODE_COPY, OUT_U8><<<grid, block, 0, st>>>(src, dst, sh, sw, dh, dw);
     else if (sh == 2 * dh && sw == 2 * dw)
-        preprocess_kernel<MODE_AREA2, OUT_U8><<<grid, block, 0, st>>>(src, dst, sh, sw, dh, dw, scale_x, scale_y);
-    else if (getenv("PN_RESIZE_PER_PIXEL"))          // the one-thread-per-pixel form (A/B)
-        preprocess_kernel<MODE_LINEAR, OUT_U8><<<grid, block, 0, st>>>(src, dst, sh, sw, dh, dw, scale_x, scale_y);
+        preprocess_kernel<MODE_AREA2, OUT_U8><<<grid, block, 0, st>>>(src, dst, sh, sw, dh, dw);
     else
         resize_linear_kernel<OUT_U8><<<dim3(ceil_div(dw, 256), ceil_div(dh, PRE_RB), n), block, 0, st>>>(src, dst, sh, sw, dh, dw, scale_x,
                                                                                                      scale_y);

@@ -46,6 +46,7 @@ constexpr int SEP_MAX_P = 6, SEP_MAX_W = 6;
 constexpr int SEP_WGT_BYTES = 9 * 64 * 4 + 64 * 4;                     // dw weights [9][64] + bias [64] fp32
 constexpr int SEP_SMEM_MAX = 232448;
 constexpr int SEP_DWW_KB_BYTES = 10 * 64 * 4;                          // resident depthwise weights + bias of one k-block
+constexpr unsigned SEP_EPI_SLEEP_NS = 200;                             // between the epilogue's polls of its accumulator barrier
 
 struct SepGeom {
     int k, nc, ho, wo, pad;
@@ -56,14 +57,10 @@ struct SepGeom {
     int n_halves, n_half, acc_bufs;       // a tile's accumulator = n_halves UMMA column blocks of n_half (<= 256) columns
     int kblocks;
     int half, cbox;                       // K <= 32: two pixel columns per warp (16 lanes each), 32-channel patch box
-    int cl;                               // CTAs per cluster (1, 2, 4): each owns 256 output channels and 1 / cl of the k-blocks
     int dww_res;                          // depthwise weights resident in shared memory (off_dww) instead of behind every patch stage
     int w_res;                            // pointwise weights resident: W stage = k-block * n_halves + column block, loaded once
     unsigned off_dww;                     // resident depthwise weights [kblocks][10][64] fp32 (SEP_LEAN & 4)
-    int teams;                            // depthwise warp teams (1, 2, 3): a team owns whole items, the teams take items in turn
-    int exp;                              // PN_SEP_EXP build only: experiment flags (1 no dw math, 2 no (staged) epilogue work, 4 no MMA, 8 no W loads,
-                                          // 16 direct epilogue without stores, 32 no patch loads, 64 no weight loads / segments, 128 no proxy fence)
-    unsigned epi_sleep_ns;                // sleep between the epilogue's polls of its accumulator barrier (PN_SEP_EPI_SLEEP, default 200)
+    int teams;                            // depthwise warp teams (1, 2): a team owns whole items, the teams take items in turn
     int p_stages, w_stages, a_stages, stg_bufs;
     unsigned patch_stage_bytes, patch_box_bytes, wgt_off, w_stage_bytes;
     unsigned off_a, off_stg, off_patch, off_bias, off_bar;   // from the 1024-aligned base; W stages sit at 0
@@ -104,34 +101,6 @@ __device__ __forceinline__ uint32_t lds_u32(uint32_t addr) {
     uint32_t r;
     asm volatile("ld.shared.b32 %0, [%1];" : "=r"(r) : "r"(addr));
     return r;
-}
-// ---- cluster helpers (N-split blocks, see the kernel header) ------------------------------------------------------
-__device__ __forceinline__ uint32_t cluster_rank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t map_to_cta(uint32_t saddr, uint32_t rank) {           // shared::cta -> shared::cluster of `rank`
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(saddr), "r"(rank));
-    return r;
-}
-__device__ __forceinline__ void remote_expect_tx(uint32_t cluster_bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.release.cluster.shared::cluster.b64 _, [%0], %1;" ::"r"(cluster_bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void dsmem_bulk_copy(uint32_t cluster_dst, uint32_t src, uint32_t bytes, uint32_t cluster_bar) {
-    asm volatile("cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(cluster_dst),
-                 "r"(src), "r"(bytes), "r"(cluster_bar)
-                 : "memory");
-}
-__device__ __forceinline__ void tc_commit_multicast(uint32_t bar, uint16_t cta_mask) {      // arrives on `bar` of every CTA in the mask
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"(cta_mask)
-                 : "memory");
 }
 __device__ __forceinline__ void sts_u32_if(uint32_t addr, uint32_t v, bool on) {     // compiles to one predicated STS; the predicate
     if (on) asm volatile("st.shared.b32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");  // is loop-invariant and stays in a P register
@@ -183,22 +152,15 @@ __device__ int g_sep_trace_cap = 0;
 #define SEP_PH(i) do { } while (0)
 #endif
 
-template <int S, int D, bool HALF, int CL>
+template <int S, int D, bool HALF>
 __global__ void __launch_bounds__(SEP_THREADS, 1)
 sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_dww,
                const __grid_constant__ CUtensorMap tmap_dwb, const __grid_constant__ CUtensorMap tmap_w,
                const __grid_constant__ CUtensorMap tmap_y, const float *__restrict__ pw_bias, __nv_bfloat16 *__restrict__ y,
                const float *__restrict__ dw_w, const float *__restrict__ dw_b, const SepGeom g) {
     constexpr int CB = 64;                                  // channels per k-block (ragged K is zero-filled by TMA)
-    // CL > 1: a cluster of CL CTAs shares every 128-pixel tile.  CTA `rank` owns output channels [rank * 256, +256) --
-    // its own pointwise weights, accumulators (double-buffered) and epilogue -- and computes the depthwise result of the
-    // k-blocks kb % CL == rank only; the finished A stage is pushed into the peers' shared memory with one DSMEM bulk copy
-    // each (completing on their a_full barrier), so the depthwise work, which bounds these blocks, is done once per tile.
-    constexpr bool CLUSTER = CL > 1;
-    const bool DWW_RES = !CLUSTER && g.dww_res != 0;         // depthwise weights resident in shared memory (per block: sep_geometry)
-    const int rank = CLUSTER ? (int)cluster_rank() : 0;
-    const long long tile_first = CLUSTER ? blockIdx.x / CL : blockIdx.x, tile_step = CLUSTER ? gridDim.x / CL : gridDim.x;
-    const int col_base = CLUSTER ? rank * g.n_tile : 0;      // first output channel of this CTA
+    const bool DWW_RES = g.dww_res != 0;                     // depthwise weights resident in shared memory (per block: sep_geometry)
+    const long long tile_first = blockIdx.x, tile_step = gridDim.x;
 
     extern __shared__ uint8_t sep_smem_raw[];
     const uint32_t base = (smem_u32(sep_smem_raw) + 1023u) & ~1023u;
@@ -221,16 +183,15 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
         tma_prefetch_desc(&tmap_y);
         for (int s = 0; s < g.p_stages; ++s) {
             mbar_init(bar(SepBars::patch_full, s), 1);
-            mbar_init(bar(SepBars::patch_empty, s), (SEP_DW_WARPS + g.teams - 1) / g.teams);
+            mbar_init(bar(SepBars::patch_empty, s), SEP_DW_WARPS / g.teams);
         }
         for (int s = 0; s < g.w_stages; ++s) {
             mbar_init(bar(SepBars::w_full, s), 1);
             mbar_init(bar(SepBars::w_empty, s), 1);
         }
         for (int s = 0; s < g.a_stages; ++s) {
-            // a stage produced by a peer is filled by its bulk copy (one expect_tx arrival + the bytes)
-            mbar_init(bar(SepBars::a_full, s), (!CLUSTER || s % CL == rank) ? (SEP_DW_WARPS + g.teams - 1) / g.teams : 1);
-            mbar_init(bar(SepBars::a_empty, s), CL);            // every CTA's MMAs have read the stage (multicast commits)
+            mbar_init(bar(SepBars::a_full, s), SEP_DW_WARPS / g.teams);
+            mbar_init(bar(SepBars::a_empty, s), 1);
         }
         for (int s = 0; s < 2; ++s) {
             mbar_init(bar(SepBars::tfull, s), 1);
@@ -251,7 +212,7 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
     {   // pointwise bias -> shared memory once (the epilogue reads it per panel)
         float *sbias = reinterpret_cast<float *>(sep_smem_raw + (base - smem_u32(sep_smem_raw)) + g.off_bias);
         const int ncp = g.n_tiles * g.panels * 64;                // padded so that ragged panels read zeros
-        for (int i = threadIdx.x; i < ncp; i += SEP_THREADS) sbias[i] = col_base + i < g.nc ? __ldg(pw_bias + col_base + i) : 0.f;
+        for (int i = threadIdx.x; i < ncp; i += SEP_THREADS) sbias[i] = i < g.nc ? __ldg(pw_bias + i) : 0.f;
     }
     if (DWW_RES) {   // depthwise weights [9, K] + bias [K] -> [k-block][tap | bias][64] fp32, ragged K zero-filled (never written by the
                      // preceding kernel, so this may run before griddepcontrol.wait like the bias above)
@@ -263,7 +224,6 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
     }
     tc_fence_before();
     __syncthreads();
-    if (CLUSTER) cluster_sync_all();                          // the peers' barriers exist before anything remote targets them
     tc_fence_after();
     pdl_launch_dependents();                                  // after the TMEM allocation is made (see stem.cu): a dependent CTA must not allocate first
     pdl_wait();                                               // everything above overlapped the previous layer's tail
@@ -279,32 +239,12 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
             uint32_t pph = 0, wph = 0;
             (void)tr_p;
             long long p_tile = tile_first, w_tile = tile_first;
-            int p_kb = rank, p_sub = 0, w_kb = 0, w_hf = 0;       // patches: this CTA's k-blocks only
+            int p_kb = 0, p_sub = 0, w_kb = 0, w_hf = 0;
             int p_img = 0, p_ty = 0, p_tx = 0, w_col = 0;
             bool p_new = true, w_new = true;
-            // cluster: this thread also pushes every finished A stage of this CTA to the peers the moment its last depthwise
-            // warp has arrived (NOT from the MMA loop: that one runs in k-block order and would make the two CTAs ping-pong)
-            int s_as = rank;
-            uint32_t s_aph = 0;
-            long long s_left = 0;
-            if (CLUSTER && tile_first < g.tiles) s_left = ((g.tiles - tile_first + tile_step - 1) / tile_step) * (g.kblocks / CL);
             const long long t0 = clock64();
-            while (p_tile < g.tiles || w_tile < g.tiles || s_left > 0) {
+            while (p_tile < g.tiles || w_tile < g.tiles) {
                 bool progress = false;
-                if (CLUSTER && s_left > 0 && mbar_test(bar(SepBars::a_full, s_as), s_aph)) {
-                    const uint32_t sa = a_addr(s_as);
-#pragma unroll
-                    for (int pr = 0; pr < CL; ++pr)
-                        if (pr != rank) {
-                            const uint32_t rbar = map_to_cta(bar(SepBars::a_full, s_as), (uint32_t)pr);
-                            remote_expect_tx(rbar, SEP_A_BYTES);
-                            dsmem_bulk_copy(map_to_cta(sa, (uint32_t)pr), sa, SEP_A_BYTES, rbar);
-                        }
-                    s_as += CL;
-                    if (s_as >= g.a_stages) { s_as -= g.a_stages; s_aph ^= 1; }
-                    --s_left;
-                    progress = true;
-                }
                 if (p_tile < g.tiles) {
                     if (p_new) {
                         const int m_tile = (int)(p_tile / g.n_tiles);
@@ -317,9 +257,6 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
                     if (mbar_test(bar(SepBars::patch_empty, ps), pph ^ 1)) {
                         const uint32_t full = bar(SepBars::patch_full, ps);
                         SEP_TRACE(3, tr_p, 0);
-#ifdef PN_SEP_EXP
-                        if (g.exp & 32) mbar_arrive(full); else {                          // experiment: no patch / weight loads
-#endif
                         mbar_expect_tx(full, g.patch_box_bytes + (DWW_RES ? 0u : (uint32_t)SEP_WGT_BYTES));
                         tma_load_4d(p_addr(ps), &tmap_x, full, p_kb * CB, p_tx * g.tw * S - g.pad,
                                     (p_ty * g.th + p_sub * g.ths) * S - g.pad, p_img);
@@ -327,31 +264,21 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
                             tma_load_2d(p_addr(ps) + g.wgt_off, &tmap_dww, full, p_kb * CB, 0);
                             tma_load_2d(p_addr(ps) + g.wgt_off + 9 * 64 * 4, &tmap_dwb, full, p_kb * CB, 0);
                         }
-#ifdef PN_SEP_EXP
-                        }
-#endif
                         SEP_TRACE(3, tr_p, 1);
                         ++tr_p;
                         if (++ps == g.p_stages) { ps = 0; pph ^= 1; }
                         if (++p_sub == g.subs) {
                             p_sub = 0;
-                            p_kb += CL;
-                            if (p_kb >= g.kblocks) { p_kb = rank; p_tile += tile_step; p_new = true; }
+                            if (++p_kb >= g.kblocks) { p_kb = 0; p_tile += tile_step; p_new = true; }
                         }
                         progress = true;
                     }
                 }
                 if (w_tile < g.tiles) {
-                    if (w_new) { w_col = col_base + (int)(w_tile % g.n_tiles) * g.n_tile; w_new = false; }
+                    if (w_new) { w_col = (int)(w_tile % g.n_tiles) * g.n_tile; w_new = false; }
                     if (mbar_test(bar(SepBars::w_empty, ws), wph ^ 1)) {
-#ifdef PN_SEP_EXP
-                        if (g.exp & 8) mbar_arrive(bar(SepBars::w_full, ws)); else {
-#endif
                         mbar_expect_tx(bar(SepBars::w_full, ws), g.w_stage_bytes);
                         tma_load_2d(w_addr(ws), &tmap_w, bar(SepBars::w_full, ws), w_kb * CB, w_col + w_hf * g.n_half);
-#ifdef PN_SEP_EXP
-                        }
-#endif
                         if (++ws == g.w_stages) { ws = 0; wph ^= 1; }
                         if (++w_hf == g.n_halves) {
                             w_hf = 0;
@@ -379,7 +306,6 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
             int as = 0, ws = 0, acc = 0, tr_i = 0;
             uint32_t aph = 0, wph = 0, acc_phase = 0;
             (void)tr_i;
-            long long kb_total = 0;                                   // k-blocks consumed (A-stage uses), for the drain below
             for (long long tile = tile_first; tile < g.tiles; tile += tile_step) {
                 mbar_wait(bar(SepBars::tempty, acc), acc_phase ^ 1);
                 tc_fence_after();
@@ -401,11 +327,7 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
                         const uint32_t sb = w_addr(ws);
 #pragma unroll
                         for (int k = 0; k < CB / 16; ++k)
-                            if (k < ksteps
-#ifdef PN_SEP_EXP
-                                && !(g.exp & 4)
-#endif
-                                )
+                            if (k < ksteps)
                                 tc_mma_bf16(d_tmem + (uint32_t)(hf * g.n_half), sep_smem_desc(sa + k * 32), sep_smem_desc(sb + k * 32), idesc,
                                             (uint32_t)((kb | k) != 0));
                         if (!g.w_res) {
@@ -413,24 +335,13 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
                             if (++ws == g.w_stages) { ws = 0; wph ^= 1; }
                         }
                     }
-                    if (CLUSTER) tc_commit_multicast(bar(SepBars::a_empty, as), (uint16_t)((1u << CL) - 1u));
-                    else tc_commit(bar(SepBars::a_empty, as));
-                    ++kb_total;
+                    tc_commit(bar(SepBars::a_empty, as));
                     SEP_TRACE(1, tr_i, 2);
                     ++tr_i;
                     if (++as == g.a_stages) { as = 0; aph ^= 1; }
                 }
                 tc_commit(bar(SepBars::tfull, acc));
                 if (++acc == g.acc_bufs) { acc = 0; acc_phase ^= 1; }
-            }
-            if (CLUSTER) {
-                // Drain: the peers' multicast commits arrive on this CTA's a_empty barriers asynchronously; every stage's
-                // last use must have collected all CL arrivals before this CTA may leave (its shared memory dies with it).
-                for (int s2 = 0; s2 < g.a_stages; ++s2) {
-                    if (kb_total <= s2) continue;
-                    const long long uses = (kb_total - s2 + g.a_stages - 1) / g.a_stages;
-                    mbar_wait(bar(SepBars::a_empty, s2), (uint32_t)((uses - 1) & 1));
-                }
             }
         }
     } else if (warp < SEP_FIRST_DW_WARP) {
@@ -475,14 +386,11 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
                 const int rem = m_tile - img * m_tiles_per_img;
                 const int ty = rem / g.tiles_x, tx = rem - ty * g.tiles_x;
                 const int oy = ty * g.th + r_ty, ox = tx * g.tw + r_tx;
-                bool row_ok = r_ty < g.th && oy < g.ho && ox < g.wo;
-#ifdef PN_SEP_EXP
-                if (g.exp & 16) row_ok = false;                           // experiment: the epilogue without its global stores
-#endif
-                const int colg = col_base + n_tile * g.n_tile;            // first global output channel of this accumulator
+                const bool row_ok = r_ty < g.th && oy < g.ho && ox < g.wo;
+                const int colg = n_tile * g.n_tile;                       // first output channel of this accumulator
                 __nv_bfloat16 *yrow = y + (((size_t)img * g.ho + oy) * g.wo + ox) * (size_t)g.nc + colg;
                 const int col_lim = g.nc - colg;                          // columns of this block that exist (ragged N)
-                mbar_wait_backoff(bar(SepBars::tfull, acc), acc_phase, g.epi_sleep_ns);
+                mbar_wait_backoff(bar(SepBars::tfull, acc), acc_phase, SEP_EPI_SLEEP_NS);
                 tc_fence_after();
                 if (issuer) SEP_TRACE(2, tr_e, 0);
                 const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * g.n_tile);
@@ -512,18 +420,10 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
             const int img = m_tile / m_tiles_per_img;
             const int rem = m_tile - img * m_tiles_per_img;
             const int ty = rem / g.tiles_x, tx = rem - ty * g.tiles_x;
-            mbar_wait_backoff(bar(SepBars::tfull, acc), acc_phase, g.epi_sleep_ns);   // idle epilogue warps must not eat issue slots
+            mbar_wait_backoff(bar(SepBars::tfull, acc), acc_phase, SEP_EPI_SLEEP_NS);   // idle epilogue warps must not eat issue slots
             tc_fence_after();
             if (issuer) SEP_TRACE(2, tr_e, 0);
             const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * g.n_tile);
-#ifdef PN_SEP_EXP
-            if (g.exp & 2) {
-                tc_fence_before();
-                mbar_arrive(bar(SepBars::tempty, acc));
-                if (++acc == g.acc_bufs) { acc = 0; acc_phase ^= 1; }
-                continue;
-            }
-#endif
 #pragma unroll 1
             for (int p = 0; p < g.panels; ++p) {
                 const int col0 = n_tile * g.n_tile + p * 64;
@@ -556,7 +456,7 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
                 fence_async_smem();                                      // generic writes -> visible to TMA
                 sep_epi_bar();
                 if (issuer) {
-                    tma_store_4d(&tmap_y, staging + (uint32_t)buf * SEP_STG_BYTES, col_base + col0, tx * g.tw, ty * g.th, img);
+                    tma_store_4d(&tmap_y, staging + (uint32_t)buf * SEP_STG_BYTES, col0, tx * g.tw, ty * g.th, img);
                     bulk_commit();
                 }
                 if (g.stg_bufs == 2) buf ^= 1;
@@ -603,24 +503,16 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
         // of one, the barriers count five arrivals, and two items are in flight at once (the rings are deep enough where
         // sep_geometry turns this on).  Every warp still walks all items in order so that its stage cursors and parities
         // follow the rings; it just steps over the other team's items.
-        // Team sizes: 10 warps are 10 / 5 + 5 / 4 + 3 + 3.  Every barrier counts the LARGEST team's arrivals whichever team uses the
-        // stage (stages rotate through the teams), so the first warp of a smaller team arrives twice.
-        const int n_teams = g.teams, dwi = warp - SEP_FIRST_DW_WARP, team_max = (SEP_DW_WARPS + n_teams - 1) / n_teams;
-        const int big_teams = SEP_DW_WARPS - n_teams * (team_max - 1);            // teams that have team_max warps (the first ones)
-        const int team = dwi < big_teams * team_max ? dwi / team_max : big_teams + (dwi - big_teams * team_max) / (team_max - 1);
-        const int team_first = team < big_teams ? team * team_max : big_teams * team_max + (team - big_teams) * (team_max - 1);
-        const int team_warps = team < big_teams ? team_max : team_max - 1;
-        const bool twice = team_warps < team_max && dwi == team_first;            // stands in for the warp this team lacks
+        const int n_teams = g.teams, dwi = warp - SEP_FIRST_DW_WARP, team_warps = SEP_DW_WARPS / n_teams;
+        const int team = dwi / team_warps, team_first = team * team_warps;
         const int n_subs = g.subs, n_pst = g.p_stages, n_ast = g.a_stages, n_kb = g.kblocks;
-        const int item_step = CLUSTER ? CL : n_teams;                    // items (k-blocks in tile order) between two of this warp's
         int tr_d = 0;
-        // cursors of this warp's first item: item `rank` of a cluster CTA, item `team` otherwise (its stages follow the first
-        // team's: both rings are deeper than one item)
-        int ps = CLUSTER ? 0 : team * n_subs, as = CLUSTER ? rank : team, kb = CLUSTER ? rank : team;
+        // cursors of this warp's first item, item `team` (its stages follow the first team's: both rings are deeper than one item)
+        int ps = team * n_subs, as = team, kb = team;
         uint32_t pph = 0, aph = 0;
         int rot = dwi - team_first;                                      // this warp's first segment in the current item
         long long tile = tile_first;
-        while (!CLUSTER && kb >= n_kb) { kb -= n_kb; tile += tile_step; }    // (single-k-block tiles: the second team starts one tile on)
+        while (kb >= n_kb) { kb -= n_kb; tile += tile_step; }              // (single-k-block tiles: the second team starts one tile on)
         (void)tr_d;
         const bool tracer = (warp == SEP_FIRST_DW_WARP && lane == 0);
         (void)tracer;
@@ -651,11 +543,7 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
               SEP_PH(1);
               const uint32_t stage = p_addr(ps);
               bool have_w = DWW_RES;
-              for (int seg = rot; seg < g.segs_per_sub
-#ifdef PN_SEP_EXP
-                   && !(g.exp & 64)                                   // experiment: no weight / table loads, no segments
-#endif
-                   ; seg += team_warps) {
+              for (int seg = rot; seg < g.segs_per_sub; seg += team_warps) {
                 if (!have_w) {
                     const uint32_t wsm = stage + g.wgt_off + (uint32_t)cp * 8u;
 #pragma unroll
@@ -668,11 +556,7 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
                 const int orow0 = sub * g.ths + s_r0;
                 const int nrows = min(s_n, (g.th - orow0 + RSTEP - 1) / RSTEP);     // rows of this segment inside the tile
                 SEP_PH(2);
-                if (nrows > 0
-#ifdef PN_SEP_EXP
-                    && !(g.exp & 1)
-#endif
-                    ) {
+                if (nrows > 0) {
                     const uint32_t src = stage + (uint32_t)(s_r0 * S) * rowb1 + (uint32_t)(s_col * S) * PIX + lane_off;
                     const int ncol_ok = g.tw - s_col;                               // strip pixels px < ncol_ok exist
                     int arow = orow0 * g.tw + s_col;                                // A-tile row == TMEM lane == staging row
@@ -758,35 +642,25 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
                 SEP_PH(4);
               }   // segments of this item
               __syncwarp();
-              if (lane == 0) {                                             // this warp no longer reads the patch
-                  mbar_arrive(bar(SepBars::patch_empty, ps));
-                  if (twice) mbar_arrive(bar(SepBars::patch_empty, ps));
-              }
+              if (lane == 0) mbar_arrive(bar(SepBars::patch_empty, ps));     // this warp no longer reads the patch
               SEP_PH(5);
               if (++ps == n_pst) { ps = 0; pph ^= 1; }
               if (++rot == team_warps) rot = 0;
             }
-#ifdef PN_SEP_EXP
-            if (!(g.exp & 128))                                       // experiment: no generic -> async proxy fence
-#endif
             fence_async_smem();                                       // A-tile writes -> visible to the tensor core
             __syncwarp();
-            if (lane == 0) {
-                mbar_arrive(bar(SepBars::a_full, as));
-                if (twice) mbar_arrive(bar(SepBars::a_full, as));
-            }
+            if (lane == 0) mbar_arrive(bar(SepBars::a_full, as));
             SEP_PH(6);
             if (tracer) { SEP_TRACE(0, tr_d, 3); ++tr_d; }
-            // on to this warp's next item: over the other team's patch stages and A stage, item_step k-blocks ahead
+            // on to this warp's next item: over the other team's patch stages and A stage, n_teams k-blocks ahead
             if (n_teams > 1) {
                 ps += (n_teams - 1) * n_subs;
                 if (ps >= n_pst) { ps -= n_pst; pph ^= 1; }
             }
-            as += item_step;
+            as += n_teams;
             if (as >= n_ast) { as -= n_ast; aph ^= 1; }
-            kb += item_step;
-            if (CLUSTER) { if (kb >= n_kb) { kb = rank; tile += tile_step; } }
-            else while (kb >= n_kb) { kb -= n_kb; tile += tile_step; }
+            kb += n_teams;
+            while (kb >= n_kb) { kb -= n_kb; tile += tile_step; }
           }
         }
 #ifdef PN_SEP_PHASES
@@ -798,7 +672,6 @@ sepconv_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant
 
     tc_fence_before();
     __syncthreads();
-    if (CLUSTER) cluster_sync_all();                          // no peer still copies into / arrives on this CTA's shared memory
     if (warp == 1) {
         tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)g.tmem_cols) : "memory");
@@ -821,13 +694,9 @@ bool sep_supported(int k, int nc, int stride, int dil) {
            ((stride == 1 && (dil == 1 || dil == 2 || dil == 4)) || (stride == 2 && dil == 1));
 }
 
-// Blocks worth running fused: whole output width in one accumulator tile (<= 512 channels), or 1024 channels shared by a
-// 4-CTA cluster; anything else would redo the depthwise work once per 512 outputs and is faster as two kernels.
-bool sep_fuse_recommended(int k, int nc, int stride, int dil) {
-    if (!sep_supported(k, nc, stride, dil)) return false;
-    if (nc <= 512) return true;
-    return nc == 1024 && k % 64 == 0 && (k / 64) % 4 == 0 && getenv("PN_SEP_CLUSTER") != nullptr;
-}
+// Blocks worth running fused: whole output width in one accumulator tile (<= 512 channels); anything wider would redo the
+// depthwise work once per 512 outputs and is faster as two kernels.
+bool sep_fuse_recommended(int k, int nc, int stride, int dil) { return sep_supported(k, nc, stride, dil) && nc <= 512; }
 
 // Tile shape, stage counts and the shared-memory carve-up for one block (pure host arithmetic, no CUDA calls).
 int sep_geometry(SepOp *op, int n, int h, int wd, int k, int nc, int stride, int dil) {
@@ -842,7 +711,7 @@ int sep_geometry(SepOp *op, int n, int h, int wd, int k, int nc, int stride, int
         op->n = n; op->h = h; op->w = wd; op->k = k; op->nc = nc;
         return PN_OK;
     }
-    if (septc_preferred(k, nc, stride, dil)) {                      // depthwise on the tensor pipe (septc.cu)
+    if (septc_supported(k, nc, stride, dil)) {                      // depthwise on the tensor pipe (septc.cu)
         op->tc_kind = true;
         op->stride = stride; op->dil = dil;
         op->ho = h; op->wo = wd;
@@ -869,26 +738,9 @@ int sep_geometry(SepOp *op, int n, int h, int wd, int k, int nc, int stride, int
     // is then done once per 512 output channels instead of once per 256.
     g.n_tiles = ceil_div(nc, 512);
     g.n_tile = nc / g.n_tiles;
-    // ... or, for 512 / 1024 output channels, a cluster of 2 / 4 CTAs shares the tile: 256 double-buffered columns each,
-    // the depthwise result of a k-block computed by one CTA and copied to the others (see the kernel).  Measured on the
-    // 512 -> 512 blocks of C2: 82 us against 72 us for the single-CTA tile (the A-stage turnaround across two SMs costs
-    // more than the overlapped epilogue wins), 4-CTA clusters are latency-bound outright -- so this path is opt-in
-    // (PN_SEP_CLUSTER=1) and exercised by the tests only.
-    g.cl = 1;
-    if ((nc == 512 || nc == 1024) && k % cb == 0 && (k / cb) % (nc / 256) == 0 && getenv("PN_SEP_CLUSTER") != nullptr) {
-        g.cl = nc / 256;
-        g.n_tiles = 1;
-        g.n_tile = 256;
-    }
-    g.n_halves = g.n_tile > 256 ? 2 : 1;
-    // W ring granularity: UMMA column blocks of n_tile / n_halves columns.  PN_SEP_NBLK=128 splits wide tiles into 128-column
-    // blocks (16 KB W stages instead of 24-32 KB: a finer ring leaves shared memory for deeper patch / A rings)
-    if (const char *e = getenv("PN_SEP_NBLK")) {
-        const int want = atoi(e);
-        if (want >= 64 && want % 16 == 0 && g.n_tile > want && g.n_tile % want == 0 && g.n_tile / want <= 4) g.n_halves = g.n_tile / want;
-    }
+    g.n_halves = g.n_tile > 256 ? 2 : 1;                            // W ring granularity: UMMA column blocks of n_tile / n_halves columns
     g.n_half = g.n_tile / g.n_halves;
-    PN_CHECK_ARG(g.n_tile * g.n_tiles * g.cl == nc && g.n_half * g.n_halves == g.n_tile && g.n_half % 16 == 0,
+    PN_CHECK_ARG(g.n_tile * g.n_tiles == nc && g.n_half * g.n_halves == g.n_tile && g.n_half % 16 == 0,
                  "pn_sepconv_block: cout %d does not split into tiles", nc);
     g.panels = ceil_div(g.n_tile, 64);
     g.acc_bufs = g.n_tile > 256 ? 1 : 2;
@@ -896,35 +748,29 @@ int sep_geometry(SepOp *op, int n, int h, int wd, int k, int nc, int stride, int
     PN_CHECK_ARG(g.tmem_cols <= 512 && g.panels * 64 <= 512, "pn_sepconv_block: TMEM budget exceeded");
     g.w_stage_bytes = (unsigned)g.n_half * 128u;
 
-    // ---- resident weights (single-CTA kernel).  Depthwise: [k-block][9 taps + bias][64] fp32 loaded once per kernel instead of
+    // ---- resident weights.  Depthwise: [k-block][9 taps + bias][64] fp32 loaded once per kernel instead of
     // travelling behind every patch stage (K <= 256; beyond that 15-20 KB resident would cost a patch stage); a warp fetches its
     // registers from there while it probes the patch barrier.  Pointwise: where every (k-block, column block) fits a stage of its
     // own (<= 80 KB in all) the W ring is loaded once and never again -- per tile that is as much L2 -> shared-memory traffic as
-    // the patches themselves, and the MMA thread loses a wait and a commit per k-block.  PN_SEP_DWWRES=0 / PN_SEP_WRES=0 switch
-    // either off (A/B).  Measured on B200 (same tiles): 128 -> 256 s2 @129^2 100.0 -> 96.2 us, 192 -> 192 @33^2 x512 135.7 -> 134.0,
-    // 128 -> 256 @91x161 114.8 -> 110.0; the freed stages matter more where they buy a deeper ring or a larger tile.
-    const char *e_dww = getenv("PN_SEP_DWWRES"), *e_wres = getenv("PN_SEP_WRES");
-    const bool dww_res = !(e_dww && e_dww[0] == '0') && g.cl == 1 && g.kblocks <= 4;
+    // the patches themselves, and the MMA thread loses a wait and a commit per k-block.  Measured on B200 (same tiles):
+    // 128 -> 256 s2 @129^2 100.0 -> 96.2 us, 192 -> 192 @33^2 x512 135.7 -> 134.0, 128 -> 256 @91x161 114.8 -> 110.0; the freed
+    // stages matter more where they buy a deeper ring or a larger tile.
+    const bool dww_res = g.kblocks <= 4;
     const int wgt_stage = dww_res ? 0 : SEP_WGT_BYTES;             // depthwise weight bytes behind each patch stage
     const int dww_bytes = dww_res ? g.kblocks * SEP_DWW_KB_BYTES : 0;
     g.dww_res = dww_res ? 1 : 0;
-    g.w_res = (!(e_wres && e_wres[0] == '0') && g.cl == 1 && g.n_tiles == 1 && g.kblocks * g.n_halves <= SEP_MAX_W &&
+    g.w_res = (g.n_tiles == 1 && g.kblocks * g.n_halves <= SEP_MAX_W &&
                (long long)g.kblocks * g.n_halves * g.w_stage_bytes <= 80 * 1024) ? 1 : 0;
     // ---- tile search: fewest (tiles x per-tile cost); one strip per depthwise thread group per sub-tile
     const int min_w = g.w_res ? g.kblocks * g.n_halves : g.n_halves >= 2 ? 3 : 2;   // default W ring entries (column blocks of a k-block, plus one ahead)
-    const int min_a = g.cl > 2 ? g.cl : 2;                         // cluster: the A ring is a multiple of the cluster size
-    const int fixed = min_a * SEP_A_BYTES + SEP_STG_BYTES + min_w * (int)g.w_stage_bytes + 1024 + 640 + 4224 + dww_bytes;   // minimum non-patch smem
+    const int fixed = 2 * SEP_A_BYTES + SEP_STG_BYTES + min_w * (int)g.w_stage_bytes + 1024 + 640 + 4224 + dww_bytes;   // minimum non-patch smem
     double best = 1e300;
     // Measured choices first (sep_tuned.inc: tools/tune_sep.py timed the tile shapes / ring depths of the blocks of the reference's
     // standard resolutions on a B200; the cost model below ranks them poorly -- up to 25 % between tiles it scores alike), the
-    // model for every other shape.  PN_SEP_TUNED=0 ignores the table; PN_SEP_TILE="th,tw,subs" / PN_SEP_STAGES / PN_SEP_TEAMS force.
+    // model for every other shape.  PN_SEP_TILE="th,tw,subs" / PN_SEP_STAGES / PN_SEP_TEAMS force a choice (tools/tune_sep.py).
     const SepTuned *tuned = nullptr;
-    {
-        const char *e = getenv("PN_SEP_TUNED");
-        if (!(e && e[0] == '0') && g.cl == 1)
-            for (const SepTuned &t : SEP_TUNED)
-                if (t.k == k && t.nc == nc && t.stride == stride && t.dil == dil && t.ho == g.ho && t.wo == g.wo) { tuned = &t; break; }
-    }
+    for (const SepTuned &t : SEP_TUNED)
+        if (t.k == k && t.nc == nc && t.stride == stride && t.dil == dil && t.ho == g.ho && t.wo == g.wo) { tuned = &t; break; }
     int f_th = 0, f_tw = 0, f_subs = 0;
     if (tuned) { f_th = tuned->th; f_tw = tuned->tw; f_subs = tuned->subs; }
     if (const char *force = getenv("PN_SEP_TILE"))
@@ -1002,7 +848,7 @@ int sep_geometry(SepOp *op, int n, int h, int wd, int k, int nc, int stride, int
     }
     g.tiles_x = ceil_div(g.wo, g.tw);
     g.tiles_y = ceil_div(g.ho, g.th);
-    g.tiles = (long long)n * g.tiles_x * g.tiles_y * g.n_tiles;       // cluster: m tiles (one cluster covers all columns)
+    g.tiles = (long long)n * g.tiles_x * g.tiles_y * g.n_tiles;
     // ---- shared-memory carve-up: W ring, A ring, output staging panels, patch ring, bias, barriers
     const long long bias_bytes = ((long long)g.n_tiles * g.panels * 64 * 4 + 127) & ~127ll;
     const long long avail = SEP_SMEM_MAX - 1024 - 640 - bias_bytes - dww_bytes;   // alignment slack, barrier block (SepBars::total)
@@ -1016,24 +862,20 @@ int sep_geometry(SepOp *op, int n, int h, int wd, int k, int nc, int stride, int
     // cannot overlap the next tile's MMAs there, so its barrier hand-offs are pure stall) -- measured on B200, fused block
     // alone: 256 -> 512 stride 2 at 65x65 95 -> 72 us, 192 -> 384 stride 2 at 33x33 110 -> 94 us, 384 -> 384 at 17x17 128 -> 113 us,
     // 512 -> 512 at 33x33 68 -> 65 us.  Double-buffered tiles keep the staged TMA-store epilogue (it overlaps the main loop;
-    // direct stores are scattered 32-byte pieces and measured 10 % slower there).  PN_SEP_DIRECT=0 / 1 forces either.
-    bool direct = g.acc_bufs == 1 && g.cl == 1;
-    if (const char *e = getenv("PN_SEP_DIRECT")) direct = atoi(e) != 0;
+    // direct stores are scattered 32-byte pieces and measured 10 % slower there).
+    const bool direct = g.acc_bufs == 1;
     const int max_a1 = direct ? 4 : 3;
     for (int stg = direct ? 0 : 2; stg >= (direct ? 0 : 1); --stg)
-        for (int ast = SEP_MAX_A; ast >= 2; --ast) {
-            if (g.cl == 1 && ast > max_a1) continue;
-            if (g.cl > 1 && ast % g.cl != 0) continue;
+        for (int ast = max_a1; ast >= 2; --ast) {
             for (int wst = g.w_res ? min_w : SEP_MAX_W; wst >= min_w; --wst)
                 for (int pst = SEP_MAX_P; pst >= 2 && pst >= g.subs + 1; --pst) {
                     if (!fits(pst, wst, ast, stg)) continue;
-                    // (a cluster CTA consumes patches for 1 / cl of the k-blocks only: two stages cover it, A stages matter more)
-                    const int want = g.cl > 1 ? (g.subs + 1 > 2 ? g.subs + 1 : 2) : 3 * g.subs > SEP_MAX_P ? SEP_MAX_P : 3 * g.subs;
+                    const int want = 3 * g.subs > SEP_MAX_P ? SEP_MAX_P : 3 * g.subs;
                     // deep patch prefetch first, then one spare W block, a third A stage, a second staging panel
                     // (direct epilogue: a fourth A stage lets the depthwise warps run further ahead while the accumulator drains;
                     // it measured better than a fourth W block)
                     const int score = (pst >= want ? 1000 : pst * 100) + (wst > min_w + (direct ? 0 : 1) ? min_w + (direct ? 0 : 1) : wst) * 20 +
-                                      (g.cl > 1 ? (ast > 4 ? 4 : ast) * 16 : ast * (direct ? 24 : 8)) + stg * 4 + (pst > want ? 1 : 0);
+                                      ast * (direct ? 24 : 8) + stg * 4 + (pst > want ? 1 : 0);
                     if (score > bestp) {
                         bestp = score;
                         g.p_stages = pst; g.w_stages = wst; g.a_stages = ast; g.stg_bufs = stg;
@@ -1051,27 +893,20 @@ int sep_geometry(SepOp *op, int n, int h, int wd, int k, int nc, int stride, int
         if (tuned && tuned->p > 0 && g.th == tuned->th && g.tw == tuned->tw && g.subs == tuned->subs) { fp = tuned->p; fw = tuned->w; fa = tuned->a; fs = tuned->stg; have = true; }
         if (const char *force = getenv("PN_SEP_STAGES")) have = sscanf(force, "%d,%d,%d,%d", &fp, &fw, &fa, &fs) == 4;
         if (have && fp >= g.subs + 1 && fp <= SEP_MAX_P && fw >= 1 &&
-            fw <= SEP_MAX_W && fa >= 2 && fa <= SEP_MAX_A && fa % g.cl == 0 && fs >= 0 && fs <= 2 && fits(fp, fw, fa, fs)) {
+            fw <= SEP_MAX_W && fa >= 2 && fa <= SEP_MAX_A && fs >= 0 && fs <= 2 && fits(fp, fw, fa, fs)) {
             g.p_stages = fp; g.w_stages = fw; g.a_stages = fa; g.stg_bufs = fs;
         }
     }
-#ifdef PN_SEP_EXP
-    if (const char *e = getenv("PN_SEP_EXP")) g.exp = atoi(e);
-#endif
     if (g.w_res && g.w_stages != g.kblocks * g.n_halves) g.w_res = 0;   // (a forced ring depth: back to the ring)
     // Depthwise warp teams (see the kernel): two items in flight need a patch stage per team and sub-tile plus one ahead, an A
     // stage per team plus the one the MMAs read, and -- for the parity of a barrier a team returns to -- a patch ring at least as
     // deep as the A ring (an item whose A stage is free has had the patch stage's previous user consumed).  PN_SEP_TEAMS=1 / 2.
-    g.teams = (g.cl == 1 && SEP_DW_WARPS % 2 == 0 && g.p_stages >= 2 * g.subs + 1 && g.a_stages >= 3 && g.p_stages >= g.a_stages) ? 2 : 1;
+    g.teams = (SEP_DW_WARPS % 2 == 0 && g.p_stages >= 2 * g.subs + 1 && g.a_stages >= 3 && g.p_stages >= g.a_stages) ? 2 : 1;
     {
         const char *e = getenv("PN_SEP_TEAMS");
         const int v = e ? atoi(e) : (tuned && tuned->p > 0 && g.th == tuned->th && g.tw == tuned->tw && g.subs == tuned->subs) ? tuned->teams : 0;
-        if (v == 1 || (v == 2 && g.cl == 1 && SEP_DW_WARPS % 2 == 0 && g.p_stages >= 2 * g.subs && g.a_stages >= 2 && g.p_stages >= g.a_stages)) g.teams = v;
-        // three teams (4 + 3 + 3 warps): three items in flight
-        if (v == 3 && g.cl == 1 && SEP_DW_WARPS >= 6 && g.p_stages >= 3 * g.subs && g.a_stages >= 3 && g.p_stages >= g.a_stages) g.teams = 3;
+        if (v == 1 || (v == 2 && SEP_DW_WARPS % 2 == 0 && g.p_stages >= 2 * g.subs && g.a_stages >= 2 && g.p_stages >= g.a_stages)) g.teams = v;
     }
-    g.epi_sleep_ns = 200;
-    if (const char *e = getenv("PN_SEP_EPI_SLEEP")) g.epi_sleep_ns = (unsigned)atoi(e);
     static_assert(SepBars::total <= 640, "barrier block exceeds its reserve");
     g.off_a = (unsigned)g.w_stages * g.w_stage_bytes;
     g.off_stg = g.off_a + (unsigned)g.a_stages * SEP_A_BYTES;
@@ -1139,54 +974,32 @@ int sep_prepare(SepOp *op, const void *x, const float *dw_w, const float *dw_b, 
     return PN_OK;
 }
 
-template <int S, int D, bool HALF, int CL>
+template <int S, int D, bool HALF>
 static int sep_launch_t(const SepOp *op, const SepGeom &g, const float *pw_bias, cudaStream_t st) {
-    static DeviceOnce once, clusters;                             // per device: attribute set / clusters that fit at once
+    static DeviceOnce once;                                       // per device: attribute set
     const int dev = current_device();
-    auto kern = sepconv_kernel<S, D, HALF, CL>;
+    auto kern = sepconv_kernel<S, D, HALF>;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
     cudaLaunchAttribute attr[1];
-    if (CL > 1) {
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    } else {                                                      // PDL (common.cuh: launch_pdl) for the single-CTA variant
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-    }
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;   // PDL (common.cuh: launch_pdl)
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.blockDim = dim3(SEP_THREADS, 1, 1);
     cfg.dynamicSmemBytes = (size_t)op->smem_bytes;
     cfg.stream = st;
     cfg.attrs = attr;
-    cfg.numAttrs = (CL > 1 || pdl_enabled()) ? 1 : 0;
+    cfg.numAttrs = pdl_enabled() ? 1 : 0;
     if (!once.get(dev)) {
         PN_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SEP_SMEM_MAX));
-        if (CL > 1) {                                             // how many clusters fit at once (GPC boundaries cost a few SMs)
-            int max_clusters = 0;
-            cfg.gridDim = dim3((unsigned)(num_sms() / CL * CL), 1, 1);
-            cfg.dynamicSmemBytes = SEP_SMEM_MAX;
-            PN_CHECK_CUDA(cudaOccupancyMaxActiveClusters(&max_clusters, kern, &cfg));
-            PN_CHECK_ARG(max_clusters > 0, "pn_sepconv_block: no %d-CTA cluster fits on this device", CL);
-            cfg.dynamicSmemBytes = (size_t)op->smem_bytes;
-            clusters.set(dev, max_clusters);
-        }
         once.set(dev, 1);
     }
-    const long long units = CL > 1 ? clusters.get(dev) : num_sms();     // persistent: one CTA (cluster) per SM (SM group)
-    const int grid = (int)(g.tiles < units ? g.tiles : units) * CL;
-    cfg.gridDim = dim3((unsigned)grid, 1, 1);
+    const long long units = num_sms();                            // persistent: one CTA per SM
+    cfg.gridDim = dim3((unsigned)(g.tiles < units ? g.tiles : units), 1, 1);
     PN_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, *reinterpret_cast<const CUtensorMap *>(op->tmap_x),
                                      *reinterpret_cast<const CUtensorMap *>(op->tmap_dww), *reinterpret_cast<const CUtensorMap *>(op->tmap_dwb),
                                      *reinterpret_cast<const CUtensorMap *>(op->tmap_w), *reinterpret_cast<const CUtensorMap *>(op->tmap_y),
                                      pw_bias, reinterpret_cast<__nv_bfloat16 *>(op->y), op->dw_w, op->dw_b, g));
     return PN_OK;
-}
-
-template <int S, int D>
-static int sep_launch_cl(const SepOp *op, const SepGeom &g, const float *pw_bias, cudaStream_t st) {
-    if (g.cl == 2) return sep_launch_t<S, D, false, 2>(op, g, pw_bias, st);
-    if (g.cl == 4) return sep_launch_t<S, D, false, 4>(op, g, pw_bias, st);
-    return sep_launch_t<S, D, false, 1>(op, g, pw_bias, st);
 }
 
 int sep_launch(const SepOp *op, const float *pw_bias, cudaStream_t st) {
@@ -1195,11 +1008,11 @@ int sep_launch(const SepOp *op, const float *pw_bias, cudaStream_t st) {
     if (op->tc_kind) return septc_launch(&op->tc, op->dw_w, op->dw_b, pw_bias, op->y, st);
     SepGeom g;
     memcpy(&g, op->geom, sizeof(g));
-    if (op->stride == 2) return sep_launch_cl<2, 1>(op, g, pw_bias, st);
-    if (g.half) return sep_launch_t<1, 1, true, 1>(op, g, pw_bias, st);
-    if (op->dil == 1) return sep_launch_cl<1, 1>(op, g, pw_bias, st);
-    if (op->dil == 2) return sep_launch_cl<1, 2>(op, g, pw_bias, st);
-    return sep_launch_cl<1, 4>(op, g, pw_bias, st);
+    if (op->stride == 2) return sep_launch_t<2, 1, false>(op, g, pw_bias, st);
+    if (g.half) return sep_launch_t<1, 1, true>(op, g, pw_bias, st);
+    if (op->dil == 1) return sep_launch_t<1, 1, false>(op, g, pw_bias, st);
+    if (op->dil == 2) return sep_launch_t<1, 2, false>(op, g, pw_bias, st);
+    return sep_launch_t<1, 4, false>(op, g, pw_bias, st);
 }
 
 void sep_describe(const SepOp *op, char *out, size_t cap) {
@@ -1215,8 +1028,8 @@ void sep_describe(const SepOp *op, char *out, size_t cap) {
     }
     SepGeom g;
     memcpy(&g, op->geom, sizeof(g));
-    snprintf(out, cap, "%s%stile %dx%d subs %d box %dx%d segs %d x %d rows n_tile %d(%dx%d) x%d kblocks %d teams %d stages p%d w%d%s a%d stg%d smem %d tiles %lld",
-             g.half ? "half " : "", g.cl == 2 ? "cluster2 " : g.cl == 4 ? "cluster4 " : "", g.th, g.tw, g.subs, g.thi, g.twi, g.segs_per_sub, g.seg_rows, g.n_tile, g.n_halves, g.n_half, g.n_tiles, g.kblocks, g.teams, g.p_stages,
+    snprintf(out, cap, "%stile %dx%d subs %d box %dx%d segs %d x %d rows n_tile %d(%dx%d) x%d kblocks %d teams %d stages p%d w%d%s a%d stg%d smem %d tiles %lld",
+             g.half ? "half " : "", g.th, g.tw, g.subs, g.thi, g.twi, g.segs_per_sub, g.seg_rows, g.n_tile, g.n_halves, g.n_half, g.n_tiles, g.kblocks, g.teams, g.p_stages,
              g.w_stages, g.w_res ? "r" : "", g.a_stages, g.stg_bufs, op->smem_bytes, g.tiles);
 }
 

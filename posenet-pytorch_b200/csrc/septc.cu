@@ -1,5 +1,5 @@
 // B3 + B4 fused with the DEPTHWISE ON THE TENSOR PIPE -- one SeperableConv block (posenet/models/mobilenet_v1.py:57-68 of the
-// reference), stride 1, dilation 1 / 2, cin and cout multiples of 64:
+// reference), stride 1, dilation 1 / 2, cin = cout = 256:
 //     y = relu6( pointwise1x1( relu6( depthwise3x3(x; dilation) + b_dw ) ) + b_pw )
 // The CUDA-core depthwise of sepconv.cu is issue-bound (~12 thread-instructions per output).  Here the 3x3 depthwise is nine
 // tcgen05.mma per 16-channel group against block-diagonal weight tiles:
@@ -16,20 +16,18 @@
 //
 // Work unit: 128 consecutive flat positions ("chunk") of one column band of one image.  Two step sequences per CTA:
 //   depthwise step d = (unit, k-block)            patch stage d % PS, diag / depthwise-accumulator buffer d % 2
-//   pointwise step s = (unit, n-tile, k-block)    W stage s % WS
-// A operands (32 TMEM columns each): cout <= 256 ("ring"): one n-tile, 4 buffers used round-robin, so the depthwise runs up to
-// four k-blocks ahead of the pointwise MMAs (covers the epilogue of a single-buffered accumulator); cout > 256 ("cache"):
-// n-tiles of 128, the A operands of ALL k-blocks of a unit stay in TMEM (<= 8 x 32 columns) and every n-tile re-reads them --
-// the depthwise is computed once per unit, not once per n-tile.
+//   pointwise step s = (unit, k-block)            W stage s % WS, A operand s % 4
+// A operands (32 TMEM columns each): 4 buffers used round-robin, so the depthwise runs up to four k-blocks ahead of the
+// pointwise MMAs (covers the epilogue of the single-buffered accumulator).
 //   warp 0        patch producer  TMA box [64 ch, wp, rows_box] (OOB zero fill == zero padding), 128B swizzle
-//   warp 15       W producer      pointwise weight tile [n_tile x 64] (128B swizzle)
+//   warp 15       W producer      pointwise weight tile [256 x 64] (128B swizzle)
 //   warps 16-17   depthwise MMA   warp 16 + w issues the 2 x 9 tap MMAs of channel groups 2w, 2w+1; commits release patch / diag stages
 //   warps 2-5     converters      tcgen05.ld depthwise accumulator -> bias, ReLU6, bf16x2 -> tcgen05.st (A operand)
 //   warp 1        pointwise MMA   4 MMAs per step, A from TMEM; commits release the W stage, the A operand, and signal the epilogue
 //   warps 6-13    epilogue        tcgen05.ld 32 accumulator columns -> bias, ReLU6 -> bf16 -> warp-private staging -> coalesced
 //                                 predicated 16-byte global stores
 //   warp 14       diag writer     the 9 x 4 diagonal weight tiles of the next k-block (576 bf16 values into pre-zeroed tiles)
-// TMEM (512 columns): accumulator(s) at 0, A operands from 256 (ring) / 128 (cache) up to 384, depthwise accumulators 2 x 64 at 384.
+// TMEM (512 columns): accumulator at 0, A operands 4 x 32 at 256, depthwise accumulators 2 x 64 at 384.
 #include <cuda.h>
 #include <stdlib.h>
 #include <string.h>
@@ -41,24 +39,25 @@ namespace pn {
 
 constexpr int TCS_WARPS = 18;
 constexpr int TCS_THREADS = TCS_WARPS * 32;
-constexpr int TCS_MAX_P = 4, TCS_MAX_W = 4, TCS_MAX_A = 8;
+constexpr int TCS_MAX_P = 4, TCS_MAX_W = 4, TCS_A_BUFS = 4;
 constexpr int TCS_DIAG_BYTES = 9 * 16 * 128;          // nine [16 x 64] bf16 tiles
 constexpr int TCS_STG_BYTES = 32 * 64;                // per epilogue warp: 32 rows x 32 bf16
 constexpr int TCS_EPI_WARPS = 8;
 constexpr int TCS_DW_ISSUERS = 2;
 constexpr int TCS_SMEM_MAX = 232448;
-constexpr uint32_t TCS_DW_COL = 384;
+constexpr uint32_t TCS_A_COL = 256, TCS_DW_COL = 384;
+// Every mbarrier poll is a shared-memory wavefront, and the shared-memory pipe is what bounds this kernel (tensor-operand
+// fetches): waiting warps sleep between polls (ns) instead of re-polling every few tens of cycles.
+constexpr unsigned TCS_SLEEP_PRODUCER = 100, TCS_SLEEP_MMA = 32, TCS_SLEEP_CONVERT = 64, TCS_SLEEP_EPI = 300, TCS_SLEEP_DIAG = 200;
 
 struct TcsGeom {
     int k, nc, h, w, n_img, dil;
     int wp, tw, bands, rows_box, chunks;
-    int n_tile, n_tiles, kblocks, acc_bufs;
-    int ring, na, a_col;                                // A operand buffers: ring of 4 (one n-tile) or one per k-block (cache)
+    int kblocks;
     int p_stages, w_stages;
     unsigned patch_bytes, patch_stage_bytes, w_stage_bytes;
     unsigned off_diag, off_patch, off_stg, off_dww, off_dwb, off_pwb, off_bar;
     unsigned magic_wp;
-    unsigned sleep_ns[5];                               // poll backoff per role: producers, MMA issuers, converters, epilogue, diag writer
     long long units;
 };
 
@@ -156,7 +155,7 @@ septc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__
             mbar_init(bar(TcsBars::tfull, s), 1);
             mbar_init(bar(TcsBars::tempty, s), TCS_EPI_WARPS * 32);
         }
-        for (int s = 0; s < TCS_MAX_A; ++s) {
+        for (int s = 0; s < TCS_A_BUFS; ++s) {
             mbar_init(bar(TcsBars::a_full, s), 128);
             mbar_init(bar(TcsBars::a_empty, s), 1);
         }
@@ -190,18 +189,6 @@ septc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__
     long long *tr = blockIdx.x == 0 ? g_tcs_trace : nullptr;
     const int tr_cap = g_tcs_trace_cap;
 #endif
-    // A operand of depthwise step (unit i, k-block kb): buffer index and how many times that buffer was used before
-    auto a_slot = [&](int i, int kb, int &ai, uint32_t &use) {
-        if (g.ring) {
-            const int d = i * g.kblocks + kb;
-            ai = d & 3;
-            use = (uint32_t)(d >> 2);
-        } else {
-            ai = kb;
-            use = (uint32_t)i;
-        }
-    };
-
     if (warp == 0) {
         // ===================== patch producer =====================
         if (lane == 0) {
@@ -213,7 +200,7 @@ septc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__
                 const int row0 = (int)__umulhi((uint32_t)(chunk * 128), g.magic_wp);
                 const int x_org = band * g.tw - g.dil, y_org = row0 - g.dil;
                 for (int kb = 0; kb < g.kblocks; ++kb, ++d) {
-                    mbar_wait_backoff(bar(TcsBars::patch_empty, ps), pph ^ 1u, g.sleep_ns[0]);
+                    mbar_wait_backoff(bar(TcsBars::patch_empty, ps), pph ^ 1u, TCS_SLEEP_PRODUCER);
                     TCS_TR(0, d, 0);
                     mbar_expect_tx(bar(TcsBars::patch_full, ps), g.patch_bytes);
                     tma_load_4d(p_addr(ps), &tmap_x, bar(TcsBars::patch_full, ps), kb * 64, x_org, y_org, img);
@@ -227,48 +214,42 @@ septc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__
             int ws = 0, s = 0;
             uint32_t wph = 0;
             for (int i = 0; i < my_units; ++i)
-                for (int nt = 0; nt < g.n_tiles; ++nt)
-                    for (int kb = 0; kb < g.kblocks; ++kb, ++s) {
-                        mbar_wait_backoff(bar(TcsBars::w_empty, ws), wph ^ 1u, g.sleep_ns[0]);
-                        TCS_TR(0, s, 1);
-                        mbar_expect_tx(bar(TcsBars::w_full, ws), g.w_stage_bytes);
-                        tma_load_2d(w_addr(ws), &tmap_w, bar(TcsBars::w_full, ws), kb * 64, nt * g.n_tile);
-                        if (++ws == g.w_stages) { ws = 0; wph ^= 1u; }
-                    }
+                for (int kb = 0; kb < g.kblocks; ++kb, ++s) {
+                    mbar_wait_backoff(bar(TcsBars::w_empty, ws), wph ^ 1u, TCS_SLEEP_PRODUCER);
+                    TCS_TR(0, s, 1);
+                    mbar_expect_tx(bar(TcsBars::w_full, ws), g.w_stage_bytes);
+                    tma_load_2d(w_addr(ws), &tmap_w, bar(TcsBars::w_full, ws), kb * 64, 0);
+                    if (++ws == g.w_stages) { ws = 0; wph ^= 1u; }
+                }
         }
     } else if (warp == 1) {
         // ===================== pointwise MMA issuer (A operand in TMEM) =====================
         if (lane == 0) {
-            const uint32_t idesc_n = tcs_idesc(g.n_tile);
+            const uint32_t idesc_n = tcs_idesc(g.nc);
             const uint64_t desc_hi = tcs_desc(0);
-            int pws = 0, s = 0, item = 0;
+            int pws = 0, s = 0;
             uint32_t pwph = 0;
             for (int i = 0; i < my_units; ++i)
-                for (int nt = 0; nt < g.n_tiles; ++nt, ++item) {
-                    const int t = g.acc_bufs == 2 ? (item & 1) : 0;
-                    const uint32_t tuse = (uint32_t)(g.acc_bufs == 2 ? item >> 1 : item);
-                    for (int kb = 0; kb < g.kblocks; ++kb, ++s) {
-                        int ai;
-                        uint32_t use;
-                        a_slot(i, kb, ai, use);
-                        TCS_TR(1, s, 0);
-                        if (kb == 0) mbar_wait_backoff(bar(TcsBars::tempty, t), (tuse & 1u) ^ 1u, g.sleep_ns[1]);
-                        mbar_wait_backoff(bar(TcsBars::w_full, pws), pwph, g.sleep_ns[1]);
-                        TCS_TR(1, s, 1);
-                        mbar_wait_backoff(bar(TcsBars::a_full, ai), use & 1u, g.sleep_ns[1]);
-                        TCS_TR(1, s, 2);
-                        tc_fence_after();
-                        const uint32_t w0 = (w_addr(pws) & 0x3FFFF) >> 4;
-                        const uint32_t acol = tmem + (uint32_t)(g.a_col + ai * 32), ccol = tmem + (uint32_t)(t * g.n_tile);
+                for (int kb = 0; kb < g.kblocks; ++kb, ++s) {
+                    const int ai = s & (TCS_A_BUFS - 1);
+                    const uint32_t use = (uint32_t)s / TCS_A_BUFS;            // earlier uses of A operand ai
+                    TCS_TR(1, s, 0);
+                    if (kb == 0) mbar_wait_backoff(bar(TcsBars::tempty, 0), ((uint32_t)i & 1u) ^ 1u, TCS_SLEEP_MMA);
+                    mbar_wait_backoff(bar(TcsBars::w_full, pws), pwph, TCS_SLEEP_MMA);
+                    TCS_TR(1, s, 1);
+                    mbar_wait_backoff(bar(TcsBars::a_full, ai), use & 1u, TCS_SLEEP_MMA);
+                    TCS_TR(1, s, 2);
+                    tc_fence_after();
+                    const uint32_t w0 = (w_addr(pws) & 0x3FFFF) >> 4;
+                    const uint32_t acol = tmem + TCS_A_COL + (uint32_t)(ai * 32);
 #pragma unroll
-                        for (int k4 = 0; k4 < 4; ++k4)
-                            tcs_mma_ts(ccol, acol + k4 * 8, desc_hi | (uint64_t)(w0 + k4 * 2), idesc_n, (kb > 0 || k4 > 0));
-                        tc_commit(bar(TcsBars::w_empty, pws));
-                        if (g.ring || nt == g.n_tiles - 1) tc_commit(bar(TcsBars::a_empty, ai));
-                        if (kb == g.kblocks - 1) tc_commit(bar(TcsBars::tfull, t));
-                        TCS_TR(1, s, 3);
-                        if (++pws == g.w_stages) { pws = 0; pwph ^= 1u; }
-                    }
+                    for (int k4 = 0; k4 < 4; ++k4)
+                        tcs_mma_ts(tmem, acol + k4 * 8, desc_hi | (uint64_t)(w0 + k4 * 2), idesc_n, (kb > 0 || k4 > 0));
+                    tc_commit(bar(TcsBars::w_empty, pws));
+                    tc_commit(bar(TcsBars::a_empty, ai));
+                    if (kb == g.kblocks - 1) tc_commit(bar(TcsBars::tfull, 0));
+                    TCS_TR(1, s, 3);
+                    if (++pws == g.w_stages) { pws = 0; pwph ^= 1u; }
                 }
         }
     } else if (warp >= 16) {
@@ -289,11 +270,11 @@ septc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__
                 for (int kb = 0; kb < g.kblocks; ++kb, ++d) {
                     const int db = d & 1;
                     const uint32_t dph = (uint32_t)(d >> 1) & 1u;
-                    mbar_wait_backoff(bar(TcsBars::dw_free, db), dph ^ 1u, g.sleep_ns[1]);            // the converters have read accumulator db (step d - 2)
+                    mbar_wait_backoff(bar(TcsBars::dw_free, db), dph ^ 1u, TCS_SLEEP_MMA);            // the converters have read accumulator db (step d - 2)
                     if (w2 == 0) TCS_TR(2, d, 0);
-                    mbar_wait_backoff(bar(TcsBars::patch_full, dps), dpph, g.sleep_ns[1]);
+                    mbar_wait_backoff(bar(TcsBars::patch_full, dps), dpph, TCS_SLEEP_MMA);
                     if (w2 == 0) TCS_TR(2, d, 1);
-                    mbar_wait_backoff(bar(TcsBars::diag_full, db), dph, g.sleep_ns[1]);
+                    mbar_wait_backoff(bar(TcsBars::diag_full, db), dph, TCS_SLEEP_MMA);
                     if (w2 == 0) TCS_TR(2, d, 2);
                     tc_fence_after();
                     const uint32_t a0 = ((p_addr(dps) & 0x3FFFF) >> 4) + qoff, b0 = ((d_addr(db) & 0x3FFFF) >> 4) + (uint32_t)w2 * 4u;
@@ -320,10 +301,9 @@ septc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__
         for (int i = 0; i < my_units; ++i)
             for (int kb = 0; kb < g.kblocks; ++kb, ++d) {
                 const int b = d & 1;
-                int ai;
-                uint32_t use;
-                a_slot(i, kb, ai, use);
-                mbar_wait_backoff(bar(TcsBars::dw_full, b), (uint32_t)(d >> 1) & 1u, g.sleep_ns[2]);
+                const int a = i * g.kblocks + kb, ai = a & (TCS_A_BUFS - 1);   // A operand of step d (== d, but written from (i, kb):
+                const uint32_t use = (uint32_t)a / TCS_A_BUFS;                 // with the counter itself ptxas spills in this kernel)
+                mbar_wait_backoff(bar(TcsBars::dw_full, b), (uint32_t)(d >> 1) & 1u, TCS_SLEEP_CONVERT);
                 if (threadIdx.x == 64) TCS_TR(3, d, 0);
                 tc_fence_after();
                 uint32_t v[32], pk[32];
@@ -343,10 +323,10 @@ septc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__
                     }
                 }
                 if (threadIdx.x == 64) TCS_TR(3, d, 1);
-                mbar_wait_backoff(bar(TcsBars::a_empty, ai), (use & 1u) ^ 1u, g.sleep_ns[2]);       // the pointwise MMAs have read the previous content
+                mbar_wait_backoff(bar(TcsBars::a_empty, ai), (use & 1u) ^ 1u, TCS_SLEEP_CONVERT);       // the pointwise MMAs have read the previous content
                 if (threadIdx.x == 64) TCS_TR(3, d, 2);
                 tc_fence_after();
-                tcs_st32(tmem + lane_off + (uint32_t)(g.a_col + ai * 32), pk);
+                tcs_st32(tmem + lane_off + TCS_A_COL + (uint32_t)(ai * 32), pk);
                 tcs_st_wait();
                 tc_fence_before();
                 mbar_arrive(bar(TcsBars::a_full, ai));
@@ -358,9 +338,9 @@ septc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__
         const uint32_t lane_off = (uint32_t)(quad * 32) << 16;
         const uint32_t stg = base + g.off_stg + (uint32_t)ew * TCS_STG_BYTES;
         const uint32_t spwb = base + g.off_pwb;
-        const int slabs = g.n_tile / 32;
+        const int slabs = g.nc / 32;
         int item = 0;
-        for (long long u = blockIdx.x; u < g.units; u += ustride) {
+        for (long long u = blockIdx.x; u < g.units; u += ustride, ++item) {
             const int img = (int)(u / per_img), rem = (int)(u - (long long)img * per_img);
             const int band = rem / g.chunks, chunk = rem - band * g.chunks;
             long long pix[4];                                     // element offset of the pixel this lane stores in pass i, or -1
@@ -371,44 +351,40 @@ septc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__
                 const int gx = band * g.tw + tx;
                 pix[i] = (tx < g.tw && gx < g.w && ty < g.h) ? (((long long)img * g.h + ty) * g.w + gx) * g.nc : -1;
             }
-            for (int nt = 0; nt < g.n_tiles; ++nt, ++item) {
-                const int t = g.acc_bufs == 2 ? (item & 1) : 0;
-                const uint32_t tuse = (uint32_t)(g.acc_bufs == 2 ? item >> 1 : item);
-                mbar_wait_backoff(bar(TcsBars::tfull, t), tuse & 1u, g.sleep_ns[3]);
-                if (threadIdx.x == 192) TCS_TR(5, item, 0);
-                tc_fence_after();
-                for (int sl = half; sl < slabs; sl += 2) {
-                    uint32_t v[32];
-                    tc_ld32(tmem + lane_off + (uint32_t)(t * g.n_tile + sl * 32), v);
-                    tc_ld_wait();
-                    if (sl + 2 >= slabs) {                        // this warp's last read of the accumulator
-                        tc_fence_before();
-                        mbar_arrive(bar(TcsBars::tempty, t));
-                        if (threadIdx.x == 192) TCS_TR(5, item, 1);
-                    }
-                    const uint32_t bcol = spwb + (uint32_t)(nt * g.n_tile + sl * 32) * 4u;
-                    const uint32_t row = stg + (uint32_t)lane * 64u;
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        const float4 b0 = tcs_lds_f4(bcol + (uint32_t)j * 32u), b1 = tcs_lds_f4(bcol + (uint32_t)j * 32u + 16u);
-                        st_shared_v4(row + (uint32_t)((j ^ ((lane >> 1) & 3)) * 16),
-                                     relu6_bf16x2(__uint_as_float(v[8 * j]) + b0.x, __uint_as_float(v[8 * j + 1]) + b0.y),
-                                     relu6_bf16x2(__uint_as_float(v[8 * j + 2]) + b0.z, __uint_as_float(v[8 * j + 3]) + b0.w),
-                                     relu6_bf16x2(__uint_as_float(v[8 * j + 4]) + b1.x, __uint_as_float(v[8 * j + 5]) + b1.y),
-                                     relu6_bf16x2(__uint_as_float(v[8 * j + 6]) + b1.z, __uint_as_float(v[8 * j + 7]) + b1.w));
-                    }
-                    __syncwarp();
-                    const int ccol = nt * g.n_tile + sl * 32 + (lane & 3) * 8;
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const int r = i * 8 + (lane >> 2);
-                        const uint4 val = ld_shared_v4(stg + (uint32_t)r * 64u + (uint32_t)(((lane & 3) ^ ((r >> 1) & 3)) * 16));
-                        if (pix[i] >= 0) tcs_stg_v4(y + pix[i] + ccol, val);
-                    }
-                    __syncwarp();
+            mbar_wait_backoff(bar(TcsBars::tfull, 0), (uint32_t)item & 1u, TCS_SLEEP_EPI);
+            if (threadIdx.x == 192) TCS_TR(5, item, 0);
+            tc_fence_after();
+            for (int sl = half; sl < slabs; sl += 2) {
+                uint32_t v[32];
+                tc_ld32(tmem + lane_off + (uint32_t)(sl * 32), v);
+                tc_ld_wait();
+                if (sl + 2 >= slabs) {                        // this warp's last read of the accumulator
+                    tc_fence_before();
+                    mbar_arrive(bar(TcsBars::tempty, 0));
+                    if (threadIdx.x == 192) TCS_TR(5, item, 1);
                 }
-                if (threadIdx.x == 192) TCS_TR(5, item, 2);
+                const uint32_t bcol = spwb + (uint32_t)(sl * 32) * 4u;
+                const uint32_t row = stg + (uint32_t)lane * 64u;
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    const float4 b0 = tcs_lds_f4(bcol + (uint32_t)j * 32u), b1 = tcs_lds_f4(bcol + (uint32_t)j * 32u + 16u);
+                    st_shared_v4(row + (uint32_t)((j ^ ((lane >> 1) & 3)) * 16),
+                                 relu6_bf16x2(__uint_as_float(v[8 * j]) + b0.x, __uint_as_float(v[8 * j + 1]) + b0.y),
+                                 relu6_bf16x2(__uint_as_float(v[8 * j + 2]) + b0.z, __uint_as_float(v[8 * j + 3]) + b0.w),
+                                 relu6_bf16x2(__uint_as_float(v[8 * j + 4]) + b1.x, __uint_as_float(v[8 * j + 5]) + b1.y),
+                                 relu6_bf16x2(__uint_as_float(v[8 * j + 6]) + b1.z, __uint_as_float(v[8 * j + 7]) + b1.w));
+                }
+                __syncwarp();
+                const int ccol = sl * 32 + (lane & 3) * 8;
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    const int r = i * 8 + (lane >> 2);
+                    const uint4 val = ld_shared_v4(stg + (uint32_t)r * 64u + (uint32_t)(((lane & 3) ^ ((r >> 1) & 3)) * 16));
+                    if (pix[i] >= 0) tcs_stg_v4(y + pix[i] + ccol, val);
+                }
+                __syncwarp();
             }
+            if (threadIdx.x == 192) TCS_TR(5, item, 2);
         }
     } else if (warp == 14) {
         // ===================== diagonal weight tiles =====================
@@ -422,7 +398,7 @@ septc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__
         for (int i = 0; i < my_units; ++i)
             for (int kb = 0; kb < g.kblocks; ++kb, ++d) {
                 const int db = d & 1;
-                mbar_wait_backoff(bar(TcsBars::diag_empty, db), ((uint32_t)(d >> 1) & 1u) ^ 1u, g.sleep_ns[4]);
+                mbar_wait_backoff(bar(TcsBars::diag_empty, db), ((uint32_t)(d >> 1) & 1u) ^ 1u, TCS_SLEEP_DIAG);
                 if (lane == 0) TCS_TR(4, d, 0);
                 if (g.kblocks > 2 || d < 2) {                      // with <= 2 k-blocks each buffer keeps its k-block for good
                     const uint32_t dst = d_addr(db);
@@ -454,26 +430,13 @@ septc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__
 }
 
 // ---- host side ---------------------------------------------------------------------------------------------
-bool septc_supported(int k, int nc, int stride, int dil) {
-    if (!(stride == 1 && (dil == 1 || dil == 2) && k % 64 == 0 && nc % 64 == 0 && k >= 64 && k <= 512 && nc >= 64 && nc <= 512)) return false;
-    return nc <= 256 || nc % 128 == 0;                  // wider blocks run n-tiles of 128 over cached A operands (<= 8 k-blocks)
-}
-// Which blocks take this path.  Measured on B200 (profiles/r01_v9_septc_experiment.md): a tap MMA costs 32 + N/4 cycles (operand
-// fetch: every M128 x N16 x K16 MMA re-reads 4 KB of patch from shared memory), so the depthwise is no cheaper here than on the
-// CUDA cores and it serialises with the pointwise MMAs on the one tensor pipe.  It wins where the CUDA-core kernel is at its
-// weakest and this one at its best -- 256 -> 256 blocks (one 256-column n-tile, A ring): 0.178 vs 0.203 ms on the dilated blocks of
-// model 50 at OS8 (C3), 0.104 vs 0.107 ms on block 5 of model 101 (C2) -- and loses elsewhere (128 -> 128: 0.199 vs 0.186 ms,
-// 512 -> 512: 0.096 vs 0.073 ms).  PN_SEP_TC=1 forces it for every supported block, PN_SEP_TC=0 turns it off.
-bool septc_enabled() {
-    const char *e = getenv("PN_SEP_TC");
-    return !(e && e[0] == '0');
-}
-bool septc_preferred(int k, int nc, int stride, int dil) {
-    if (!septc_enabled() || !septc_supported(k, nc, stride, dil)) return false;
-    const char *e = getenv("PN_SEP_TC");
-    if (e && e[0] == '1') return true;
-    return k == 256 && nc == 256;
-}
+// Which blocks take this path: 256 -> 256, stride 1, dilation 1 or 2.  Measured on B200 (profiles/r01_v9_septc_experiment.md):
+// a tap MMA costs 32 + N/4 cycles (operand fetch: every M128 x N16 x K16 MMA re-reads 4 KB of patch from shared memory), so the
+// depthwise is no cheaper here than on the CUDA cores and it serialises with the pointwise MMAs on the one tensor pipe.  It wins
+// where the CUDA-core kernel is at its weakest and this one at its best -- 256 -> 256 blocks (one 256-column accumulator, A
+// ring): 0.178 vs 0.203 ms on the dilated blocks of model 50 at OS8 (C3), 0.104 vs 0.107 ms on block 5 of model 101 (C2) -- and
+// loses on the other widths it was tried at (128 -> 128: 0.199 vs 0.186 ms, 512 -> 512: 0.096 vs 0.073 ms).
+bool septc_supported(int k, int nc, int stride, int dil) { return stride == 1 && (dil == 1 || dil == 2) && k == 256 && nc == 256; }
 
 int septc_geometry(SepTcOp *op, int n, int h, int wd, int k, int nc, int dil) {
     PN_CHECK_ARG(septc_supported(k, nc, 1, dil), "septc: unsupported block");
@@ -481,20 +444,13 @@ int septc_geometry(SepTcOp *op, int n, int h, int wd, int k, int nc, int dil) {
     memset(&g, 0, sizeof(g));
     g.k = k; g.nc = nc; g.h = h; g.w = wd; g.n_img = n; g.dil = dil;
     g.kblocks = k / 64;
-    g.ring = nc <= 256;
-    g.n_tile = g.ring ? nc : 128;
-    g.n_tiles = nc / g.n_tile;
-    g.acc_bufs = (g.ring && g.n_tile <= 128) ? 2 : 1;
-    g.na = g.ring ? 4 : g.kblocks;
-    g.a_col = g.ring ? 256 : 128;
-    g.w_stage_bytes = (unsigned)g.n_tile * 128u;
+    g.w_stage_bytes = (unsigned)nc * 128u;
     const unsigned table_bytes = (unsigned)((9 * k * 2 + 15) / 16 * 16 + k * 4 + nc * 4);
     const long long fixed = 1024 + 2LL * TCS_DIAG_BYTES + (long long)TCS_EPI_WARPS * TCS_STG_BYTES + table_bytes + TcsBars::total;
     // column bands: pitch wp = tw + 2 dil (one band over the whole width shares the zero gap: wp = w + dil).  Cost per unit in
     // shared-memory cycles (128 B/clk): 9 tap reads of 128 rows + (half) the patch write per k-block, W write + read per pointwise
-    // step, + a per-unit overhead; the weights are fitted to band sweeps (PN_TCS_BANDS) on the C2 / C3 blocks: wide bands win.
+    // step, + a per-unit overhead; the weights are fitted to band sweeps on the C2 / C3 blocks: wide bands win.
     double best = 1e30;
-    const int force_bands = getenv("PN_TCS_BANDS") ? atoi(getenv("PN_TCS_BANDS")) : 0;      // tuning aid
     for (int bands = 1; bands <= 16; ++bands) {
         const int tw = ceil_div(wd, bands);
         if (bands > 1 && ceil_div(wd, tw) != bands) continue;
@@ -506,11 +462,10 @@ int septc_geometry(SepTcOp *op, int n, int h, int wd, int k, int nc, int dil) {
         const long long stage = (patch + 1023) / 1024 * 1024;
         if (fixed + 2 * stage + 2LL * g.w_stage_bytes > TCS_SMEM_MAX) continue;
         const int chunks = ceil_div((h - 1) * wp + tw, 128);
-        const double per_unit = g.kblocks * (1152.0 + patch / 256.0) + (double)g.n_tiles * g.kblocks * (2.0 * g.w_stage_bytes / 128.0) + 600.0;
+        const double per_unit = g.kblocks * (1152.0 + patch / 256.0) + g.kblocks * (2.0 * g.w_stage_bytes / 128.0) + 600.0;
         const double cost = (double)bands * chunks * per_unit;
         // (measured: fewer, wider bands win even when they leave room for two patch stages only -- C3 0.178 ms with 4 bands / 2
         // stages against 0.193 ms with 7 bands / 3 stages -- so the stage count is not part of the cost)
-        if (force_bands > 0 && bands != force_bands) continue;
         if (cost < best) {
             best = cost;
             g.bands = bands; g.tw = tw; g.wp = wp; g.rows_box = rows_box; g.chunks = chunks;
@@ -531,23 +486,6 @@ int septc_geometry(SepTcOp *op, int n, int h, int wd, int k, int nc, int dil) {
     if (total(3, 2) <= TCS_SMEM_MAX) g.p_stages = 3;
     while (g.w_stages < TCS_MAX_W && total(g.p_stages, g.w_stages + 1) <= TCS_SMEM_MAX) ++g.w_stages;
     if (g.p_stages == 3 && total(4, g.w_stages) <= TCS_SMEM_MAX) g.p_stages = 4;
-    if (const char *force = getenv("PN_TCS_STAGES")) {
-        int fp = 0, fw = 0;
-        if (sscanf(force, "%d,%d", &fp, &fw) == 2 && fp >= 2 && fp <= TCS_MAX_P && fw >= 2 && fw <= TCS_MAX_W && total(fp, fw) <= TCS_SMEM_MAX) {
-            g.p_stages = fp; g.w_stages = fw;
-        }
-    }
-    // Every mbarrier poll is a shared-memory wavefront, and the shared-memory pipe is what bounds this kernel (tensor-operand
-    // fetches): waiting warps sleep between polls instead of re-polling every few tens of cycles (PN_TCS_SLEEP="p,m,c,e,d" in ns).
-    {
-        const unsigned def_ns[5] = {100, 32, 64, 300, 200};
-        for (int i = 0; i < 5; ++i) g.sleep_ns[i] = def_ns[i];
-        if (const char *e = getenv("PN_TCS_SLEEP")) {
-            unsigned v[5];
-            if (sscanf(e, "%u,%u,%u,%u,%u", &v[0], &v[1], &v[2], &v[3], &v[4]) == 5)
-                for (int i = 0; i < 5; ++i) g.sleep_ns[i] = v[i];
-        }
-    }
     g.off_diag = (unsigned)g.w_stages * g.w_stage_bytes;
     g.off_patch = g.off_diag + 2u * TCS_DIAG_BYTES;
     g.off_stg = g.off_patch + (unsigned)g.p_stages * g.patch_stage_bytes;
@@ -573,10 +511,10 @@ int septc_prepare(SepTcOp *op, const void *x, const void *pw_w, int n, int h, in
         const uint32_t box[4] = {64u, (uint32_t)g.wp, (uint32_t)g.rows_box, 1u};
         if ((rc = encode_tmap(op->tmap_x, x, 2, 4, dims, strides, box, 3)) != PN_OK) return rc;
     }
-    {   // pointwise weights [Nc, K] bf16, box [64, n_tile], 128B swizzle
+    {   // pointwise weights [Nc, K] bf16, box [64, Nc], 128B swizzle
         const uint64_t dims[2] = {(uint64_t)k, (uint64_t)nc};
         const uint64_t strides[1] = {(uint64_t)k * 2};
-        const uint32_t box[2] = {64u, (uint32_t)g.n_tile};
+        const uint32_t box[2] = {64u, (uint32_t)nc};
         if ((rc = encode_tmap(op->tmap_w, pw_w, 2, 2, dims, strides, box, 3)) != PN_OK) return rc;
     }
     return PN_OK;
@@ -602,8 +540,8 @@ int septc_launch(const SepTcOp *op, const float *dw_w, const float *dw_b, const 
 void septc_describe(const SepTcOp *op, char *out, size_t cap) {
     TcsGeom g;
     memcpy(&g, op->geom, sizeof(g));
-    snprintf(out, cap, "tensor-pipe depthwise: bands %d x %d cols pitch %d box rows %d chunks %d n_tile %d x%d (acc bufs %d, A %s x%d) kblocks %d stages p%d w%d smem %d units %lld",
-             g.bands, g.tw, g.wp, g.rows_box, g.chunks, g.n_tile, g.n_tiles, g.acc_bufs, g.ring ? "ring" : "cache", g.na, g.kblocks, g.p_stages, g.w_stages, op->smem_bytes, g.units);
+    snprintf(out, cap, "tensor-pipe depthwise: bands %d x %d cols pitch %d box rows %d chunks %d kblocks %d stages p%d w%d smem %d units %lld",
+             g.bands, g.tw, g.wp, g.rows_box, g.chunks, g.kblocks, g.p_stages, g.w_stages, op->smem_bytes, g.units);
 }
 
 }  // namespace pn

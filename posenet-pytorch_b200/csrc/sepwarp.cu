@@ -543,21 +543,16 @@ sepwarpf_kernel(const __grid_constant__ CUtensorMap tmap_x, const float *__restr
 // ---- host side ---------------------------------------------------------------------------------------------
 // block shapes with an instantiation of the full-warp kernel (measured against the CTA pipeline on the blocks of models 75 / 50)
 static bool sepwarp_full_shape(int k, int nc, int stride) {
-    const char *e = getenv("PN_SEPWARP_FULL");
-    if (e && e[0] == '0') return false;
     // (64 -> 64 stride 1, the third block of model 50, was measured too -- sepwarpf_kernel<4, 8, 1>: 0.164 vs 0.160 ms on the CTA
     // pipeline at 181 x 321 x 32 -- and stays there)
     return k == 48 && nc == 96 && stride == 2;
 }
 
 bool sepwarp_supported(int k, int nc, int stride, int dil) {
-    if (dil == 1 && sepwarp_full_shape(k, nc, stride) && getenv("PN_NO_SEPWARP") == nullptr) return true;
-    if (!(dil == 1 && k >= 8 && k <= 32 && k % 8 == 0 && nc >= 8 && nc <= 64 && nc % 8 == 0 && getenv("PN_NO_SEPWARP") == nullptr)) return false;
-    if (stride == 1) return true;
-    // stride 2: cin 17..32 (the half-warp layout; narrower blocks would idle half its lanes).  PN_SEPWARP_S2=0 sends these blocks
-    // back to the CTA pipeline of sepconv.cu.
-    const char *e = getenv("PN_SEPWARP_S2");
-    return stride == 2 && k > 16 && !(e && e[0] == '0');
+    if (dil == 1 && sepwarp_full_shape(k, nc, stride)) return true;
+    if (!(dil == 1 && k >= 8 && k <= 32 && k % 8 == 0 && nc >= 8 && nc <= 64 && nc % 8 == 0)) return false;
+    // stride 2: cin 17..32 (the half-warp layout; narrower blocks would idle half its lanes)
+    return stride == 1 || (stride == 2 && k > 16);
 }
 
 // strips / row blocks / item count: pure host arithmetic (no CUDA calls beyond the cached SM count); h, wd: the INPUT map
@@ -578,33 +573,25 @@ int sepwarp_geometry(SepWarpOp *op, int n, int h, int wd, int k, int nc, int str
     // of input rows within 2 % across row-block counts; the per-item overhead is nil).  With only a handful of items per warp the
     // quantisation of that sum is worth 5-20 %, so every row-block count (blocks of at least 8 output rows) is simulated and the
     // best one taken: 64 x 257 x 257: 7 -> 10 blocks, 512 x 129 x 129: 2 -> 4, 32 x 361 x 641 stride 2: 11 -> 7.
-    // PN_SWP_ITEMS=n brings back the rule it replaces (about n items per warp).
     const int warps = num_sms() * SWP_WARPS;
     const int max_nq = ceil_div(g.h, 8);
     long long nq = 1;
-    if (const char *e = getenv("PN_SWP_ITEMS")) {
-        const long long per_warp = atoi(e) > 0 ? atoi(e) : 6;
-        nq = (per_warp * warps + (long long)n * g.strips - 1) / ((long long)n * g.strips);
-        if (nq > max_nq) nq = max_nq;
-        if (nq < 1) nq = 1;
-    } else {
-        std::vector<long long> load((size_t)warps);
-        long long best = -1;
-        for (int cand = 1; cand <= max_nq; ++cand) {
-            const int rb = ceil_div(g.h, cand);
-            if (ceil_div(g.h, rb) != cand) continue;                       // (the same blocks as a smaller count)
-            const long long items_c = (long long)n * g.strips * cand;
-            if (items_c > (1ll << 22)) break;                              // (plan-time work bound; never reached by the reference's sizes)
-            std::fill(load.begin(), load.end(), 0ll);
-            int wi = 0, xs = 0, q = 0;
-            for (long long it = 0; it < items_c; ++it) {
-                load[(size_t)wi] += (long long)(rb < g.h - q * rb ? rb : g.h - q * rb) * stride + (3 - stride);
-                if (++wi == warps) wi = 0;
-                if (++xs == g.strips) { xs = 0; if (++q == cand) q = 0; }
-            }
-            const long long worst = *std::max_element(load.begin(), load.end());
-            if (best < 0 || worst < best) { best = worst; nq = cand; }
+    std::vector<long long> load((size_t)warps);
+    long long best = -1;
+    for (int cand = 1; cand <= max_nq; ++cand) {
+        const int rb = ceil_div(g.h, cand);
+        if (ceil_div(g.h, rb) != cand) continue;                           // (the same blocks as a smaller count)
+        const long long items_c = (long long)n * g.strips * cand;
+        if (items_c > (1ll << 22)) break;                                  // (plan-time work bound; never reached by the reference's sizes)
+        std::fill(load.begin(), load.end(), 0ll);
+        int wi = 0, xs = 0, q = 0;
+        for (long long it = 0; it < items_c; ++it) {
+            load[(size_t)wi] += (long long)(rb < g.h - q * rb ? rb : g.h - q * rb) * stride + (3 - stride);
+            if (++wi == warps) wi = 0;
+            if (++xs == g.strips) { xs = 0; if (++q == cand) q = 0; }
         }
+        const long long worst = *std::max_element(load.begin(), load.end());
+        if (best < 0 || worst < best) { best = worst; nq = cand; }
     }
     g.rb = ceil_div(g.h, (int)nq);
     g.nq = ceil_div(g.h, g.rb);

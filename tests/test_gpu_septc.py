@@ -1,9 +1,9 @@
-"""Depthwise on the tensor pipe (csrc/septc.cu; default for 256 -> 256 blocks, PN_SEP_TC=1 forces it for every supported block) through the C ABI on the B200.
+"""Depthwise on the tensor pipe (csrc/septc.cu; the 256 -> 256 blocks at stride 1, dilation 1 or 2) through the C ABI on the B200.
 
 (1) pn_dwtc_probe: the hardware behaviours the kernel relies on -- a SWIZZLE_128B UMMA descriptor advanced by whole 128-byte
     rows reads a shifted view of the TMA-written patch (depthwise taps; equal to numpy fp32 up to rare one-ulp flips of the bf16 rounding), and tcgen05.mma takes
     its A operand from TMEM (pointwise on the depthwise result).
-(2) pn_sepconv_block with PN_SEP_TC=1 against a torch fp32 reference of mobilenet_v1.py:57-68 (SeperableConv) with the
+(2) pn_sepconv_block on those blocks against a torch fp32 reference of mobilenet_v1.py:57-68 (SeperableConv) with the
     kernel's rounding points: bf16 input, bf16 depthwise weights, bf16 depthwise output, bf16 output."""
 import ctypes as C
 
@@ -79,16 +79,16 @@ def test_shifted_descriptor_depthwise_and_tmem_operand(case):
     assert valid >= 100 and flips <= valid * 64 // 500
 
 
-SHAPES = [  # n, h, w, cin, cout, dilation -- ring mode (cout <= 256), cache mode (cout > 256), ragged bands, tiny maps
-    (2, 5, 3, 64, 64, 1), (1, 12, 33, 64, 64, 1), (3, 33, 33, 512, 512, 1), (2, 65, 65, 256, 256, 1), (2, 129, 129, 128, 128, 1),
-    (1, 46, 81, 128, 256, 1), (1, 46, 81, 256, 256, 2), (5, 17, 17, 384, 384, 1), (1, 91, 161, 256, 256, 2), (2, 33, 33, 192, 192, 1),
-    (1, 1, 1, 64, 128, 1), (2, 33, 33, 256, 512, 1),
+SHAPES = [  # n, h, w, cin, cout, dilation -- the blocks of models 101 / 50, one and two bands (ragged), tiny maps
+    (2, 65, 65, 256, 256, 1), (3, 33, 33, 256, 256, 1), (5, 17, 17, 256, 256, 1), (1, 45, 81, 256, 256, 1), (1, 12, 33, 256, 256, 1),
+    (2, 5, 3, 256, 256, 1), (1, 1, 1, 256, 256, 1),
+    (1, 91, 161, 256, 256, 2), (1, 46, 81, 256, 256, 2), (2, 33, 33, 256, 256, 2), (1, 12, 33, 256, 256, 2), (2, 5, 3, 256, 256, 2),
+    (1, 1, 1, 256, 256, 2), (4, 9, 9, 256, 256, 2),
 ]
 
 
-@pytest.mark.parametrize("shape", SHAPES)
-def test_sepconv_block_on_the_tensor_pipe(shape, monkeypatch):
-    monkeypatch.setenv("PN_SEP_TC", "1")
+@pytest.mark.parametrize("shape", SHAPES, ids=lambda s: "n%d-%dx%d-%dto%d-d%d" % s)
+def test_sepconv_block_on_the_tensor_pipe(shape):
     n, h, w, cin, cout, dil = shape
     buf = C.create_string_buffer(512)
     assert nat.load().pn_sepconv_describe(n, h, w, cin, cout, 1, dil, buf, 512) == 0
@@ -116,11 +116,8 @@ def test_sepconv_block_on_the_tensor_pipe(shape, monkeypatch):
     assert torch.equal(y, y2)                                # deterministic
 
 
-def test_default_policy(monkeypatch):
-    """Unset: only the 256 -> 256 blocks (where it measured faster) take the tensor-pipe depthwise; PN_SEP_TC=0: none."""
+def test_tensor_pipe_takes_the_256_blocks_only():
+    """Only the 256 -> 256 blocks (where it measured faster) take the tensor-pipe depthwise."""
     buf = C.create_string_buffer(512)
-    monkeypatch.delenv("PN_SEP_TC", raising=False)
     assert nat.load().pn_sepconv_describe(2, 33, 33, 512, 512, 1, 1, buf, 512) == 0 and b"tensor-pipe" not in buf.value
     assert nat.load().pn_sepconv_describe(2, 91, 161, 256, 256, 1, 2, buf, 512) == 0 and b"tensor-pipe" in buf.value
-    monkeypatch.setenv("PN_SEP_TC", "0")
-    assert nat.load().pn_sepconv_describe(2, 91, 161, 256, 256, 1, 2, buf, 512) == 0 and b"tensor-pipe" not in buf.value

@@ -63,83 +63,68 @@ def test_sepconv_tile_geometry_is_host_computable():
     assert lib.pn_sepconv_describe(2, 9, 9, 64, 64, 2, 2, buf, 256) != 0            # never produced by the tables
 
 
-def test_tensor_pipe_depthwise_policy_and_geometry(monkeypatch):
-    """PN_SEP_TC=1 routes stride-1 blocks with 64-multiple widths (<= 512) to csrc/septc.cu; band layout is host arithmetic."""
+def test_tensor_pipe_depthwise_routing_and_geometry():
+    """The 256 -> 256 blocks at stride 1, dilation 1 or 2 run on csrc/septc.cu (measured faster there); band layout is host
+    arithmetic."""
     import ctypes as C
     lib, buf = nat.load(), C.create_string_buffer(512)
-    monkeypatch.delenv("PN_SEP_TC", raising=False)                  # default policy: the 256 -> 256 blocks only
-    assert lib.pn_sepconv_describe(64, 33, 33, 512, 512, 1, 1, buf, 512) == 0 and b"tensor-pipe" not in buf.value
-    assert lib.pn_sepconv_describe(32, 91, 161, 256, 256, 1, 2, buf, 512) == 0 and b"tensor-pipe" in buf.value
-    monkeypatch.setenv("PN_SEP_TC", "0")
-    assert lib.pn_sepconv_describe(32, 91, 161, 256, 256, 1, 2, buf, 512) == 0 and b"tensor-pipe" not in buf.value
-    monkeypatch.setenv("PN_SEP_TC", "1")
-    for shp, want in (((64, 33, 33, 512, 512, 1, 1), b"bands 1 x 33 cols pitch 34"), ((64, 129, 129, 128, 128, 1, 1), b"A ring x4"),
-                      ((32, 91, 161, 256, 256, 1, 2), b"tensor-pipe"), ((512, 17, 17, 384, 384, 1, 1), b"A cache x6")):
+    for shp, want in (((64, 33, 33, 256, 256, 1, 1), b"bands 1 x 33 cols pitch 34"), ((32, 91, 161, 256, 256, 1, 2), b"kblocks 4"),
+                      ((2, 5, 3, 256, 256, 1, 2), b"tensor-pipe")):
         assert lib.pn_sepconv_describe(*shp, buf, 512) == 0, lib.pn_last_error_string()
         assert b"tensor-pipe depthwise" in buf.value and want in buf.value, buf.value
-    for shp in ((64, 65, 65, 256, 512, 2, 1), (64, 257, 257, 32, 64, 1, 1), (2, 33, 33, 1024, 1024, 1, 2), (3, 65, 65, 96, 96, 1, 1)):
-        assert lib.pn_sepconv_describe(*shp, buf, 512) == 0 and b"tensor-pipe" not in buf.value     # stride 2, narrow, wide, ragged
+    for shp in ((64, 33, 33, 512, 512, 1, 1), (64, 129, 129, 128, 128, 1, 1), (512, 17, 17, 384, 384, 1, 1), (64, 65, 65, 256, 512, 2, 1),
+                (64, 65, 65, 256, 256, 2, 1), (2, 33, 33, 256, 256, 1, 4), (64, 257, 257, 32, 64, 1, 1), (2, 33, 33, 1024, 1024, 1, 2),
+                (3, 65, 65, 96, 96, 1, 1)):
+        assert lib.pn_sepconv_describe(*shp, buf, 512) == 0 and b"tensor-pipe" not in buf.value, shp    # other widths, stride 2, dilation 4
 
 
-def test_measured_tile_table_and_team_policy(monkeypatch):
+def test_measured_tile_table_and_forced_teams(monkeypatch):
     """csrc/sep_tuned.inc: every row is a configuration the geometry code accepts as written (tile, ring depths, teams), it is
-    what the described block gets, PN_SEP_TUNED=0 falls back to the cost model, and forced teams need rings deep enough."""
+    what the described block gets, and forced teams need rings deep enough."""
     import ctypes as C
     import re
     lib, buf = nat.load(), C.create_string_buffer(512)
-    for k in ("PN_SEP_TUNED", "PN_SEP_TILE", "PN_SEP_STAGES", "PN_SEP_TEAMS", "PN_SEP_TC", "PN_SEP_WRES", "PN_SEP_DWWRES"):
+    for k in ("PN_SEP_TILE", "PN_SEP_STAGES", "PN_SEP_TEAMS"):
         monkeypatch.delenv(k, raising=False)
     inc = os.path.join(os.path.dirname(nat.__file__), "..", "csrc", "sep_tuned.inc")
     rows = [tuple(int(v) for v in m.group(1).split(",")) for m in re.finditer(r"^\s*\{([\d, ]+)\}", open(inc).read(), re.M)]
     assert len(rows) >= 5
     pat = re.compile(r"tile (\d+)x(\d+) subs (\d+) .* teams (\d+) stages p(\d+) w(\d+)r? a(\d+) stg(\d+)")
-    # (two of the table's blocks -- 32 -> 64 and 48 -> 96 stride 2 -- run on the warp-autonomous kernel by default; their rows are what
-    # the CTA pipeline uses when that path is switched off)
-    monkeypatch.setenv("PN_SEPWARP_S2", "0")
-    monkeypatch.setenv("PN_SEPWARP_FULL", "0")
     for (k, nc, s, d, ho, wo, th, tw, subs, p, w, a, stg, teams) in rows:
         h, wd = (ho - 1) * s + 1, (wo - 1) * s + 1                   # an input size that gives this output size (pad = dilation for stride 1)
         assert lib.pn_sepconv_describe(4, h, wd, k, nc, s, d, buf, 512) == 0, lib.pn_last_error_string()
         got = tuple(int(v) for v in pat.search(buf.value.decode()).groups())
         assert got == (th, tw, subs, teams, p, w, a, stg), (buf.value, (k, nc, s, d, ho, wo))
-    monkeypatch.delenv("PN_SEPWARP_S2")
-    monkeypatch.delenv("PN_SEPWARP_FULL")
-    k, nc, s, d, ho, wo, th, tw, subs = rows[0][:9]
-    monkeypatch.setenv("PN_SEP_TUNED", "0")
-    assert lib.pn_sepconv_describe(4, (ho - 1) * s + 1, (wo - 1) * s + 1, k, nc, s, d, buf, 512) == 0 and b"tile" in buf.value
-    monkeypatch.delenv("PN_SEP_TUNED")
-    # three teams of 4 + 3 + 3 warps only where three items fit the rings (p >= 3 subs, a >= 3, p >= a); otherwise the request is ignored
-    monkeypatch.setenv("PN_SEP_TEAMS", "3")
-    assert lib.pn_sepconv_describe(64, 129, 129, 128, 128, 1, 1, buf, 512) == 0 and b"teams 3" in buf.value
-    assert lib.pn_sepconv_describe(64, 257, 257, 64, 128, 2, 1, buf, 512) == 0 and b"teams 1" in buf.value      # p2 a2
-    # resident pointwise weights: one stage per (k-block, column block), marked "r"; PN_SEP_WRES=0 brings the ring back
+    # forced teams: one team of ten warps always; two teams of five only where two items fit the rings (p >= 2 subs, a >= 2, p >= a),
+    # otherwise the request is ignored
+    assert lib.pn_sepconv_describe(64, 129, 129, 128, 128, 1, 1, buf, 512) == 0 and b"teams 2" in buf.value
+    assert lib.pn_sepconv_describe(64, 257, 257, 64, 128, 2, 1, buf, 512) == 0 and b"teams 1" in buf.value
+    monkeypatch.setenv("PN_SEP_TEAMS", "1")
+    assert lib.pn_sepconv_describe(64, 129, 129, 128, 128, 1, 1, buf, 512) == 0 and b"teams 1" in buf.value
+    monkeypatch.setenv("PN_SEP_TEAMS", "2")
+    assert lib.pn_sepconv_describe(64, 257, 257, 64, 128, 2, 1, buf, 512) == 0 and b"teams 2" in buf.value      # p2 a2
+    assert lib.pn_sepconv_describe(64, 65, 65, 128, 256, 2, 1, buf, 512) == 0 and b"teams 1" in buf.value        # p4 with 3 subs
+    # resident pointwise weights: one stage per (k-block, column block), marked "r"
     monkeypatch.delenv("PN_SEP_TEAMS")
     assert lib.pn_sepconv_describe(64, 129, 129, 128, 128, 1, 1, buf, 512) == 0 and b" w2r " in buf.value
     assert lib.pn_sepconv_describe(64, 33, 33, 512, 512, 1, 1, buf, 512) == 0 and b"r a" not in buf.value      # 512 KB of W: ring
-    monkeypatch.setenv("PN_SEP_WRES", "0")
-    assert lib.pn_sepconv_describe(64, 129, 129, 128, 128, 1, 1, buf, 512) == 0 and b"r a" not in buf.value
 
 
-def test_warp_autonomous_block_policy(monkeypatch):
+def test_warp_autonomous_block_routing():
     """csrc/sepwarp.cu: which fused blocks run warp-autonomous -- cin <= 32 / cout <= 64 at stride 1 (quarter-warp layout up to cin
-    16), stride 2 for cin 17..32, the full-warp layout for 48 -> 96 stride 2 -- with their switches, and the output geometry of the
-    stride-2 strips."""
+    16), stride 2 for cin 17..32, the full-warp layout for 48 -> 96 stride 2 -- and the output geometry of the stride-2 strips."""
     import ctypes as C
     lib, buf = nat.load(), C.create_string_buffer(512)
-    for k in ("PN_NO_SEPWARP", "PN_SEPWARP_S2", "PN_SEPWARP_FULL", "PN_SWP_ITEMS"):
-        monkeypatch.delenv(k, raising=False)
+
     def desc(*shape):
         assert lib.pn_sepconv_describe(*shape, buf, 512) == 0, lib.pn_last_error_string()
         return buf.value.decode()
     assert desc(32, 721, 1281, 16, 32, 1, 1).startswith("warp-autonomous strips 161 x")            # 1281 / 8
     # row blocks: the count that minimises the largest per-warp sum of input rows under the round-robin item assignment (148 SMs x 16
-    # warps); PN_SWP_ITEMS=6 is the rule it replaced
+    # warps)
     assert "strips 33 x 10 row blocks of 26 rows" in desc(64, 257, 257, 32, 64, 1, 1)
     assert "strips 17 x 4 row blocks of 33 rows" in desc(512, 129, 129, 24, 48, 1, 1)
     assert "strips 41 x 7 row blocks of 26 rows" in desc(32, 361, 641, 32, 64, 2, 1)
-    monkeypatch.setenv("PN_SWP_ITEMS", "6")
-    assert "strips 33 x 7 row blocks of 37 rows" in desc(64, 257, 257, 32, 64, 1, 1)
-    monkeypatch.delenv("PN_SWP_ITEMS")
     d = desc(32, 721, 1281, 32, 64, 2, 1)
     assert d.startswith("warp-autonomous stride 2 strips 81 x") and "k16 slices 2, n8 tiles 8" in d   # output 361 x 641: 641 / 8
     d = desc(512, 129, 129, 48, 96, 2, 1)
@@ -147,23 +132,15 @@ def test_warp_autonomous_block_policy(monkeypatch):
     assert desc(32, 181, 321, 64, 64, 1, 1).startswith("tile ")                                       # measured slower there: CTA pipeline
     assert desc(32, 721, 1281, 16, 32, 2, 1).startswith("tile ")                                      # stride 2 needs cin > 16
     assert desc(64, 257, 257, 64, 128, 2, 1).startswith("tile ")
-    monkeypatch.setenv("PN_SEPWARP_S2", "0")
-    assert desc(32, 721, 1281, 32, 64, 2, 1).startswith("tile ")
-    monkeypatch.setenv("PN_SEPWARP_FULL", "0")
-    assert desc(512, 129, 129, 48, 96, 2, 1).startswith("tile ")
-    monkeypatch.setenv("PN_NO_SEPWARP", "1")
-    assert desc(64, 257, 257, 32, 64, 1, 1).startswith("half tile ") or desc(64, 257, 257, 32, 64, 1, 1).startswith("tile ")
 
 
-def test_warp_autonomous_row_blocks_minimise_the_busiest_warp(monkeypatch):
+def test_warp_autonomous_row_blocks_minimise_the_busiest_warp():
     """sepwarp_geometry picks the row-block count whose round-robin item assignment leaves the busiest warp the least input rows:
     a Python model of the same simulation (items strips-fastest over 148 x 16 warps, cost = input rows of the block) agrees with the
     library on random shapes of the three layouts, and the rows cover the map exactly."""
     import ctypes as C
     import re
     lib, buf = nat.load(), C.create_string_buffer(512)
-    for k in ("PN_NO_SEPWARP", "PN_SEPWARP_S2", "PN_SEPWARP_FULL", "PN_SWP_ITEMS"):
-        monkeypatch.delenv(k, raising=False)
     warps = 148 * 16
 
     def model(n, ho, strips, s):

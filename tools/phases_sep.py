@@ -31,7 +31,7 @@ def run(n, h, w, cin, cout, stride, dil):
     t = buf.cpu().numpy()[:16 * 8].reshape(16, 8)
     desc = C.create_string_buffer(512)
     lib.pn_sepconv_describe(n, h, w, cin, cout, stride, dil, desc, 512)
-    print("== %s exp=%s: %s" % ((n, h, w, cin, cout, stride, dil), os.environ.get("PN_SEP_EXP", "-"), desc.value.decode()))
+    print("== %s: %s" % ((n, h, w, cin, cout, stride, dil), desc.value.decode()))
     rows = [r for r in t if r.sum() > 0]
     tot = sum(float(r.sum()) for r in rows) / len(rows)
     print("   %d depthwise warps of block 0, %.0f cycles each (kernel %.1f us incl. launch)" % (len(rows), tot, e0.elapsed_time(e1) * 1e3))

@@ -1,5 +1,5 @@
 """Device time of one pointwise GEMM shape (pn_pwconv_gemm, bf16), median over launches inside one CUDA graph.
-usage: python tools/time_gemm.py m,k,n [...]   (PN_GEMM_PAIR=0/1 selects the single-CTA / CTA-pair kernel)"""
+usage: python tools/time_gemm.py m,k,n [...]"""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [os.path.join(ROOT, "posenet-pytorch_b200"), os.path.join(ROOT, "tests"), ROOT]
@@ -41,8 +41,7 @@ def run(m, k, n, reps=20):
         ts.append(e0.elapsed_time(e1) * 1e3 / reps)
     ts.sort()
     t = ts[len(ts) // 2]
-    print("%s pair=%s: median %.1f us  %.0f TFLOP/s  rel err (first 512 rows) %.2e" % ((m, k, n), os.environ.get("PN_GEMM_PAIR", "auto"), t,
-                                                                                      2.0 * m * k * n / t / 1e6, err), flush=True)
+    print("%s: median %.1f us  %.0f TFLOP/s  rel err (first 512 rows) %.2e" % ((m, k, n), t, 2.0 * m * k * n / t / 1e6, err), flush=True)
 
 
 if __name__ == "__main__":

@@ -47,8 +47,7 @@ def run(n, h, w, cin, cout, stride, dil, reps=20):
     ts.sort()
     desc = C.create_string_buffer(512)
     lib.pn_sepconv_describe(n, h, w, cin, cout, stride, dil, desc, 512)
-    print("%s exp=%s: median %.1f us  min %.1f us | %s" % ((n, h, w, cin, cout, stride, dil), os.environ.get("PN_SEP_EXP", "-"), ts[len(ts) // 2], ts[0],
-                                                          desc.value.decode()), flush=True)
+    print("%s: median %.1f us  min %.1f us | %s" % ((n, h, w, cin, cout, stride, dil), ts[len(ts) // 2], ts[0], desc.value.decode()), flush=True)
 
 
 if __name__ == "__main__":

@@ -8,11 +8,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [os.path.join(ROOT, "posenet-pytorch_b200"), os.path.join(ROOT, "tests"), ROOT]
 import torch
 
-os.environ.setdefault("PN_SEP_TC", "1")          # the path under test is opt-in
 import abi
 from posenet import _native as nat
 
-shape = tuple(int(v) for v in (sys.argv[1].split(",") if len(sys.argv) > 1 else "64,33,33,512,512,1,1".split(",")))
+shape = tuple(int(v) for v in (sys.argv[1].split(",") if len(sys.argv) > 1 else "64,33,33,256,256,1,1".split(",")))
 n, h, w, cin, cout, stride, dil = shape
 lo, hi = (int(sys.argv[2]), int(sys.argv[3])) if len(sys.argv) > 3 else (16, 28)
 g = torch.Generator().manual_seed(1)

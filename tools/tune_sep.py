@@ -71,7 +71,7 @@ def make_timer(shape):
 
 
 def ab(shape, envs):
-    """Times explicit configurations: envs = "PN_SEP_TEAMS=3,PN_SEP_STAGES=4.2.4.1;..." ('.' stands for ',' inside a value)."""
+    """Times explicit configurations: envs = "PN_SEP_TEAMS=2,PN_SEP_STAGES=4.2.4.1;..." ('.' stands for ',' inside a value)."""
     describe, timeit = make_timer(shape)
     for spec in [""] + envs.split(";"):
         env = dict(kv.split("=") for kv in spec.split(",") if kv)
