@@ -305,6 +305,18 @@ typedef enum pn_yuv_layout {
 int pn_yuv_to_bgr(const uint8_t *src, int n_img, int h, int w, int64_t src_stride, int layout, uint8_t *dst, int64_t dst_stride,
                   pn_stream_t stream);
 
+/* ---- N8: the inverse, for video sinks (ffmpeg rawvideo, GStreamer appsrc, v4l2loopback, hardware encoders take YUV): a batch
+ * of BGR frames converted to YUV ON THE DEVICE, bit-exact with cv2.cvtColor(frame, cv2.COLOR_BGR2YUV_<layout>), for the five
+ * layouts cv2 writes: PN_YUV_I420 (COLOR_BGR2YUV_I420 / _IYUV), PN_YUV_YV12, PN_YUV_YUY2 (_YUY2 / _YUYV / _YUNV), PN_YUV_UYVY
+ * (_UYVY / _Y422 / _UYNV) and PN_YUV_YVYU.  NV12 / NV21 (cv2 writes neither) give PN_ERR_ARG.  4:2:0 takes its chroma from the
+ * top-left pixel of each 2x2 block, 4:2:2 from the average of each horizontal pair, as cv2 does.
+ *
+ * Frame i is read from src + i * src_stride (dense [h, w, 3] BGR, src_stride >= h * w * 3) and written at dst + i * dst_stride
+ * in cv2's output layout (dst_stride >= h * w * 3 / 2 or h * w * 2).  Sizes follow cv2: w even, h even for 4:2:0.  Any strides;
+ * nothing outside the frames is read or written.  The launch geometry depends only on the arguments (graph-capturable). */
+int pn_bgr_to_yuv(const uint8_t *src, int n_img, int h, int w, int64_t src_stride, int layout, uint8_t *dst, int64_t dst_stride,
+                  pn_stream_t stream);
+
 /* ---- Whole-network plan: mobilenet_v1.py:130-162 (MobileNetV1.__init__/forward) --------------------
  * The layer table is computed by the caller (posenet/models/mobilenet_v1.py mirrors
  * _to_output_strided_layers, mobilenet_v1.py:8-39) and passed in explicitly. */

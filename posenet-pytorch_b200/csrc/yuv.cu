@@ -182,3 +182,144 @@ extern "C" int pn_yuv_to_bgr(const uint8_t *src, int n_img, int h, int w, int64_
     PN_CHECK_LAUNCH();
     return PN_OK;
 }
+
+namespace pn {
+
+namespace {
+
+// N8: the inverse, BGR -> YUV (cv2.cvtColor(frame, COLOR_BGR2YUV_<layout>)) of the five layouts cv2 writes.  The same tile
+// (ROW_PAIRS row pairs x TILE_W pixels), the same staging: the BGR rows come in as aligned 16-byte loads, thread t converts
+// pixels 2t, 2t + 1 of every row into shared copies of the output rows, and those go out as 16-byte stores.
+constexpr int BGR_SLOT = 3 * TILE_W + 32;
+constexpr int OUT_SEGS = ROWS + 2 * ROW_PAIRS;  // r0 of every row, r1 and r2 of every row pair (4:2:0 only)
+
+template <int L>
+__global__ void __launch_bounds__(YUV_THREADS, 12) bgr_to_yuv_kernel(YuvArgs a) {
+    __shared__ __align__(16) uint8_t s_in[ROWS][BGR_SLOT];
+    __shared__ __align__(16) uint8_t s_r0[ROWS][R0_SLOT];
+    __shared__ __align__(16) uint8_t s_c[2][ROW_PAIRS][C_SLOT];
+    __shared__ int s_lead[OUT_SEGS + ROWS];     // the output segments' leads, then the BGR rows'
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int x0 = blockIdx.x * TILE_W, y0 = blockIdx.y * ROWS;
+    const int npix = min(TILE_W, a.w - x0);
+    const uint8_t *frame = a.src + blockIdx.z * a.src_stride;
+    uint8_t *out = a.dst + blockIdx.z * a.dst_stride;
+
+    // segment k of the output: r0 of row k (k < ROWS), else r1 / r2 of row pair (k - ROWS) % ROW_PAIRS
+    auto out_seg = [&](int k) {
+        Seg s;
+        const int which = k < ROWS ? 0 : 1 + (k - ROWS) / ROW_PAIRS;
+        const int row = k < ROWS ? k : 2 * ((k - ROWS) % ROW_PAIRS);
+        s.n = 0;
+        s.g = out;
+        s.slot = k < ROWS ? s_r0[k] : s_c[which - 1][(k - ROWS) % ROW_PAIRS];
+        if (y0 + row < a.h) {
+            const uint8_t *r0, *r1, *r2;
+            yuv::frame_rows(L, out, a.h, a.w, y0 + row, &r0, &r1, &r2);
+            s.g = const_cast<uint8_t *>(which == 0 ? r0 : which == 1 ? r1 : r2) + yuv::row_bytes(L, which, x0);
+            s.n = yuv::row_bytes(L, which, npix);
+        }
+        s.lead = s.n > 0 ? (int)(reinterpret_cast<uintptr_t>(s.g) & 15) : 0;
+        return s;
+    };
+    if (threadIdx.x < OUT_SEGS) s_lead[threadIdx.x] = out_seg(threadIdx.x).lead;
+
+    // ---- stage the BGR rows, two per warp: every lane issues all its 16-byte loads before it stores any
+    constexpr int IN_PER_WARP = ROWS / WARPS;
+    Seg segs[IN_PER_WARP];
+    uint4 v[IN_PER_WARP][2];
+#pragma unroll
+    for (int j = 0; j < IN_PER_WARP; ++j) {
+        const int row = warp + WARPS * j;
+        Seg &s = segs[j];
+        s.slot = s_in[row];
+        s.n = y0 + row < a.h ? 3 * npix : 0;
+        s.g = const_cast<uint8_t *>(frame) + ((long long)(y0 + row) * a.w + x0) * 3;
+        s.lead = s.n > 0 ? (int)(reinterpret_cast<uintptr_t>(s.g) & 15) : 0;
+        if (lane == 0) s_lead[OUT_SEGS + row] = s.lead;
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {
+            const int off = 16 * (lane + 32 * q) - s.lead;
+            if (off >= 0 && off + 16 <= s.n) v[j][q] = __ldg(reinterpret_cast<const uint4 *>(s.g + off));
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < IN_PER_WARP; ++j) {
+        const Seg &s = segs[j];
+        const int nb = seg_blocks(s);
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {
+            const int blk = lane + 32 * q, off = 16 * blk - s.lead;
+            if (blk >= nb) continue;
+            if (off >= 0 && off + 16 <= s.n) {
+                *reinterpret_cast<uint4 *>(s.slot + 16 * blk) = v[j][q];
+            } else {
+                for (int b = 0; b < 16; ++b)
+                    if (off + b >= 0 && off + b < s.n) s.slot[16 * blk + b] = s.g[off + b];
+            }
+        }
+    }
+
+    __syncthreads();
+
+    // ---- convert: thread t owns pixels 2t, 2t + 1 of every row of the tile; every row is at its global address mod 16 in its
+    // slot, the input ones as staged, the output ones as they are written back
+    const int xl = 2 * threadIdx.x;
+    if (xl < npix) {
+#pragma unroll
+        for (int row = 0; row < ROWS; ++row) {
+            if (y0 + row >= a.h) break;
+            const int p = row >> 1;
+            yuv::put_pair(L, s_in[row] + s_lead[OUT_SEGS + row], xl, (row & 1) == 0, s_r0[row] + s_lead[row],
+                          s_c[0][p] + s_lead[ROWS + p], s_c[1][p] + s_lead[ROWS + ROW_PAIRS + p]);
+        }
+    }
+    __syncthreads();
+
+    // ---- write the output segments back, OUT_SEGS / WARPS per warp
+#pragma unroll 1
+    for (int j = 0; j < OUT_SEGS / WARPS; ++j) {
+        const Seg s = out_seg(warp + WARPS * j);
+        const int nb = seg_blocks(s);
+        for (int blk = lane; blk < nb; blk += 32) {
+            const int off = 16 * blk - s.lead;
+            if (off >= 0 && off + 16 <= s.n) {
+                *reinterpret_cast<uint4 *>(s.g + off) = *reinterpret_cast<const uint4 *>(s.slot + 16 * blk);
+            } else {
+                for (int b = 0; b < 16; ++b)
+                    if (off + b >= 0 && off + b < s.n) s.g[off + b] = s.slot[16 * blk + b];
+            }
+        }
+    }
+}
+
+}  // namespace
+
+}  // namespace pn
+
+extern "C" int pn_bgr_to_yuv(const uint8_t *src, int n_img, int h, int w, int64_t src_stride, int layout, uint8_t *dst,
+                             int64_t dst_stride, pn_stream_t stream) {
+    PN_CHECK_ARG(src && dst, "pn_bgr_to_yuv: null pointer");
+    PN_CHECK_ARG(n_img > 0 && n_img <= 65535, "pn_bgr_to_yuv: n_img %d out of 1..65535", n_img);
+    PN_CHECK_ARG(layout == PN_YUV_I420 || layout == PN_YUV_YV12 || layout == PN_YUV_YUY2 || layout == PN_YUV_UYVY ||
+                     layout == PN_YUV_YVYU,
+                 "pn_bgr_to_yuv: layout %d: cv2 writes I420, YV12, YUY2, UYVY and YVYU", layout);
+    PN_CHECK_ARG(h > 0 && w > 0 && w % 2 == 0 && (h % 2 == 0 || !yuv::is_420(layout)) && h <= (1 << 18) && w <= (1 << 18),
+                 "pn_bgr_to_yuv: frame size %d x %d: the width must be even, and the height too for 4:2:0", h, w);
+    PN_CHECK_ARG(src_stride >= 3ll * h * w, "pn_bgr_to_yuv: src_stride %lld < h*w*3", (long long)src_stride);
+    PN_CHECK_ARG(dst_stride >= yuv::frame_bytes(layout, h, w), "pn_bgr_to_yuv: dst_stride %lld < the frame's %lld bytes",
+                 (long long)dst_stride, (long long)yuv::frame_bytes(layout, h, w));
+    YuvArgs a;
+    a.src = src; a.dst = dst; a.src_stride = src_stride; a.dst_stride = dst_stride; a.h = h; a.w = w;
+    const dim3 grid(ceil_div(w, TILE_W), ceil_div(h, ROWS), n_img);
+    const cudaStream_t st = as_stream(stream);
+    switch (layout) {
+    case PN_YUV_I420: bgr_to_yuv_kernel<PN_YUV_I420><<<grid, YUV_THREADS, 0, st>>>(a); break;
+    case PN_YUV_YV12: bgr_to_yuv_kernel<PN_YUV_YV12><<<grid, YUV_THREADS, 0, st>>>(a); break;
+    case PN_YUV_YUY2: bgr_to_yuv_kernel<PN_YUV_YUY2><<<grid, YUV_THREADS, 0, st>>>(a); break;
+    case PN_YUV_UYVY: bgr_to_yuv_kernel<PN_YUV_UYVY><<<grid, YUV_THREADS, 0, st>>>(a); break;
+    default:          bgr_to_yuv_kernel<PN_YUV_YVYU><<<grid, YUV_THREADS, 0, st>>>(a); break;
+    }
+    PN_CHECK_LAUNCH();
+    return PN_OK;
+}

@@ -10,7 +10,7 @@ This is the batched form of what the reference's ``benchmark.py:32-44`` does per
         ...
 
 Options on top of that (``overlay=`` draws the poses on the frames, ``encode=`` returns them as JPEG files, or as PNG files
-with ``encode_ext=".png"``, ``jpeg=True`` takes JPEG files in, ``yuv=code`` video frames in YUV): ``source_coords=True`` maps the keypoint coordinates back to the submitted frames ON THE DEVICE
+with ``encode_ext=".png"``, ``jpeg=True`` takes JPEG files in, ``yuv=code`` video frames in YUV, ``yuv_out=code`` returns the drawn frames in YUV): ``source_coords=True`` maps the keypoint coordinates back to the submitted frames ON THE DEVICE
 (``image_demo.py:50``), ``mixed=True`` accepts frames of different sizes in one batch (every file of a directory
 pre-processed at its own size, ``benchmark.py:24-29``), ``gather=True`` all-gathers the records of every rank's shard over
 NCCL inside the step (one process per GPU, ``posenet.sharding``).
@@ -28,7 +28,7 @@ from posenet.decode_multi import decode_multiple_poses_batch, split_pose_records
 class BatchPipeline:
     def __init__(self, model, batch, height, width, depth=2, use_graph=True, output_stride=None, scale_factor=1.0,
                  source_coords=False, mixed=False, gather=False, group=None, overlay=None, jpeg=False, encode=None, encode_ext=".jpg",
-                 reduce=1, arena_bytes=None, yuv=None, **decode_kw):
+                 reduce=1, arena_bytes=None, yuv=None, yuv_out=None, **decode_kw):
         """``height`` x ``width``: size of the uint8 frames handed to ``submit`` (``mixed=True``: the LARGEST frame; each
         frame of a batch then comes with its own size).  The network runs at ``valid_resolution(width * scale_factor,
         height * scale_factor)`` (utils.py:7-10); frames of any other size go through the bit-exact cv2 resize
@@ -66,7 +66,15 @@ class BatchPipeline:
         instead of the frames: one per submitted frame in mixed mode, ``batch`` otherwise.  Params the device encoder does not
         do raise ValueError here.
         ``encode_ext``: ``".jpg"`` (the default) or ``".png"``: the files are then PNG (``pn_png_encode``, bit-exact with
-        ``cv2.imencode(".png", frame)``; ``encode`` must be ``[]``)."""
+        ``cv2.imencode(".png", frame)``; ``encode`` must be ``[]``).
+        ``yuv_out``: a ``cv2.COLOR_BGR2YUV_*`` code of a layout cv2 writes (I420 / IYUV, YV12, YUY2 / YUYV / YUNV, UYVY / Y422 /
+        UYNV, YVYU; needs ``overlay``), for handing the drawn frames to a video sink.  The step's graph converts the drawn frames
+        right after drawing them (``pn_bgr_to_yuv``, bit-exact with ``cv2.cvtColor(frame, yuv_out)``), and the in-graph
+        device-to-host copy carries only those 1.5 or 2 bytes a pixel.  ``result`` returns them as the fifth item instead of the
+        BGR frames: uint8 ``[batch, h*3/2, w]`` (4:2:0) or ``[batch, h, w, 2]`` (4:2:2), cv2's layout.  ``height`` x ``width`` must
+        be sizes cv2 converts (even width; even height for 4:2:0).  Works with ``yuv``, ``jpeg``, ``reduce``, ``source_coords`` and
+        ``gather`` (the frames stay on their rank); not with ``encode`` (one output form per pipeline) or ``mixed`` (frames of
+        their own, possibly odd, sizes).  ValueError otherwise."""
         self.yuv = None
         if yuv is not None:
             from posenet import yuv as yuv_mod
@@ -74,6 +82,15 @@ class BatchPipeline:
             if jpeg or mixed:
                 raise ValueError("yuv= takes video frames of one size: not with jpeg=True or mixed=True")
             self.yuv_bytes = int(np.prod(yuv_mod.frame_shape(self.yuv, int(height), int(width))))
+        self.yuv_out = None
+        if yuv_out is not None:
+            from posenet import yuv as yuv_mod
+            self.yuv_out = yuv_mod.layout_of_output(yuv_out)
+            if overlay is None:
+                raise ValueError("yuv_out= converts the drawn frames: it needs overlay=")
+            if encode is not None or mixed:
+                raise ValueError("yuv_out= returns frames of one size as YUV: not with encode= or mixed=True")
+            self.yuv_out_shape = yuv_mod.frame_shape(self.yuv_out, int(height), int(width))
         nat.require_device()
         assert depth >= 1
         self.model, self.batch, self.h, self.w = model, int(batch), int(height), int(width)
@@ -112,6 +129,7 @@ class BatchPipeline:
             self.h2d, self.d2h, self.compute = torch.cuda.Stream(dev), torch.cuda.Stream(dev), torch.cuda.Stream(dev)
             self.collect_all = self.gather and self.rank == 0      # this rank's D2H copy carries every rank's records
             self.nrec = self.batch * self.P * (1 + 5 * NUM_KEYPOINTS)
+            self.frame_shape = (self.h, self.w, 3) if self.yuv_out is None else self.yuv_out_shape     # of a returned frame
             nrec = self.nrec
             self.slots = []
             self._ws = {}
@@ -123,8 +141,10 @@ class BatchPipeline:
                          rec_host=torch.zeros((self.world if self.collect_all else 1) * nrec, dtype=torch.float64).pin_memory(),
                          scales=torch.ones((self.batch, 2), dtype=torch.float64, device=dev) if self.mixed else None,
                          scales_host=torch.ones((self.batch, 2), dtype=torch.float64).pin_memory() if self.mixed else None,
-                         frames_host=torch.empty((self.batch, self.h, self.w, 3), dtype=torch.uint8).pin_memory()
+                         frames_host=torch.empty((self.batch,) + self.frame_shape, dtype=torch.uint8).pin_memory()
                          if self.overlay and self.encode is None else None,
+                         yuv_out=torch.empty((self.batch,) + self.yuv_out_shape, dtype=torch.uint8, device=dev)
+                         if self.yuv_out is not None else None,
                          hw=torch.zeros((self.batch, 2), dtype=torch.int32, device=dev) if self.overlay and self.mixed else None,
                          hw_host=torch.zeros((self.batch, 2), dtype=torch.int32).pin_memory() if self.overlay and self.mixed else None,
                          yuv=torch.empty(self.batch * self.yuv_bytes, dtype=torch.uint8, device=dev) if self.yuv is not None else None,
@@ -157,7 +177,7 @@ class BatchPipeline:
             self.h2d_bytes_per_batch = self.slots[0]["x"].numel() if self.yuv is None else self.slots[0]["yuv"].numel()
             self.d2h_bytes_per_batch = (self.world if self.collect_all else 1) * nrec * 8
             if self.overlay and self.encode is None:
-                self.d2h_bytes_per_batch += self.slots[0]["x"].numel()         # mixed mode copies only the bytes in use
+                self.d2h_bytes_per_batch += self.slots[0]["frames_host"].numel()   # mixed mode copies only the bytes in use
             elif self.encode is not None:
                 # the offsets, plus the files: an estimate (file_share of the frames' raw size); result() copies exactly the
                 # bytes in use and records them in last_file_bytes
@@ -185,7 +205,7 @@ class BatchPipeline:
 
     def _enqueue(self, s):
         """The captured part of a step: (YUV -> BGR ->) (uniform resize ->) stem .. heads -> candidates -> greedy decode
-        (-> coordinate scaling) (-> overlay on the submitted frames)."""
+        (-> coordinate scaling) (-> overlay on the submitted frames (-> JPEG / PNG files | -> BGR -> YUV)))."""
         x = s["x"]
         lib = nat.load()
         if self.yuv is not None:
@@ -212,6 +232,9 @@ class BatchPipeline:
                       "pn_draw_poses")
             if self.encode is not None:
                 s["enc"].encode(x, self.h * self.w * 3, s["hw"] if self.mixed else None)
+            if self.yuv_out is not None:
+                from posenet.yuv import convert_out
+                convert_out(x, self.batch, self.h, self.w, self.yuv_out, s["yuv_out"])
 
     def _resize_mixed(self, s, shapes):
         """Per-frame cv2-exact resize of frames stored at their own size (row i of the slot's input buffer holds frame i
@@ -337,7 +360,7 @@ class BatchPipeline:
                     s["frames_host"].view(self.batch, -1)[:len(shapes), :used].copy_(s["x"].view(self.batch, -1)[:len(shapes), :used],
                                                                                    non_blocking=True)
                 elif self.overlay and not self.mixed:
-                    s["frames_host"].copy_(s["x"], non_blocking=True)
+                    s["frames_host"].copy_(s["x"] if self.yuv_out is None else s["yuv_out"], non_blocking=True)
                 if enc is not None:
                     s["status_host"].copy_(s["dec"].status, non_blocking=True)
                 s["out"].record(self.d2h)
@@ -349,7 +372,7 @@ class BatchPipeline:
     def result(self, ticket, copy=True, source_coords=None, gathered=False):
         """Block until the ticket's records are on the host; returns the reference's 4-tuple for this rank's batch
         (numpy float64: [batch,P], [batch,P,17], [batch,P,17,2], [batch,P,17,2]).  With ``overlay``, a fifth item holds this
-        rank's drawn frames: uint8 [batch,h,w,3], or in mixed mode a list of [h_i,w_i,3] arrays, one per submitted frame (with
+        rank's drawn frames: uint8 [batch,h,w,3] (with ``yuv_out``, in its YUV layout), or in mixed mode a list of [h_i,w_i,3] arrays, one per submitted frame (with
         ``encode``: their JPEG or PNG files, a list of ``bytes``).  With
         ``jpeg``, the last item is the int32 decode status [batch].  ``gathered=True`` (rank 0 of a
         ``gather=True`` pipeline): the records of ALL ranks' batches instead, leading dimension ``world * batch`` (rank-major).
