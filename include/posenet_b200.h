@@ -222,6 +222,39 @@ int pn_jpeg_parse(const uint8_t *file_host, int64_t nbytes, pn_jpeg_desc *desc_h
  * entries are in TIFF order, of known types, with their data inside the segment, and all such entries agree.  Other files with an
  * orientation other than 1 stay PN_JPEG_HOST as with pn_jpeg_parse. */
 int pn_jpeg_parse_oriented(const uint8_t *file_host, int64_t nbytes, pn_jpeg_desc *desc_host);
+
+/* Progressive files (SOF2, Huffman-coded, jdphuff.c), decoded ON THE DEVICE when the caller opts in with
+ * pn_jpeg_parse_progressive.  Such a descriptor is kind PN_JPEG_SUPPORTED_PROGRESSIVE: its geometry is that of one interleaved scan
+ * of all components (one component: the plane's own block grid), restart_interval covers the whole image, n_segments is 1 and
+ * huff[] is unused.  Its scans are described by a scan table the caller stores in the byte arena at file_offset +
+ * align8(file_bytes), 8-byte aligned: a pn_jpeg_scans header, then n_scans pn_jpeg_scan, then n_huff pn_jpeg_huff.
+ * A scan's wave is the length of the longest chain of earlier scans it depends on (same component, overlapping coefficients):
+ * the scans of one wave touch disjoint coefficients and are decoded in parallel, waves in order. */
+enum { PN_JPEG_SUPPORTED_PROGRESSIVE = 2 };
+#define PN_JPEG_MAX_SCANS 64      /* scans of a progressive file; more: PN_JPEG_HOST */
+#define PN_JPEG_MAX_SCAN_HUFF 32  /* derived Huffman tables its scans use (a DHT redefining a slot counts again); more: PN_JPEG_HOST */
+typedef struct pn_jpeg_scan {
+    int64_t start, end;        /* entropy-coded bytes [start, end) from the start of the file, RST markers included */
+    int32_t restart_interval;  /* MCUs per restart interval in this scan (blocks in a one-component scan), 0 for none */
+    int32_t wave;
+    uint8_t ncomp, ss, se, ah, al;
+    uint8_t comp[3];           /* frame component indices, in scan order */
+    uint8_t dc[3], ac[3];      /* indices into the table's pn_jpeg_huff[]: DC tables of a first DC scan, the AC table of an AC scan */
+    uint8_t pad[2];
+} pn_jpeg_scan;
+typedef struct pn_jpeg_scans {
+    int32_t n_scans, n_huff, n_waves, pad;
+} pn_jpeg_scans;
+/* Baseline files come back exactly as pn_jpeg_parse (oriented = 0) or pn_jpeg_parse_oriented (oriented != 0) return them, with
+ * *scans_bytes = 0.  A progressive file is PN_JPEG_SUPPORTED_PROGRESSIVE with its scan table in scans_host (*scans_bytes bytes)
+ * when libjpeg-turbo decodes it without a warning and without block smoothing: a complete scan script (every coefficient of every
+ * component refined to Al = 0), a legal progression (Ah equal to the coefficient's previous Al, Al <= 13, DC scans with Se = 0,
+ * AC scans with one component and 1 <= Ss <= Se <= 63, no AC scan before the component's DC), at most PN_JPEG_MAX_SCANS scans and
+ * PN_JPEG_MAX_SCAN_HUFF tables, and everything the baseline parser asks of a file's other headers.  Other progressive files are
+ * PN_JPEG_HOST (PN_JPEG_WHY_PROGRESSIVE), as are files whose table needs more than scans_cap bytes (*scans_bytes is then what it
+ * needs).  Host only. */
+int pn_jpeg_parse_progressive(const uint8_t *file_host, int64_t nbytes, int oriented, pn_jpeg_desc *desc_host, void *scans_host,
+                              int64_t scans_cap, int64_t *scans_bytes);
 /* Device workspace (bytes, 256-byte aligned base) pn_jpeg_decode needs for up to n_img files of together at most arena_bytes
  * bytes, none larger than max_h x max_w. */
 int pn_jpeg_workspace(int n_img, int64_t arena_bytes, int max_h, int max_w, size_t *bytes_host);

@@ -1,6 +1,6 @@
 // pn_jpeg_decode: baseline JPEG files -> uint8 BGR frames on the device, bit-exact with cv2.imdecode (arithmetic: jpeg_decode.cuh).
 //
-// One call decodes a batch in ten launches whose geometry depends only on the arguments (so the call can be captured in a graph):
+// One call decodes a batch in eleven launches whose geometry depends only on the arguments (so the call can be captured in a graph):
 //   plan      validate every descriptor (a warp per image) and size its share of the workspace
 //   layout    exclusive prefix sums of the shares (one CTA)
 //   destuff   one CTA per image: drop 0xFF00 stuffing, find the restart markers and the end of the scan, cut every restart
@@ -13,6 +13,9 @@
 //   walk      one warp per segment chases the merge points from subsequence 0, whose start is exact: the true path is path 0
 //             up to m[0], then path m[0], ...  Every chain element gets its true exit state and block count
 //   write     every subsequence decodes from its true entry and stores the blocks that begin in it (DC as a difference)
+//   progressive  one warp per progressive image (pn_jpeg_parse_progressive's kind 2): its waves in order, the lanes decoding the
+//             (scan, restart segment) pairs of a wave serially from the raw file bytes into the zeroed coefficient array
+//             (jpeg_progressive.cuh).  The stages from destuff to write and dc have nothing to do for such an image
 //   dc        one warp per segment: per-component prefix sums of the DC differences (reset at every restart marker)
 //   idct      eight threads per block, into per-component sample planes: jpeg_idct_islow, or at 1/2, 1/4, 1/8 (scale_denom,
 //             cv2's IMREAD_REDUCED_COLOR_*) the component's scaled IDCT (jidctred.c), ssize x ssize samples per block
@@ -24,6 +27,7 @@
 // (Weissenberger & Schmidt, "Massively Parallel Huffman Decoding on GPUs", ICPP 2018, for the self-synchronisation.)
 #include "common.cuh"
 #include "jpeg_decode.cuh"
+#include "jpeg_progressive.cuh"
 
 namespace pn {
 namespace {
@@ -126,11 +130,61 @@ __device__ __forceinline__ BitSrc seg_src(const Ws &ws, const pn_jpeg_desc &d, c
     return BitSrc{ws.ds + d.file_offset + sg.start, sg.end - sg.start};
 }
 
+// A progressive descriptor's scan table (the warp of plan_kernel; the descriptor's own fields are checked there): inside the arena
+// and 8-byte aligned, every scan a legal one over the frame's components with its bytes inside the file and its tables in the
+// table, DC tables with symbols <= 15, and no two scans of one wave on a shared (component, coefficient) -- nor a scan in a wave
+// at or before one it depends on.
+__device__ bool scan_table_ok(const Args &a, const pn_jpeg_desc &d, int lane) {
+    const int64_t t = scan_table_offset(d);
+    const bool head_ok = d.file_offset >= 0 && d.file_bytes > 0 && t + (int64_t)sizeof(pn_jpeg_scans) <= a.arena &&
+                         ((uintptr_t)(a.files + t) & 7) == 0;
+    if (!__all_sync(0xffffffffu, head_ok)) return false;
+    const uint8_t *tab = a.files + t;
+    const pn_jpeg_scans h = *reinterpret_cast<const pn_jpeg_scans *>(tab);
+    if (h.n_scans < 1 || h.n_scans > PN_JPEG_MAX_SCANS || h.n_huff < 0 || h.n_huff > PN_JPEG_MAX_SCAN_HUFF || h.n_waves < 1 ||
+        h.n_waves > h.n_scans || t + scan_table_bytes(h.n_scans, h.n_huff) > a.arena)
+        return false;
+    const pn_jpeg_scan *sc = table_scans(tab);
+    const pn_jpeg_huff *huff = table_huff(tab);
+    bool ok = true;
+    for (int s = lane; s < h.n_scans; s += 32) {
+        const pn_jpeg_scan S = sc[s];
+        const bool dc = S.ss == 0;
+        bool g = S.ncomp >= 1 && S.ncomp <= d.ncomp && S.se <= 63 && S.ss <= S.se && (dc ? S.se == 0 : S.ncomp == 1) &&
+                 S.al <= 13 && S.ah <= 13 && S.wave >= 0 && S.wave < h.n_waves && S.restart_interval >= 0 && S.start >= 0 &&
+                 S.start <= S.end && S.end <= d.file_bytes;
+        int blocks = 0;
+        for (int i = 0; g && i < S.ncomp; ++i) {
+            const int c = S.comp[i];
+            g = c < d.ncomp;
+            for (int j = 0; g && j < i; ++j) g = S.comp[j] != c;
+            if (!g) break;
+            blocks += d.comp[c].h * d.comp[c].v;
+            if (dc && S.ah == 0) {
+                g = S.dc[i] < h.n_huff;
+                for (int e = 0; g && e < 256; ++e) g = (huff[S.dc[i]].lookup[e] & 0xFF) <= 15 && huff[S.dc[i]].huffval[e] <= 15;
+            }
+            if (!dc) g = g && S.ac[i] < h.n_huff;
+        }
+        g = g && blocks <= PN_JPEG_MAX_BLOCKS;
+        for (int u = 0; g && u < s; ++u) {
+            const pn_jpeg_scan &T = sc[u];
+            bool shared = false;
+            for (int x = 0; x < T.ncomp && x < 3; ++x)
+                for (int y = 0; y < S.ncomp; ++y) shared = shared || T.comp[x] == S.comp[y];
+            g = !(shared && T.ss <= S.se && S.ss <= T.se) || T.wave < S.wave;
+        }
+        ok = ok && g;
+    }
+    return __all_sync(0xffffffffu, ok);
+}
+
 // ---- plan: one warp per image validates its descriptor and sizes its share of the workspace ----------------------------------
 __global__ void __launch_bounds__(32) plan_kernel(Args a, Ws ws) {
     const int lane = threadIdx.x, i = blockIdx.x;
         const pn_jpeg_desc &d = a.descs[i];
-        bool ok = d.kind == PN_JPEG_SUPPORTED;
+        const bool prog = d.kind == PN_JPEG_SUPPORTED_PROGRESSIVE;
+        bool ok = d.kind == PN_JPEG_SUPPORTED || prog;
         const bool skipped = !ok;
         const long long rh = ((long long)d.height + a.denom - 1) / a.denom, rw = ((long long)d.width + a.denom - 1) / a.denom;
         const bool tr = orient_transposes(d.orientation);          // the oriented frame is rw x rh
@@ -164,17 +218,18 @@ __global__ void __launch_bounds__(32) plan_kernel(Args a, Ws ws) {
         }
         // DC symbols are extra-bit counts: at most 15 (what jpeg_make_d_derived_tbl enforces)
         bool tables_ok = true;
-        for (int c = 0; ok && c < d.ncomp; ++c) {
+        for (int c = 0; ok && !prog && c < d.ncomp; ++c) {
             const pn_jpeg_huff &t = d.huff[d.comp[c].dc];
             for (int e = lane; e < 256; e += 32) tables_ok &= (t.lookup[e] & 0xFF) <= 15 && t.huffval[e] <= 15;
         }
+        if (prog) ok = ok && canonical_mcu(d) && scan_table_ok(a, d, lane);
         ok = ok && __all_sync(0xffffffffu, tables_ok);
         if (lane == 0) {
             ImgWs &w = ws.img[i];
             w.status = skipped ? PN_JPEG_SKIPPED : ok ? PN_JPEG_OK : PN_JPEG_ERR_DESC;
             w.ds_len = 0;
-            w.nseg = ok ? d.n_segments : 0;
-            w.sub_cap = ok ? (int)(d.n_segments + d.file_bytes * 8 / SUB_BITS) : 0;
+            w.nseg = ok && !prog ? d.n_segments : 0;
+            w.sub_cap = ok && !prog ? (int)(d.n_segments + d.file_bytes * 8 / SUB_BITS) : 0;
             w.nsub = 0;
             w.nblk = ok ? mcus * d.blocks_per_mcu : 0;
             long long pb = 0;                  // plane offsets within the image's share; layout_kernel adds its base
@@ -257,7 +312,7 @@ constexpr int DS_PER_THREAD = 8;
 __global__ void __launch_bounds__(THREADS, 1) destuff_kernel(Args a, Ws ws) {
     const int i = blockIdx.x;
     ImgWs &w = ws.img[i];
-    if (w.status != PN_JPEG_OK) return;
+    if (w.status != PN_JPEG_OK || a.descs[i].kind != PN_JPEG_SUPPORTED) return;
     const pn_jpeg_desc &d = a.descs[i];
     const uint8_t *f = a.files + d.file_offset;
     const long long n = d.file_bytes, p0 = d.scan_offset;
@@ -550,6 +605,80 @@ __global__ void __launch_bounds__(THREADS) write_kernel(Args a, Ws ws) {
     }
 }
 
+// ---- progressive: one warp per image, the (scan, restart segment) pairs of each wave across the lanes ------------------------------
+// The warp walks the scans of a wave in table order and cuts them at their RST markers (searched 32 bytes at a time), 32 segments
+// per round; each lane then decodes its segment serially.  Waves are separated by __syncwarp, since a wave's scans refine the
+// coefficients of the earlier ones.
+__device__ int64_t warp_next_restart(const uint8_t *f, int64_t p, int64_t end, int lane) {
+    for (int64_t b = p; b + 1 < end; b += 32) {
+        const int64_t q = b + lane;
+        const unsigned hit = __ballot_sync(0xffffffffu, q + 1 < end && f[q] == 0xFF && (f[q + 1] & 0xF8) == 0xD0);
+        if (hit) return b + __ffs(hit) - 1;
+    }
+    return end;
+}
+
+__global__ void __launch_bounds__(32) progressive_kernel(Args a, Ws ws) {
+    const int i = blockIdx.x, lane = threadIdx.x;
+    const pn_jpeg_desc &d = a.descs[i];
+    ImgWs &w = ws.img[i];
+    if (d.kind != PN_JPEG_SUPPORTED_PROGRESSIVE || w.status != PN_JPEG_OK) return;
+    const uint8_t *file = a.files + d.file_offset, *tab = a.files + scan_table_offset(d);
+    const pn_jpeg_scans h = *reinterpret_cast<const pn_jpeg_scans *>(tab);
+    const pn_jpeg_scan *sc = table_scans(tab);
+    const pn_jpeg_huff *huff = table_huff(tab);
+    int16_t *coef = ws.coef + w.blk_base * 64;
+    for (long long j = lane; j < w.nblk * 8; j += 32) reinterpret_cast<uint4 *>(coef)[j] = make_uint4(0, 0, 0, 0);
+    __syncwarp();
+    int status = PN_JPEG_OK;
+    for (int wave = 0; wave < h.n_waves && status == PN_JPEG_OK; ++wave) {
+        int s = 0;
+        while (s < h.n_scans && sc[s].wave != wave) ++s;
+        int64_t p = s < h.n_scans ? sc[s].start : 0, k = 0;
+        while (s < h.n_scans && status == PN_JPEG_OK) {
+            int mine = -1;                     // this lane's pair: scan, segment, bytes
+            int64_t my_k = 0, my_p = 0, my_e = 0;
+            for (int n = 0; n < 32 && s < h.n_scans; ++n) {
+                const pn_jpeg_scan &S = sc[s];
+                const bool more = k + 1 < scan_segments(d, S);
+                int64_t e = S.end;
+                if (more) {
+                    e = warp_next_restart(file, p, S.end, lane);
+                    if (e == S.end || file[e + 1] != 0xD0 + (k & 7)) {
+                        status = PN_JPEG_ERR_RESTART;
+                        break;
+                    }
+                }
+                if (lane == n) {
+                    mine = s;
+                    my_k = k;
+                    my_p = p;
+                    my_e = e;
+                }
+                if (more) {
+                    p = e + 2;
+                    ++k;
+                } else {
+                    do ++s; while (s < h.n_scans && sc[s].wave != wave);
+                    p = s < h.n_scans ? sc[s].start : 0;
+                    k = 0;
+                }
+            }
+            int st = PN_JPEG_OK;
+            if (status == PN_JPEG_OK && mine >= 0) {
+                const pn_jpeg_scan &S = sc[mine];
+                const int64_t units = scan_units(d, S), ri = S.restart_interval > 0 ? S.restart_interval : units;
+                const int64_t u0 = my_k * ri;
+                st = decode_scan_segment(d, S, huff, file, my_p, my_e, u0, units - u0 < ri ? units - u0 : ri, coef);
+            }
+            st = __reduce_min_sync(0xffffffffu, st);
+            if (status == PN_JPEG_OK) status = st;
+            __syncwarp();
+        }
+    }
+    if (lane == 0 && status != PN_JPEG_OK) w.status = status;
+}
+
 // ---- DC: per-component running sums, one warp per segment ----------------------------------------------------------------------
 __global__ void __launch_bounds__(THREADS) dc_kernel(Args a, Ws ws) {
     const int lane = threadIdx.x & 31;
@@ -791,6 +920,8 @@ extern "C" int pn_jpeg_decode_scaled(const uint8_t *files, int64_t arena_bytes, 
     walk_kernel<<<grid, THREADS, 0, st>>>(a, w);
     PN_CHECK_LAUNCH();
     write_kernel<<<grid, THREADS, 0, st>>>(a, w);
+    PN_CHECK_LAUNCH();
+    progressive_kernel<<<n_img, 32, 0, st>>>(a, w);
     PN_CHECK_LAUNCH();
     dc_kernel<<<grid, THREADS, 0, st>>>(a, w);
     PN_CHECK_LAUNCH();

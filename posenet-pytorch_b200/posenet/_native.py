@@ -17,7 +17,8 @@ NUM_PARTS, NUM_EDGES, HEAD_CHANNELS, HEAD_ROWS = 17, 16, 115, 128
 ABI_VERSION = 5
 PLAN_UNFUSED = 1
 DRAW_KEYPOINTS, DRAW_SKELETON = 1, 2
-JPEG_SUPPORTED, JPEG_HOST = 0, 1
+JPEG_SUPPORTED, JPEG_HOST, JPEG_SUPPORTED_PROGRESSIVE = 0, 1, 2
+JPEG_MAX_SCANS, JPEG_MAX_SCAN_HUFF = 64, 32
 JPEG_WHY = {name: i for i, name in enumerate((
     "none", "not_jpeg", "truncated", "progressive", "arithmetic", "lossless", "precision", "multi_scan", "components", "rgb",
     "no_dht", "exif_orientation", "sampling", "bad_table", "unknown"))}
@@ -69,6 +70,21 @@ class JpegDesc(C.Structure):
                 ("quant", (C.c_int16 * 64) * 3), ("huff", JpegHuff * 4)]
 
 
+class JpegScan(C.Structure):
+    """pn_jpeg_scan: one scan of a progressive file (pn_jpeg_parse_progressive's scan table)."""
+    _fields_ = [("start", C.c_int64), ("end", C.c_int64), ("restart_interval", C.c_int32), ("wave", C.c_int32)] + \
+               [(n, C.c_uint8) for n in ("ncomp", "ss", "se", "ah", "al")] + \
+               [("comp", C.c_uint8 * 3), ("dc", C.c_uint8 * 3), ("ac", C.c_uint8 * 3), ("pad", C.c_uint8 * 2)]
+
+
+class JpegScans(C.Structure):
+    """pn_jpeg_scans: the head of a scan table, followed by n_scans JpegScan and n_huff JpegHuff."""
+    _fields_ = [(n, C.c_int32) for n in ("n_scans", "n_huff", "n_waves", "pad")]
+
+
+JPEG_SCAN_TABLE_MAX = C.sizeof(JpegScans) + JPEG_MAX_SCANS * C.sizeof(JpegScan) + JPEG_MAX_SCAN_HUFF * C.sizeof(JpegHuff)
+
+
 _SIGNATURES = {
     "pn_abi_version": (C.c_int, []),
     "pn_last_error_string": (C.c_char_p, []),
@@ -102,6 +118,8 @@ _SIGNATURES = {
                                 C.c_int, C.c_double, C.c_double, C.c_int, C.c_void_p]),
     "pn_jpeg_parse": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(JpegDesc)]),
     "pn_jpeg_parse_oriented": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(JpegDesc)]),
+    "pn_jpeg_parse_progressive": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.POINTER(JpegDesc), C.c_void_p, C.c_int64,
+                                            C.POINTER(C.c_int64)]),
     "pn_jpeg_workspace": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
     "pn_jpeg_decode": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int64, C.c_void_p,
                                  C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),

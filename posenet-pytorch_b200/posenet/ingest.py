@@ -36,6 +36,10 @@ cv2.imread rotates them; a directory of portraits and landscapes has both frame 
     stream = posenet.ImageStream(paths, batch=64, height=1008, width=1008, mixed=True, decode="gpu", reduce=4, orientation="gpu")
     pipe = posenet.BatchPipeline(model, 64, 1008, 1008, jpeg=True, mixed=True, reduce=4, arena_bytes=stream.arena_bytes,
                                  source_coords=True)
+
+Progressive files (web images, CDN output) decoded on the GPU too; the pipeline is the same:
+
+    stream = posenet.ImageStream(paths, batch=64, decode="gpu", progressive="gpu")
 """
 import concurrent.futures
 import ctypes as C
@@ -47,7 +51,7 @@ import numpy as np
 import torch
 
 from posenet import _native as nat
-from posenet.jpeg import frame_size, imread_flag, parser
+from posenet.jpeg import align8, check_progressive, frame_size, imread_flag, parse_progressive, parser
 
 
 class EncodedBatch:
@@ -76,7 +80,7 @@ class EncodedBatch:
 
 class ImageStream:
     def __init__(self, paths, batch, height=None, width=None, workers=None, slots=4, keep=2, pinned=None, mixed=False, decode="cv2",
-                 reduce=1, arena_bytes=None, orientation="cv2"):
+                 reduce=1, arena_bytes=None, orientation="cv2", progressive="cv2"):
         """``mixed``: the files may have different sizes (each at most ``height`` x ``width``); a batch row then holds its frame
         contiguously at the frame's own size and ``batches()`` also yields the list of ``(h, w)`` -- the input format of a
         ``BatchPipeline(..., mixed=True)``, which resizes every frame on the GPU like ``_process_input`` (utils.py:13-26) does.
@@ -94,6 +98,10 @@ class ImageStream:
         ``orientation="gpu"`` (with ``decode="gpu"`` only): files whose EXIF orientation is certain are decoded on the GPU and
         rotated there as cv2.imread rotates them (``pn_jpeg_parse_oriented``); shapes and size checks use the rotated size, so
         portraits and landscapes need ``mixed=True`` as with ``decode="cv2"``.
+        ``progressive="gpu"`` (with ``decode="gpu"`` only): progressive files the GPU decodes (``pn_jpeg_parse_progressive``) go
+        to the arena too, each file 8-byte aligned and followed by its scan table.  A worker reads and parses a file in buffers
+        of its own and then takes exactly the space the file and its table need; a file and its table that do not fit the
+        arena's remaining space are decoded by cv2.
 
         ``reduce`` (1, 2, 4 or 8): every file is decoded at 1 / reduce, as ``cv2.imread(path, cv2.IMREAD_REDUCED_COLOR_<reduce>)``
         does (JPEG files: ceil(h / reduce) x ceil(w / reduce), scaled in the DCT domain).  ``height`` / ``width`` are then the
@@ -131,6 +139,11 @@ class ImageStream:
         if orientation == "gpu" and decode != "gpu":
             raise ValueError("orientation='gpu' rotates files in the GPU decode: it needs decode='gpu'")
         self.orientation = orientation
+        check_progressive(progressive)
+        if progressive == "gpu" and decode != "gpu":
+            raise ValueError("progressive='gpu' decodes progressive files on the GPU: it needs decode='gpu'")
+        self.progressive = progressive
+        self._scratch = threading.local()        # progressive="gpu": each worker's file and scan-table buffers
         if arena_bytes is None:
             r = self.reduce
             arena_bytes = self._bufs[0].numel() if r == 1 else self.batch * (r * self.height) * (r * self.width)
@@ -162,6 +175,8 @@ class ImageStream:
 
     def _load_encoded(self, path, enc, row):
         """Read one file into the arena and parse it; cv2 decodes it into its raw row when the GPU cannot."""
+        if self.progressive == "gpu":
+            return self._load_progressive(path, enc, row)
         try:
             with open(path, "rb") as f:
                 size = os.fstat(f.fileno()).st_size
@@ -178,13 +193,54 @@ class ImageStream:
             d = nat.JpegDesc()
             nat.check(parser(self.orientation)(view.ctypes.data, size, C.byref(d)), "pn_jpeg_parse")
             if d.kind == nat.JPEG_SUPPORTED:
-                h, w = frame_size(d, self.reduce)
-                self._check_size(path, h, w)
-                d.file_offset = off
-                k = C.sizeof(nat.JpegDesc)
-                enc.descs.numpy()[row * k:(row + 1) * k] = np.frombuffer(bytes(d), np.uint8)
-                enc.shapes[row] = (h, w)
+                self._place(path, enc, row, d, off)
                 return
+        self._load_host(path, enc, row)
+
+    def _load_progressive(self, path, enc, row):
+        """progressive="gpu": read and parse one file in this worker's scratch buffers, then take exactly the arena space it
+        needs (8-byte aligned: the file, then its scan table at file_offset + align8(size)) and copy it there."""
+        sc = self._scratch
+        if not hasattr(sc, "table"):
+            sc.table = np.zeros(nat.JPEG_SCAN_TABLE_MAX, np.uint8)
+            sc.buf = np.zeros(0, np.uint8)
+        try:
+            with open(path, "rb") as f:
+                size = os.fstat(f.fileno()).st_size
+                if sc.buf.size < size:
+                    sc.buf = np.zeros(max(size, 2 * sc.buf.size), np.uint8)
+                view = sc.buf[:size]
+                n = f.readinto(memoryview(view))
+        except OSError:
+            raise IOError("Image file not found or unreadable: %s" % path)
+        if n == size:
+            d, tb = parse_progressive(view, self.orientation, sc.table)
+            if d.kind in (nat.JPEG_SUPPORTED, nat.JPEG_SUPPORTED_PROGRESSIVE):
+                need = align8(size) + tb if d.kind == nat.JPEG_SUPPORTED_PROGRESSIVE else size
+                with enc.lock:
+                    off = align8(enc.used)
+                    fits = off + need <= enc.arena.numel()
+                    if fits:
+                        enc.used = off + need
+                if fits:
+                    arena = enc.arena.numpy()
+                    arena[off:off + size] = view
+                    if d.kind == nat.JPEG_SUPPORTED_PROGRESSIVE:
+                        arena[off + align8(size):off + need] = sc.table[:tb]
+                    self._place(path, enc, row, d, off)
+                    return
+        self._load_host(path, enc, row)
+
+    def _place(self, path, enc, row, d, off):
+        """Record the descriptor of a file the GPU decodes, stored at arena offset ``off``."""
+        h, w = frame_size(d, self.reduce)
+        self._check_size(path, h, w)
+        d.file_offset = off
+        k = C.sizeof(nat.JpegDesc)
+        enc.descs.numpy()[row * k:(row + 1) * k] = np.frombuffer(bytes(d), np.uint8)
+        enc.shapes[row] = (h, w)
+
+    def _load_host(self, path, enc, row):
         self._load(path, enc.raw.numpy()[row], enc.shapes, row)
         with enc.lock:
             enc.host_rows.append(row)

@@ -5,9 +5,10 @@ and, at 1/2, 1/4, 1/8, with ``cv2.IMREAD_REDUCED_COLOR_*`` (``pn_jpeg_decode_sca
     rows, status, shapes = posenet.imdecode_batch(buffers)            # sizes differ: row i holds frame i at its own size
     frames, status = posenet.imdecode_batch(buffers, reduce=4)        # at 1/4 (cv2.IMREAD_REDUCED_COLOR_4), ceil(h/4) x ceil(w/4)
     out = posenet.imdecode_batch(buffers, orientation="gpu")          # EXIF-rotated files (phone portraits) rotated on the GPU too
+    out = posenet.imdecode_batch(buffers, progressive="gpu")          # progressive files (web images) decoded on the GPU too
 
-``status[i]``: 0 decoded on the GPU, 1 decoded by cv2 on the host (progressive, arithmetic-coded, 12-bit, CMYK / RGB-coded or
-truncated files, EXIF-rotated ones unless ``orientation="gpu"``, anything the parser does not know) and uploaded, < 0 the file's
+``status[i]``: 0 decoded on the GPU, 1 decoded by cv2 on the host (progressive files unless ``progressive="gpu"``, arithmetic-coded,
+12-bit, CMYK / RGB-coded or truncated files, EXIF-rotated ones unless ``orientation="gpu"``, anything the parser does not know) and uploaded, < 0 the file's
 entropy-coded data is malformed: its frame is zeros (cv2 decodes such files with a warning; its recovery is not reproduced).
 
     files = posenet.imencode_batch(frames, [cv2.IMWRITE_JPEG_QUALITY, 90])   # list of bytes, one per frame"""
@@ -49,17 +50,48 @@ def parser(orientation):
     return lib.pn_jpeg_parse_oriented if orientation == "gpu" else lib.pn_jpeg_parse
 
 
+PROGRESSIVES = ("cv2", "gpu")
+
+
+def check_progressive(progressive):
+    """ValueError unless ``progressive`` is "cv2" (progressive files decoded on the host) or "gpu"."""
+    if progressive not in PROGRESSIVES:
+        raise ValueError("progressive=%r: 'cv2' (progressive files decoded on the host) or 'gpu'" % (progressive,))
+
+
+def align8(n):
+    return (int(n) + 7) & ~7
+
+
+def parse_progressive(view, orientation, table):
+    """pn_jpeg_parse_progressive of the uint8 array ``view`` with the scan table written into the uint8 array ``table`` (any
+    size): ``(desc, table_bytes)``.  A progressive file whose table does not fit ``table`` is JPEG_HOST."""
+    d, n = nat.JpegDesc(), C.c_int64()
+    nat.check(nat.load().pn_jpeg_parse_progressive(view.ctypes.data if view.size else C.c_void_p(1), view.size,
+                                                   int(orientation == "gpu"), C.byref(d),
+                                                   table.ctypes.data if table.size else None, table.size, C.byref(n)),
+              "pn_jpeg_parse_progressive")
+    return d, n.value
+
+
 def frame_size(desc, reduce):
     """The frame a SUPPORTED descriptor decodes to at 1 / reduce: the reduced size, transposed for EXIF orientations 5..8."""
     h, w = reduced_size(desc.height, desc.width, reduce)
     return (w, h) if 5 <= desc.orientation <= 8 else (h, w)
 
 
-def parse(buf, orientation="cv2"):
+def parse(buf, orientation="cv2", progressive="cv2"):
     """pn_jpeg_parse (``orientation="gpu"``: pn_jpeg_parse_oriented) on the bytes of one file: a ``_native.JpegDesc`` (``kind``
-    JPEG_SUPPORTED / JPEG_HOST, ``why``, ``orientation``)."""
+    JPEG_SUPPORTED / JPEG_HOST, ``why``, ``orientation``).  ``progressive="gpu"``: pn_jpeg_parse_progressive, which also accepts
+    the progressive files the GPU decodes (kind JPEG_SUPPORTED_PROGRESSIVE); returns ``(desc, table)`` with the file's scan
+    table as ``bytes`` (empty for other kinds), to be stored at ``file_offset + align8(file_bytes)``, 8-byte aligned."""
     fn = parser(orientation)
+    check_progressive(progressive)
     a = np.frombuffer(buf, np.uint8) if not isinstance(buf, np.ndarray) else np.ascontiguousarray(buf, np.uint8).reshape(-1)
+    if progressive == "gpu":
+        table = np.zeros(nat.JPEG_SCAN_TABLE_MAX, np.uint8)
+        d, n = parse_progressive(a, orientation, table)
+        return d, table[:n].tobytes() if d.kind == nat.JPEG_SUPPORTED_PROGRESSIVE else b""
     d = nat.JpegDesc()
     nat.check(fn(a.ctypes.data if a.size else C.c_void_p(1), a.size, C.byref(d)), "pn_jpeg_parse")
     return d
@@ -98,7 +130,7 @@ class Decoder:
             C.c_void_p(self.status.data_ptr()), nat.stream_ptr()), "pn_jpeg_decode_scaled")
 
 
-def imdecode_batch(buffers, device=None, reduce=1, orientation="cv2"):
+def imdecode_batch(buffers, device=None, reduce=1, orientation="cv2", progressive="cv2"):
     """Decode the JPEG files in ``buffers`` (bytes / uint8 arrays) on the GPU.  Returns ``(frames, status)`` when all frames
     share one size (frames: CUDA uint8 [N, h, w, 3]), else ``(rows, status, shapes)``: rows is CUDA uint8 [N, H * W * 3] (H x W
     the largest frame) with frame i stored contiguously from the start of row i, shapes the list of (h_i, w_i).  status: CUDA
@@ -110,20 +142,32 @@ def imdecode_batch(buffers, device=None, reduce=1, orientation="cv2"):
 
     ``orientation``: "cv2" (default) leaves files with an EXIF orientation other than 1 to cv2 on the host; "gpu" decodes those
     whose orientation is certain on the GPU, flipped / rotated as cv2 does (frame i is then the rotated frame, w x h for
-    orientations 5..8; the rest stay cv2's).  Anything else is a ValueError."""
+    orientations 5..8; the rest stay cv2's).  Anything else is a ValueError.
+
+    ``progressive``: "cv2" (default) leaves progressive files to cv2 on the host; "gpu" decodes on the GPU those with a complete
+    scan script that libjpeg decodes without a warning (``pn_jpeg_parse_progressive``), with status 0, at every ``reduce`` and
+    orientation.  Anything else is a ValueError."""
     flag = imread_flag(reduce)
     parser(orientation)
+    check_progressive(progressive)
     nat.require_device()
     bufs = [np.frombuffer(b, np.uint8) if not isinstance(b, np.ndarray) else np.ascontiguousarray(b, np.uint8).reshape(-1)
             for b in buffers]
     assert bufs, "no buffers"
-    descs, host_imgs, shapes = [], {}, []
+    descs, host_imgs, shapes, pieces = [], {}, [], []
     offset = 0
     for i, b in enumerate(bufs):
-        d = parse(b, orientation)
-        if d.kind == nat.JPEG_SUPPORTED:
+        d, table = parse(b, orientation, "gpu") if progressive == "gpu" else (parse(b, orientation), b"")
+        if d.kind in (nat.JPEG_SUPPORTED, nat.JPEG_SUPPORTED_PROGRESSIVE):
+            if progressive == "gpu":                  # files 8-byte aligned, each scan table at file_offset + align8(size)
+                offset = align8(offset)
             d.file_offset = offset
+            pieces.append((offset, b))
             offset += b.size
+            if table:
+                offset = align8(offset)
+                pieces.append((offset, np.frombuffer(table, np.uint8)))
+                offset += len(table)
             shapes.append(frame_size(d, reduce))
         else:
             img = cv2.imdecode(b, flag)
@@ -136,8 +180,10 @@ def imdecode_batch(buffers, device=None, reduce=1, orientation="cv2"):
     dec = Decoder(len(bufs), max(offset, 1), H, W, device, reduce)
     dev = dec.arena.device
     if offset:
-        arena = torch.from_numpy(np.concatenate([b for b, d in zip(bufs, descs) if d.kind == nat.JPEG_SUPPORTED]))
-        dec.arena[:offset].copy_(arena.pin_memory(), non_blocking=True)
+        arena = np.zeros(offset, np.uint8)
+        for at, piece in pieces:
+            arena[at:at + piece.size] = piece
+        dec.arena[:offset].copy_(torch.from_numpy(arena).pin_memory(), non_blocking=True)
     dec.descs.copy_(torch.from_numpy(desc_bytes(descs)).pin_memory(), non_blocking=True)
     rows = torch.empty((len(bufs), H * W * 3), dtype=torch.uint8, device=dev)
     for i, img in host_imgs.items():
