@@ -3,18 +3,19 @@
 (1) pn_dwtc_probe: the hardware behaviours the kernel relies on -- a SWIZZLE_128B UMMA descriptor advanced by whole 128-byte
     rows reads a shifted view of the TMA-written patch (depthwise taps; equal to numpy fp32 up to rare one-ulp flips of the bf16 rounding), and tcgen05.mma takes
     its A operand from TMEM (pointwise on the depthwise result).
-(2) pn_sepconv_block on those blocks against a torch fp32 reference of mobilenet_v1.py:57-68 (SeperableConv) with the
-    kernel's rounding points: bf16 input, bf16 depthwise weights, bf16 depthwise output, bf16 output."""
+(2) pn_sepconv_block on those blocks, every output cell against an fp64 reference of mobilenet_v1.py:57-68 (SeperableConv) with
+    the kernel's rounding points -- bf16 input, bf16 depthwise weights, bf16 depthwise output, bf16 output -- within the bound of
+    tests/sepref.py."""
 import ctypes as C
 
 import numpy as np
 import pytest
 import torch
-import torch.nn.functional as F
 
 pytestmark = pytest.mark.gpu
 
 import abi  # noqa: E402
+import sepref  # noqa: E402
 from posenet import _native as nat  # noqa: E402
 
 DEV = "cuda"
@@ -93,25 +94,16 @@ def test_sepconv_block_on_the_tensor_pipe(shape):
     buf = C.create_string_buffer(512)
     assert nat.load().pn_sepconv_describe(n, h, w, cin, cout, 1, dil, buf, 512) == 0
     assert b"tensor-pipe depthwise" in buf.value, buf.value
-    g = torch.Generator().manual_seed(h * 7 + cin + dil)
-    x = (torch.rand((n, h, w, cin), generator=g) * 6).to(torch.bfloat16)
-    wd = torch.randn((cin, 1, 3, 3), generator=g) * 0.35
-    bd = torch.randn(cin, generator=g) * 0.3
-    wp = (torch.randn((cout, cin), generator=g) * (1.5 / cin ** 0.5)).to(torch.bfloat16)
-    bp = torch.randn(cout, generator=g) * 0.5
-    t = F.relu6(F.conv2d(x.float().permute(0, 3, 1, 2), wd.to(torch.bfloat16).float(), bd, padding=dil, dilation=dil, groups=cin))
-    t = t.to(torch.bfloat16).float()
-    ref = F.relu6(F.conv2d(t, wp.float().reshape(cout, cin, 1, 1), bp)).permute(0, 2, 3, 1)
-    w9 = wd.reshape(cin, 9).t().contiguous().to(DEV)
+    x, w9, bd, wp, bp = sepref.make_case(n, h, w, cin, cout, seed=h * 7 + cin + dil)
+    # fp64 reference with bf16 depthwise weights; the depthwise sum accumulates on the tensor core (sepref.EPS_TC)
+    ref, bound = sepref.reference(x, w9, bd, wp, bp, 1, dil, dw_bf16=True, dw_eps=sepref.EPS_TC)
     y = torch.full((n, h, w, cout), float("nan"), dtype=torch.bfloat16, device=DEV)
-    xd, bdd, wpd, bpd = x.to(DEV), bd.to(DEV), wp.to(DEV), bp.to(DEV)
+    xd, w9, bdd, wpd, bpd = x.to(DEV), w9.to(DEV), bd.to(DEV), wp.to(DEV), bp.to(DEV)
     nat.check(nat.load().pn_sepconv_block(P(xd), P(w9), P(bdd), P(wpd), P(bpd), P(y), n, h, w, cin, cout, 1, dil, nat.stream_ptr()),
               "pn_sepconv_block")
     torch.cuda.synchronize()
-    yf = y.float().cpu()
-    assert not torch.isnan(yf).any(), "%d output cells never written" % int(torch.isnan(yf).sum())
-    err = float((yf - ref).abs().max() / ref.abs().max())
-    assert err < 6e-3, err                                   # one bf16 output rounding + rare 1-ulp flips of the intermediate
+    ratio = sepref.check(y, ref, bound, str(shape))
+    print("%s: max |err| / bound %.3f" % (shape, ratio))
     y2 = abi.sepconv(xd, w9, bdd, wpd, bpd, 1, dil)
     assert torch.equal(y, y2)                                # deterministic
 
