@@ -350,6 +350,31 @@ int pn_yuv_to_bgr(const uint8_t *src, int n_img, int h, int w, int64_t src_strid
 int pn_bgr_to_yuv(const uint8_t *src, int n_img, int h, int w, int64_t src_stride, int layout, uint8_t *dst, int64_t dst_stride,
                   pn_stream_t stream);
 
+/* ---- N9: pose tracking across video frames: the bounding-box tracker of TF.js pose-detection (BoundingBoxTracker), run ON
+ * THE DEVICE on the records pn_decode_greedy writes, so that pose k of frame t keeps its id in frame t + 1.
+ *
+ * A stream is a video source with an id in 0 .. n_streams-1; stream_ids (device int32 [n_img]) names the stream of each row, and
+ * a row whose id is outside 0 .. n_streams-1 is not tracked.  Each stream holds up to max_tracks tracks (id, box, the stream
+ * frame at which it was last matched), a frame counter and the count of ids it issued.  Rows are frames, taken in row order per
+ * stream.  A detection is a record with pose_score > 0; its box is the min / max of y and x over its keypoints with score >=
+ * min_part_score (none: an empty box).  Per frame: the stream's counter becomes t; tracks with t - last > max_age are dropped
+ * (stably); each detection in record order takes the unmatched track of largest IoU among those with IoU >= min_similarity (the
+ * first such track on a tie), which takes its box and last = t, or else gets a new track with the next id (1, 2, ... per
+ * stream); the tracks are then stably sorted by last, descending, and the first max_tracks kept.  IoU in float64 without FMA:
+ * inter = (min(ymax) - max(ymin)) * (min(xmax) - max(xmin)) when both factors are > 0 and neither box is empty, else 0;
+ * IoU = inter / (area_a + area_b - inter), 0 when that union is <= 0.
+ *
+ * pose_scores [n_img, P], keypoint_scores [n_img, P, 17], keypoint_coords [n_img, P, 17, 2] (y, x): float64, 8-byte aligned;
+ * P <= 256.  ids: device int64 [n_img, P]: the track id of each detection, -1 for records that are not detections and for
+ * untracked rows.  state: device, pn_track_state_bytes(n_streams, max_tracks) bytes, 8-byte aligned; ALL ZERO BYTES IS THE
+ * START of every stream (zero a stream's pn_track_state_bytes(1, max_tracks) bytes at state + s * that to reset it).  The
+ * state must be used with one (n_streams, max_tracks) only.  max_tracks <= 256, max_age >= 0.  One warp per stream: the
+ * launch geometry depends only on n_streams, so the call can be captured in a CUDA graph. */
+int pn_track_state_bytes(int n_streams, int max_tracks, size_t *bytes_host);
+int pn_track_poses(const double *pose_scores, const double *keypoint_scores, const double *keypoint_coords, int n_img, int P,
+                   const int *stream_ids, void *state, int n_streams, int max_tracks, int max_age, double min_similarity,
+                   double min_part_score, int64_t *ids, pn_stream_t stream);
+
 /* ---- Whole-network plan: mobilenet_v1.py:130-162 (MobileNetV1.__init__/forward) --------------------
  * The layer table is computed by the caller (posenet/models/mobilenet_v1.py mirrors
  * _to_output_strided_layers, mobilenet_v1.py:8-39) and passed in explicitly. */

@@ -24,6 +24,7 @@ JPEG_WHY = {name: i for i, name in enumerate((
     "no_dht", "exif_orientation", "sampling", "bad_table", "unknown"))}
 JPEG_OK, JPEG_SKIPPED = 0, 1
 YUV_I420, YUV_YV12, YUV_NV12, YUV_NV21, YUV_YUY2, YUV_UYVY, YUV_YVYU = range(7)
+TRACK_MAX_POSES, TRACK_MAX_TRACKS = 256, 256
 
 
 class NativeError(RuntimeError):
@@ -136,6 +137,9 @@ _SIGNATURES = {
                                 C.c_void_p, C.c_size_t, C.c_void_p]),
     "pn_yuv_to_bgr": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]),
     "pn_bgr_to_yuv": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_void_p, C.c_int64, C.c_void_p]),
+    "pn_track_state_bytes": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
+    "pn_track_poses": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                 C.c_int, C.c_double, C.c_double, C.c_void_p, C.c_void_p]),
     "pn_plan_query": (C.c_int, [C.POINTER(NetDesc), C.POINTER(C.c_size_t), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "pn_plan_create": (C.c_int, [C.POINTER(NetDesc), C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p)]),
     "pn_plan_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

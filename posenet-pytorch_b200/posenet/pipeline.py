@@ -10,7 +10,7 @@ This is the batched form of what the reference's ``benchmark.py:32-44`` does per
         ...
 
 Options on top of that (``overlay=`` draws the poses on the frames, ``encode=`` returns them as JPEG files, or as PNG files
-with ``encode_ext=".png"``, ``jpeg=True`` takes JPEG files in, ``yuv=code`` video frames in YUV, ``yuv_out=code`` returns the drawn frames in YUV): ``source_coords=True`` maps the keypoint coordinates back to the submitted frames ON THE DEVICE
+with ``encode_ext=".png"``, ``jpeg=True`` takes JPEG files in, ``yuv=code`` video frames in YUV, ``yuv_out=code`` returns the drawn frames in YUV, ``track=PoseTracker(...)`` gives the poses of video streams track ids): ``source_coords=True`` maps the keypoint coordinates back to the submitted frames ON THE DEVICE
 (``image_demo.py:50``), ``mixed=True`` accepts frames of different sizes in one batch (every file of a directory
 pre-processed at its own size, ``benchmark.py:24-29``), ``gather=True`` all-gathers the records of every rank's shard over
 NCCL inside the step (one process per GPU, ``posenet.sharding``).
@@ -28,7 +28,7 @@ from posenet.decode_multi import decode_multiple_poses_batch, split_pose_records
 class BatchPipeline:
     def __init__(self, model, batch, height, width, depth=2, use_graph=True, output_stride=None, scale_factor=1.0,
                  source_coords=False, mixed=False, gather=False, group=None, overlay=None, jpeg=False, encode=None, encode_ext=".jpg",
-                 reduce=1, arena_bytes=None, yuv=None, yuv_out=None, **decode_kw):
+                 reduce=1, arena_bytes=None, yuv=None, yuv_out=None, track=None, **decode_kw):
         """``height`` x ``width``: size of the uint8 frames handed to ``submit`` (``mixed=True``: the LARGEST frame; each
         frame of a batch then comes with its own size).  The network runs at ``valid_resolution(width * scale_factor,
         height * scale_factor)`` (utils.py:7-10); frames of any other size go through the bit-exact cv2 resize
@@ -74,7 +74,20 @@ class BatchPipeline:
         BGR frames: uint8 ``[batch, h*3/2, w]`` (4:2:0) or ``[batch, h, w, 2]`` (4:2:2), cv2's layout.  ``height`` x ``width`` must
         be sizes cv2 converts (even width; even height for 4:2:0).  Works with ``yuv``, ``jpeg``, ``reduce``, ``source_coords`` and
         ``gather`` (the frames stay on their rank); not with ``encode`` (one output form per pipeline) or ``mixed`` (frames of
-        their own, possibly odd, sizes).  ValueError otherwise."""
+        their own, possibly odd, sizes).  ValueError otherwise.
+        ``track``: a ``posenet.PoseTracker`` on the pipeline's device.  ``submit`` then takes ``streams=``, one stream id per
+        row (-1: not tracked), which travel in the host-to-device copy with the batch; the step's graph runs ``pn_track_poses``
+        on the records after the decode and after ``source_coords`` scaling (boxes in frame pixels then), before the overlay,
+        and the device-to-host stream copies the ids back after the records.  ``result`` appends them as the last item, int64
+        ``[batch, P]`` (after the decode status with ``jpeg``).  The tracker's ``min_part_score=None`` takes the decode's
+        ``score_threshold``.  Works with every option but ``gather`` (each rank would hold its own tracks): ValueError."""
+        self.track = track
+        if track is not None:
+            from posenet.track import PoseTracker
+            if not isinstance(track, PoseTracker):
+                raise ValueError("track= takes a posenet.PoseTracker")
+            if gather:
+                raise ValueError("track= keeps the tracks on this rank: not with gather=True")
         self.yuv = None
         if yuv is not None:
             from posenet import yuv as yuv_mod
@@ -119,6 +132,11 @@ class BatchPipeline:
         self.P = int(self.decode_kw.get("max_pose_detections", 10))
         dev = model._device()
         self.dev = dev
+        if track is not None:
+            if track.device != torch.device(dev):
+                raise ValueError("the tracker's state is on %s, the pipeline runs on %s" % (track.device, dev))
+            self.track_part_score = track.min_part_score if track.min_part_score is not None else \
+                float(self.decode_kw.get("score_threshold", 0.5))
         self.world, self.rank, self.group = 1, 0, group
         if gather:
             import torch.distributed as dist
@@ -149,6 +167,10 @@ class BatchPipeline:
                          hw_host=torch.zeros((self.batch, 2), dtype=torch.int32).pin_memory() if self.overlay and self.mixed else None,
                          yuv=torch.empty(self.batch * self.yuv_bytes, dtype=torch.uint8, device=dev) if self.yuv is not None else None,
                          shapes=None,
+                         streams=torch.full((self.batch,), -1, dtype=torch.int32, device=dev) if track is not None else None,
+                         streams_host=torch.full((self.batch,), -1, dtype=torch.int32).pin_memory() if track is not None else None,
+                         ids=torch.empty((self.batch, self.P), dtype=torch.int64, device=dev) if track is not None else None,
+                         ids_host=torch.empty((self.batch, self.P), dtype=torch.int64).pin_memory() if track is not None else None,
                          copied=torch.cuda.Event(), done=torch.cuda.Event(), out=torch.cuda.Event(), graph=None, busy=False)
                 self.slots.append(s)
             self.jpeg = bool(jpeg)
@@ -182,6 +204,10 @@ class BatchPipeline:
                 # the offsets, plus the files: an estimate (file_share of the frames' raw size); result() copies exactly the
                 # bytes in use and records them in last_file_bytes
                 self.d2h_bytes_per_batch += 8 * (self.batch + 1) + int(self.slots[0]["x"].numel() * self.file_share)
+            if track is not None:
+                self.h2d_bytes_per_batch += self.slots[0]["streams"].numel() * 4
+                self.d2h_bytes_per_batch += self.slots[0]["ids"].numel() * 8
+                track.stream = self.compute                          # reset() is ordered with the steps
             self.last_file_bytes = 0
             # warm up (plans, workspaces) and capture one graph per slot on the compute stream
             self.compute.wait_stream(torch.cuda.current_stream(dev))
@@ -205,7 +231,7 @@ class BatchPipeline:
 
     def _enqueue(self, s):
         """The captured part of a step: (YUV -> BGR ->) (uniform resize ->) stem .. heads -> candidates -> greedy decode
-        (-> coordinate scaling) (-> overlay on the submitted frames (-> JPEG / PNG files | -> BGR -> YUV)))."""
+        (-> coordinate scaling) (-> tracking) (-> overlay on the submitted frames (-> JPEG / PNG files | -> BGR -> YUV)))."""
         x = s["x"]
         lib = nat.load()
         if self.yuv is not None:
@@ -223,6 +249,8 @@ class BatchPipeline:
                                                    C.c_void_p(s["scales"].data_ptr()) if self.mixed else None,
                                                    float(self.scale[0]), float(self.scale[1]), nat.stream_ptr()),
                       "pn_scale_keypoint_coords")
+        if self.track is not None:                                   # the warm-up's stream ids are all -1: the state stays
+            self.track.launch(ps, ks, kc, s["streams"], s["ids"], self.track_part_score)
         if self.overlay:
             x = s["x"]
             nat.check(lib.pn_draw_poses(C.c_void_p(x.data_ptr()), self.batch, self.h, self.w, self.h * self.w * 3,
@@ -272,15 +300,25 @@ class BatchPipeline:
             x[enc.n_valid:].zero_()                                    # rows without a file decode as black frames
         s["h2d_bytes"] = n
 
-    def submit(self, host_batch, shapes=None):
+    def submit(self, host_batch, shapes=None, streams=None):
         """Enqueue one batch (uint8 [batch,h,w,3], ideally pinned; with ``yuv``, the frames in cv2's YUV layout).  Returns a
         ticket for ``result``; if the slot is still in flight its previous result must have been collected.
 
         ``mixed=True``: ``host_batch`` is uint8 ``[batch, h*w*3]`` (or ``[batch,h,w,3]``) whose row i starts with frame i
         stored contiguously at its own size ``shapes[i] = (h_i, w_i)`` (``h_i <= h``, ``w_i <= w``); rows without a frame
-        (``len(shapes) < batch``) decode as black frames."""
+        (``len(shapes) < batch``) decode as black frames.
+
+        ``streams`` (``track=`` pipelines, required there): the stream id of every row, ``batch`` integers in
+        -1..n_streams-1; ValueError otherwise."""
         s = self.slots[self._next]
         assert not s["busy"], "pipeline full: collect result() of the oldest ticket first"
+        if self.track is None:
+            if streams is not None:
+                raise ValueError("streams= are for track= pipelines")
+        else:
+            if streams is None:
+                raise ValueError("track=: pass streams=, the stream id of every row (-1: not tracked)")
+            s["streams_host"].numpy()[:] = self.track.stream_ids(streams, self.batch)
         enc = None
         if self.jpeg:
             from posenet.ingest import EncodedBatch
@@ -332,6 +370,8 @@ class BatchPipeline:
                     s["x"].copy_(host_batch.view(s["x"].shape), non_blocking=True)
                 if self.overlay and self.mixed:
                     s["hw"].copy_(s["hw_host"], non_blocking=True)
+                if self.track is not None:
+                    s["streams"].copy_(s["streams_host"], non_blocking=True)
                 s["copied"].record(self.h2d)
             with torch.cuda.stream(self.compute):
                 self.compute.wait_event(s["copied"])
@@ -363,6 +403,8 @@ class BatchPipeline:
                     s["frames_host"].copy_(s["x"] if self.yuv_out is None else s["yuv_out"], non_blocking=True)
                 if enc is not None:
                     s["status_host"].copy_(s["dec"].status, non_blocking=True)
+                if self.track is not None:
+                    s["ids_host"].copy_(s["ids"], non_blocking=True)
                 s["out"].record(self.d2h)
         s["busy"] = True
         ticket = self._next
@@ -374,7 +416,7 @@ class BatchPipeline:
         (numpy float64: [batch,P], [batch,P,17], [batch,P,17,2], [batch,P,17,2]).  With ``overlay``, a fifth item holds this
         rank's drawn frames: uint8 [batch,h,w,3] (with ``yuv_out``, in its YUV layout), or in mixed mode a list of [h_i,w_i,3] arrays, one per submitted frame (with
         ``encode``: their JPEG or PNG files, a list of ``bytes``).  With
-        ``jpeg``, the last item is the int32 decode status [batch].  ``gathered=True`` (rank 0 of a
+        ``jpeg``, the int32 decode status [batch] follows; with ``track``, the int64 track ids [batch, P] come last.  ``gathered=True`` (rank 0 of a
         ``gather=True`` pipeline): the records of ALL ranks' batches instead, leading dimension ``world * batch`` (rank-major).
         ``source_coords`` is a construction-time option (the scaling runs on the device); passing a different value here is an
         error."""
@@ -400,6 +442,8 @@ class BatchPipeline:
                 frames = (fr.copy() if copy else fr,)
         if self.jpeg:
             frames = frames + (s["status_host"].numpy().copy(),)
+        if self.track is not None:
+            frames = frames + (s["ids_host"].numpy().copy(),)
         if not gathered:
             own = flat[self.rank * self.nrec:(self.rank + 1) * self.nrec] if self.collect_all else flat
             return split_pose_records(own, self.batch, self.P) + frames
@@ -442,7 +486,8 @@ class BatchPipeline:
 
     def run(self, batches, copy=True, source_coords=None):
         """Generator: yields the pose records of every batch of ``batches`` in order, keeping ``depth`` batches in flight.
-        Items are uint8 batches, or ``(batch, shapes)`` pairs for a ``mixed=True`` pipeline."""
+        Items are uint8 batches, or ``(batch, shapes)`` pairs for a ``mixed=True`` pipeline, ``(batch, shapes, streams)`` for
+        a ``track=`` one (``shapes`` None unless mixed)."""
         pending = []
         for hb in batches:
             if len(pending) == len(self.slots):
