@@ -375,6 +375,33 @@ int pn_track_poses(const double *pose_scores, const double *keypoint_scores, con
                    const int *stream_ids, void *state, int n_streams, int max_tracks, int max_age, double min_similarity,
                    double min_part_score, int64_t *ids, pn_stream_t stream);
 
+/* ---- N10: One Euro smoothing of tracked keypoints (Casiez et al., CHI 2012, the filter TF.js pose-detection runs per tracked
+ * pose), ON THE DEVICE, on the ids pn_track_poses writes, so that a still person's keypoints stop jittering.
+ *
+ * Streams and rows as for pn_track_poses (stream_ids: device int32 [n_img]; a row whose id is outside 0 .. n_streams-1 is left
+ * as it is).  Each stream holds a frame counter, which advances on every row of the stream, and a table of up to max_tracks
+ * entries: a track id, the stream frame of its last update (last), and per coordinate the previous raw value, previous
+ * filtered value and previous filtered derivative (float64).  Per frame: the counter becomes t; entries with t - last > max_age
+ * are dropped (stably); each detection (record with id >= 1) in record order updates the entry of its id, or else appends a
+ * fresh entry, or else (table full) replaces the entry of smallest last < t (the first on a tie); when every entry was updated
+ * in this frame, or its id was already met in this frame, the record keeps its coordinates.  A fresh entry keeps x and stores
+ * x_prev = x_hat = x, dx_hat = 0.  An update, per coordinate, in float64 without FMA and in this order:
+ *   rate = fps / (t - last); dx = (x - x_prev) * rate; a_d = 1 / (1 + rate / (2 pi d_cutoff));
+ *   dx_hat = a_d dx + (1 - a_d) dx_hat; cutoff = min_cutoff + beta |dx_hat|; a = 1 / (1 + rate / (2 pi cutoff));
+ *   x_hat = a x + (1 - a) x_hat; x_prev = x; the output is x_hat.
+ * All 17 keypoints are filtered whatever their score; scores are never read.
+ *
+ * ids: device int64 [n_img, P] (pn_track_poses's output); keypoint_coords: device float64 [n_img, P, 17, 2] (y, x), smoothed
+ * IN PLACE; 8-byte aligned; P <= 256.  state: device, pn_smooth_state_bytes(n_streams, max_tracks) bytes, 8-byte aligned,
+ * contiguous per stream; ALL ZERO BYTES IS THE START of every stream (zero a stream's pn_smooth_state_bytes(1, max_tracks)
+ * bytes at state + s * that to reset it, together with its tracks).  The state must be used with one (n_streams, max_tracks)
+ * only.  max_tracks <= 256, max_age >= 0; fps, min_cutoff, d_cutoff finite and > 0, beta finite and >= 0.  One CTA per
+ * stream: the launch geometry depends only on n_streams, so the call can be captured in a CUDA graph. */
+int pn_smooth_state_bytes(int n_streams, int max_tracks, size_t *bytes_host);
+int pn_smooth_keypoints(const int64_t *ids, double *keypoint_coords, int n_img, int P, const int *stream_ids, void *state,
+                        int n_streams, int max_tracks, int max_age, double fps, double min_cutoff, double beta, double d_cutoff,
+                        pn_stream_t stream);
+
 /* ---- Whole-network plan: mobilenet_v1.py:130-162 (MobileNetV1.__init__/forward) --------------------
  * The layer table is computed by the caller (posenet/models/mobilenet_v1.py mirrors
  * _to_output_strided_layers, mobilenet_v1.py:8-39) and passed in explicitly. */

@@ -19,7 +19,7 @@ from posenet.jpeg import imdecode_batch, imencode_batch  # noqa: F401  (baseline
 from posenet.png import imencode_png_batch  # noqa: F401  (PNG encode on the GPU, bit-exact with cv2)
 from posenet.yuv import yuv_to_bgr_batch  # noqa: F401  (YUV video frames to BGR on the GPU, bit-exact with cv2.cvtColor)
 from posenet.yuv import bgr_to_yuv_batch  # noqa: F401  (BGR frames to YUV on the GPU, bit-exact with cv2.cvtColor)
-from posenet.track import PoseTracker  # noqa: F401  (pose track ids across video frames, on the GPU)
+from posenet.track import OneEuro, PoseTracker  # noqa: F401  (pose track ids and keypoint smoothing across video frames, on the GPU)
 from posenet.utils import *  # noqa: F401,F403
 from posenet.utils import _process_input, process_input_gpu, resize_u8_gpu  # noqa: F401
 from posenet.utils import draw_skel_and_kp_batch, draw_skeleton_batch  # noqa: F401  (overlays drawn on the GPU)

@@ -140,6 +140,9 @@ _SIGNATURES = {
     "pn_track_state_bytes": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
     "pn_track_poses": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                  C.c_int, C.c_double, C.c_double, C.c_void_p, C.c_void_p]),
+    "pn_smooth_state_bytes": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
+    "pn_smooth_keypoints": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                      C.c_double, C.c_double, C.c_double, C.c_double, C.c_void_p]),
     "pn_plan_query": (C.c_int, [C.POINTER(NetDesc), C.POINTER(C.c_size_t), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "pn_plan_create": (C.c_int, [C.POINTER(NetDesc), C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p)]),
     "pn_plan_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -80,7 +80,11 @@ class BatchPipeline:
         on the records after the decode and after ``source_coords`` scaling (boxes in frame pixels then), before the overlay,
         and the device-to-host stream copies the ids back after the records.  ``result`` appends them as the last item, int64
         ``[batch, P]`` (after the decode status with ``jpeg``).  The tracker's ``min_part_score=None`` takes the decode's
-        ``score_threshold``.  Works with every option but ``gather`` (each rank would hold its own tracks): ValueError."""
+        ``score_threshold``.  Works with every option but ``gather`` (each rank would hold its own tracks): ValueError.
+        A tracker with ``smoothing=OneEuro(...)`` also runs ``pn_smooth_keypoints`` in the step's graph, right after the
+        tracking: the keypoint coordinates of tracked rows are smoothed in place, so the returned records, the overlay, the
+        ``encode`` files and the ``yuv_out`` frames carry the smoothed coordinates; ids, byte counts and ``result``'s items
+        are as without it."""
         self.track = track
         if track is not None:
             from posenet.track import PoseTracker
@@ -231,7 +235,7 @@ class BatchPipeline:
 
     def _enqueue(self, s):
         """The captured part of a step: (YUV -> BGR ->) (uniform resize ->) stem .. heads -> candidates -> greedy decode
-        (-> coordinate scaling) (-> tracking) (-> overlay on the submitted frames (-> JPEG / PNG files | -> BGR -> YUV)))."""
+        (-> coordinate scaling) (-> tracking (-> smoothing)) (-> overlay on the submitted frames (-> JPEG / PNG files | -> BGR -> YUV)))."""
         x = s["x"]
         lib = nat.load()
         if self.yuv is not None:
@@ -251,6 +255,8 @@ class BatchPipeline:
                       "pn_scale_keypoint_coords")
         if self.track is not None:                                   # the warm-up's stream ids are all -1: the state stays
             self.track.launch(ps, ks, kc, s["streams"], s["ids"], self.track_part_score)
+            if self.track.smoothing is not None:                     # the boxes and ids come from the raw coordinates
+                self.track.launch_smooth(s["ids"], kc, s["streams"])
         if self.overlay:
             x = s["x"]
             nat.check(lib.pn_draw_poses(C.c_void_p(x.data_ptr()), self.batch, self.h, self.w, self.h * self.w * 3,
